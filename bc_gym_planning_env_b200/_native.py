@@ -113,8 +113,12 @@ class BcgStepOut(C.Structure):
     ]
 
 
+class BcgEnvRows(C.Structure):
+    _fields_ = [("f", C.c_void_p), ("i", C.c_void_p)]
+
+
 _STRUCTS = [BcgParams, BcgMapDesc, BcgPathDesc, BcgFootprintLut, BcgBatch, BcgStateLayout, BcgStepOut, BcgTurnParams,
-            BcgAisleSlots, BcgMiniGenParams, BcgMiniParams]
+            BcgAisleSlots, BcgMiniGenParams, BcgMiniParams, BcgEnvRows]
 
 # fixed rows / words of include/bcg_b200.h
 F_ROBOT, F_DROBOT, F_DPOSE, F_TIME, F_MIN_DIST, F_EP_RETURN, F_FIXED = 0, 7, 14, 17, 18, 19, 20
@@ -126,6 +130,9 @@ ROBOT_TRICYCLE, ROBOT_DIFFDRIVE = 0, 1
 MAP_ONLY_LETHAL = 1
 BATCH_SPARSE_EGO_ONLY = 1
 REWARD_CONTINUOUS, REWARD_PURE_PURSUIT = 0, 1
+# per-env parameter rows (BcgEnvRows)
+EP_F_SP, EP_F_AP, EP_F_PM, EP_F_ALPHA, EP_F_ROWS = 0, 1, 2, 3, 9
+EP_I_DELAY_CONTROL, EP_I_DELAY_POSE, EP_I_DELAY_STATE, EP_I_TIMEOUT, EP_I_NOISE_ON, EP_I_ROWS = 0, 1, 2, 3, 4, 5
 
 # every symbol include/bcg_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
@@ -140,6 +147,9 @@ SYMBOLS = {
     "bcg_encode_map_tensor_maps": (C.c_int, [C.POINTER(BcgMapDesc), C.c_int32, _P, C.POINTER(C.c_int32), C.c_int32,
                                              C.c_int32, _P]),
     "bcg_init_state": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P]),
+    "bcg_init_state_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P]),
+    "bcg_generate_aisles_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows),
+                                           C.POINTER(BcgAisleSlots), _P, _P, C.c_uint64, C.c_double, _P]),
     "bcg_generate_aisles": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgAisleSlots), _P, _P, C.c_uint64,
                                       C.c_double, _P]),
     "bcg_generate_minis": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgAisleSlots), _P,
@@ -149,6 +159,8 @@ SYMBOLS = {
                            C.POINTER(BcgStepOut), _P]),
     "bcg_step_events": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64,
                                   C.POINTER(BcgStepOut), C.POINTER(C.c_void_p), _P]),
+    "bcg_step_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
+                                C.POINTER(BcgStepOut), C.POINTER(C.c_void_p), _P]),
     "bcg_kinematic_step": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64, _P]),
     "bcg_collision": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, _P, _P, _P]),
     "bcg_collision_u8": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, _P, _P]),
@@ -164,6 +176,8 @@ SYMBOLS = {
     "bcg_project_poses": (C.c_int, [C.POINTER(C.c_double), _P, C.c_int64, _P, _P]),
     "bcg_observe_ego_path": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.c_int32, _P, _P, _P]),
     "bcg_rollout": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64, C.POINTER(BcgStepOut), _P]),
+    "bcg_rollout_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
+                                   C.POINTER(BcgStepOut), _P]),
     "bcg_alloc_image_memory": (C.c_int, [C.c_int64, C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
     "bcg_free_image_memory": (C.c_int, [_P, C.c_int64]),
 }

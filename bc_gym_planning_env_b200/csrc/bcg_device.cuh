@@ -270,6 +270,27 @@ __device__ __forceinline__ void delay_peek(const double* ring, int64_t stride, i
   for (int c = 0; c < NCOMP; ++c) v[c] = ring[(int64_t)(head * NCOMP + c) * stride];
 }
 
+// ---- per-env parameters (BcgEnvRows) ---------------------------------------------------------------------------------
+// The batch-wide params with env e's own values of the per-env fields in place, so that every device function keeps
+// reading one BcgParams.  The delays of `p` are the ring capacities: a row delay is clamped to [0, capacity], so what a
+// kernel touches never depends on the row contents.
+__device__ __forceinline__ BcgParams with_env_rows(const BcgParams& p, const BcgEnvRows& r, int64_t N, int e) {
+  BcgParams q = p;
+  const double* f = r.f + e;
+  const int32_t* i = r.i + e;
+  q.spatial_precision = __ldg(f + BCG_EP_F_SP * N);
+  q.angular_precision = __ldg(f + BCG_EP_F_AP * N);
+  q.progress_multiplier = __ldg(f + BCG_EP_F_PM * N);
+#pragma unroll
+  for (int k = 0; k < 6; ++k) q.alpha[k] = __ldg(f + (BCG_EP_F_ALPHA + k) * N);
+  q.delay_control = min(max(__ldg(i + BCG_EP_I_DELAY_CONTROL * N), 0), p.delay_control);
+  q.delay_pose = min(max(__ldg(i + BCG_EP_I_DELAY_POSE * N), 0), p.delay_pose);
+  q.delay_state = min(max(__ldg(i + BCG_EP_I_DELAY_STATE * N), 0), p.delay_state);
+  q.iteration_timeout = __ldg(i + BCG_EP_I_TIMEOUT * N);
+  q.noise_on = __ldg(i + BCG_EP_I_NOISE_ON * N);
+  return q;
+}
+
 // ---- footprint table lookup ----------------------------------------------------------------------
 // Work records: what the warp-per-env kernels need to know about one env, resolved by the thread-per-env
 // kernels (kinematics / pose-prep) and stored array-of-structures so that a warp gets everything with one

@@ -147,6 +147,12 @@ int check_batch(const BcgParams* p, const BcgBatch* b) {
   return BCG_OK;
 }
 
+// per-env parameter rows: NULL (batch-wide) or both row arrays
+int check_rows(const BcgEnvRows* rows) {
+  if (rows) BCG_REQUIRE(rows->f && rows->i, "null per-env parameter rows");
+  return BCG_OK;
+}
+
 // ---- kernels -------------------------------------------------------------------------------------
 
 // robot.step for every env (stand-alone bcg_kinematic_step): envs/base/env.py:371-373 (control delay) + robot model, the
@@ -590,6 +596,18 @@ struct __align__(16) StepRecord {     // 144 bytes, at the start of the env's sl
 static_assert(sizeof(StepRecord) == 144 && sizeof(StepRecord) <= BCG_WORK_BYTES, "StepRecord is 144 bytes");
 static_assert(offsetof(StepRecord, path_off) == 80 && offsetof(StepRecord, chunk_pitch) == 96 && offsetof(StepRecord, drobot) == 112,
               "move_kernel stores the record field by field");
+// batches with per-env parameters: env e's spatial / angular precision and progress multiplier (3 doubles), written by
+// move_kernel behind the StepRecord so that reward_kernel's lane groups read them with the record, not from the rows
+#define BCG_SR_ENV_OFF 144
+static_assert(BCG_SR_ENV_OFF >= sizeof(StepRecord) && BCG_SR_ENV_OFF + 24 <= BCG_WORK_BYTES, "per-env fields fit the work slot");
+__device__ __forceinline__ BcgParams with_slot_precision(const BcgParams& p, const uint8_t* fields) {
+  BcgParams q = p;
+  const double2 prec = reinterpret_cast<const double2*>(fields)[0];
+  q.spatial_precision = prec.x;
+  q.angular_precision = prec.y;
+  q.progress_multiplier = reinterpret_cast<const double*>(fields)[2];
+  return q;
+}
 #define BCG_SR_HIT 1
 #define BCG_SR_COLLIDED_AFTER 2
 #define BCG_SR_TIMED_OUT 4
@@ -663,14 +681,20 @@ __device__ __forceinline__ void write_goal_from_transform(const BcgParams& p, co
 
 // MIN_BLOCKS is the register budget: 8 CTAs per SM = 128 registers (1 024 envs in flight per SM: the large batch needs
 // the warps), 6 = 168 registers (no spills; ~3.5 us less on the chain when the whole batch fits one wave of 384 per SM).
-template <int MIN_BLOCKS>
+// ROWS: the batch has per-env parameters (`rows`, unused otherwise).  `p` then carries env e's own values, loaded with
+// the env's other top-of-kernel loads, and the goal tolerances and the progress multiplier are forwarded to
+// reward_kernel at BCG_SR_ENV_OFF of the work slot.  (The copy is kept in the kernel body, not behind a function call:
+// that way the instantiation without rows compiles to the same instructions as before rows existed.)
+template <int MIN_BLOCKS, bool ROWS>
 __global__ void __launch_bounds__(BCG_MOVE_THREADS, MIN_BLOCKS)
-move_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L, const void* __restrict__ actions,
-            const int action_is_f64, const uint64_t step_index_arg, const BcgStepOut out, const int ego_cap) {
+move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, const void* __restrict__ actions,
+            const int action_is_f64, const uint64_t step_index_arg, const BcgStepOut out, const int ego_cap,
+            const BcgEnvRows rows) {
   pdl_wait();                                            // the previous step's kernels are done with the records and rows
   pdl_launch_next();
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= b.n_envs) return;
+  const BcgParams p = ROWS ? with_env_rows(p_batch, rows, b.n_envs, e) : p_batch;
   const int64_t N = b.n_envs;
   const uint64_t step_index = b.step_counter ? *reinterpret_cast<const volatile uint64_t*>(b.step_counter) : step_index_arg;
   if (e == 0 && b.ego_list) b.ego_list[N] = b.ego_list[N + 1] = 0;       // hand-over count, env counter of the sparse kernel
@@ -816,6 +840,10 @@ move_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L, const v
   reinterpret_cast<int4*>(dst + 96)[0] = make_int4(rec.chunk_pitch, rec.target, rec.flags, rec.iter_after);
   reinterpret_cast<float4*>(dst + 112)[0] = make_float4(rec.drobot[0], rec.drobot[1], rec.drobot[2], rec.drobot[3]);
   reinterpret_cast<float2*>(dst + 128)[0] = make_float2(rec.drobot[4], rec.drobot[5]);
+  if (ROWS) {
+    reinterpret_cast<double2*>(dst + BCG_SR_ENV_OFF)[0] = make_double2(p.spatial_precision, p.angular_precision);
+    reinterpret_cast<double*>(dst + BCG_SR_ENV_OFF)[2] = p.progress_multiplier;
+  }
 }
 
 // auto-reset of env e (env.py:293-303) by its lane group: the rows, the observation and the egocentric record of the
@@ -855,9 +883,11 @@ __device__ __forceinline__ void reset_env_rows(const BcgParams& p, const BcgBatc
 // G lanes per env (power of two, 1 < G <= 32): 32 / G envs per warp.  Measured (profiles/r2_notes.md): 65 536 envs G = 8
 // 0.045 ms, 16: 0.050, 32: 0.065; 8 192 envs 0.022 / 0.018 / 0.019; 256 envs 0.0147 / 0.0121 / 0.0108 -- a large batch
 // wants few warps (the straight-line code is paid per warp), a small one a short chain (a chunk in one round).
-template <int G>
+// ROWS: the batch has per-env parameters; env e's goal tolerances and progress multiplier come from its work slot, where
+// move_kernel left them (in the kernel body for the reason given at move_kernel)
+template <int G, bool ROWS>
 __global__ void __launch_bounds__(BCG_REWARD_THREADS, BCG_REWARD_RESIDENT / BCG_REWARD_THREADS)
-reward_kernel(const BcgParams p, const BcgBatch b, const BcgStepOut out, const int ego_cap) {
+reward_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStepOut out, const int ego_cap) {
   pdl_wait();                                            // move_kernel's records
   pdl_launch_next();
   const int e = (blockIdx.x * blockDim.x + threadIdx.x) / G;
@@ -866,7 +896,9 @@ reward_kernel(const BcgParams p, const BcgBatch b, const BcgStepOut out, const i
   const int64_t N = b.n_envs;
   {
     // the env's record: a group-uniform 144-byte read (env 0's for the idle groups of the last warp)
-    const StepRecord rec = *reinterpret_cast<const StepRecord*>(reinterpret_cast<const uint8_t*>(b.work) + (int64_t)(active ? e : 0) * BCG_WORK_BYTES);
+    const uint8_t* const slot = reinterpret_cast<const uint8_t*>(b.work) + (int64_t)(active ? e : 0) * BCG_WORK_BYTES;
+    const StepRecord rec = *reinterpret_cast<const StepRecord*>(slot);
+    const BcgParams p = ROWS ? with_slot_precision(p_batch, slot + BCG_SR_ENV_OFF) : p_batch;
     PathRef pd;
     pd.P = b.path_arena + rec.path_off;
     pd.C = pd.P + 5 * (int64_t)rec.path_pitch;
@@ -996,19 +1028,25 @@ __device__ __forceinline__ void init_env_state(const BcgParams& p, const BcgBatc
   }
 }
 
-// one warp per env
-__global__ void __launch_bounds__(256) init_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L) {
+// one warp per env; ROWS: the env's own goal tolerances from `rows`
+template <bool ROWS>
+__global__ void __launch_bounds__(256) init_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L, const BcgEnvRows rows) {
   const int e = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const unsigned lane = threadIdx.x & 31;
   if (e >= b.n_envs) return;
-  init_env_state(p, b, L, e, path_ref(b, b.paths[b.path_id[e]]), lane);
+  if (ROWS)
+    init_env_state(with_env_rows(p, rows, b.n_envs, e), b, L, e, path_ref(b, b.paths[b.path_id[e]]), lane);
+  else
+    init_env_state(p, b, L, e, path_ref(b, b.paths[b.path_id[e]]), lane);
 }
 
-// bcg_generate_aisles: one CTA per env (see bcg_generate.cuh)
+// bcg_generate_aisles: one CTA per env (see bcg_generate.cuh); ROWS: the initial state uses the env's own goal tolerances
+template <bool ROWS>
 __global__ void __launch_bounds__(256) generate_aisles_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L,
                                                               const BcgAisleSlots slots, const uint8_t* __restrict__ mask,
                                                               const BcgTurnParams* __restrict__ turn_params,
-                                                              const uint64_t draw_index, const double path_delta) {
+                                                              const uint64_t draw_index, const double path_delta,
+                                                              const BcgEnvRows rows) {
   const int e = blockIdx.x;
   if (mask && !mask[e]) return;
   const int tid = threadIdx.x, nthr = blockDim.x;
@@ -1109,7 +1147,10 @@ __global__ void __launch_bounds__(256) generate_aisles_kernel(const BcgParams p,
   if (warp == 0) {
     PathRef pr;
     pr.P = P; pr.C = Cb; pr.n = shape.n; pr.pitch = pp; pr.chunk_pitch = slots.chunk_pitch;
-    init_env_state(p, b, L, e, pr, lane);
+    if (ROWS)
+      init_env_state(with_env_rows(p, rows, b.n_envs, e), b, L, e, pr, lane);
+    else
+      init_env_state(p, b, L, e, pr, lane);
   }
 }
 
@@ -2463,6 +2504,7 @@ int64_t bcg_sizeof(int32_t which) {
     case 8: return sizeof(BcgAisleSlots);
     case 9: return sizeof(BcgMiniGenParams);
     case 10: return sizeof(BcgMiniParams);
+    case 11: return sizeof(BcgEnvRows);
     default: return -1;
   }
 }
@@ -2619,16 +2661,30 @@ int bcg_encode_map_tensor_maps(const BcgMapDesc* maps_host, int32_t n_maps, cons
   return BCG_OK;
 }
 
-int bcg_init_state(const BcgParams* p, const BcgBatch* b, void* stream) {
+int bcg_init_state_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, void* stream) {
   if (int rc = check_batch(p, b)) return rc;
-  init_kernel<<<blocks_for((int64_t)b->n_envs * 32, 256), 256, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p));
+  if (int rc = check_rows(rows)) return rc;
+  const int64_t grid = blocks_for((int64_t)b->n_envs * 32, 256);
+  if (rows)
+    init_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p), *rows);
+  else
+    init_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p), BcgEnvRows{nullptr, nullptr});
   BCG_CHECK_CUDA(cudaGetLastError());
   return BCG_OK;
 }
 
+int bcg_init_state(const BcgParams* p, const BcgBatch* b, void* stream) { return bcg_init_state_rows(p, b, nullptr, stream); }
+
 int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgAisleSlots* slots, const uint8_t* mask,
                         const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta, void* stream) {
+  return bcg_generate_aisles_rows(p, b, nullptr, slots, mask, turn_params, draw_index, path_delta, stream);
+}
+
+int bcg_generate_aisles_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
+                             const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
+                             void* stream) {
   if (int rc = check_batch(p, b)) return rc;
+  if (int rc = check_rows(rows)) return rc;
   BCG_REQUIRE(slots && slots->gen_state, "null slots / gen_state");
   BCG_REQUIRE(b->cell_tile_arena, "bcg_generate_aisles needs the cell-tile arena");
   BCG_REQUIRE(!b->map_tmaps, "bcg_generate_aisles cannot re-encode TMA tensor maps; use cell-tile or plain-load staging");
@@ -2638,8 +2694,12 @@ int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgAisleSlo
               "bad slot sizes");
   BCG_REQUIRE(path_delta > 0, "path_delta must be positive");
   BCG_REQUIRE((int)(0.05 / p->resolution) <= 1, "walls are drawn one pixel thick: resolution must be above 0.025 m");
-  generate_aisles_kernel<<<b->n_envs, 256, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p), *slots, mask, turn_params,
-                                                                     draw_index, path_delta);
+  if (rows)
+    generate_aisles_kernel<true><<<b->n_envs, 256, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p), *slots, mask, turn_params,
+                                                                           draw_index, path_delta, *rows);
+  else
+    generate_aisles_kernel<false><<<b->n_envs, 256, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p), *slots, mask, turn_params,
+                                                                            draw_index, path_delta, BcgEnvRows{nullptr, nullptr});
   BCG_CHECK_CUDA(cudaGetLastError());
   return BCG_OK;
 }
@@ -2839,9 +2899,46 @@ int bcg_observe_ego(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, f
   return BCG_OK;
 }
 
+}  // extern "C"
+
+// move_kernel of one step, at the register tier the batch size picks
+template <bool ROWS>
+static int launch_move_kernel(const BcgParams* p, const BcgBatch* b, const BcgEnvRows& rows, const BcgStateLayout& L,
+                              const void* actions, int32_t action_is_f64, uint64_t step_index, const BcgStepOut* out,
+                              int cap, bool pdl, cudaStream_t s) {
+  int sms = 0;
+  if (int rc = sm_count_of_current_device(&sms)) return rc;
+  const int move_blocks = (int)blocks_for(b->n_envs, BCG_MOVE_THREADS);
+  if (move_blocks <= sms * BCG_MOVE_FEWER_BLOCKS)
+    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEWER_BLOCKS, ROWS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows));
+  else if (move_blocks <= sms * BCG_MOVE_FEW_BLOCKS)
+    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEW_BLOCKS, ROWS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows));
+  else
+    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_MIN_BLOCKS, ROWS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows));
+  return BCG_OK;
+}
+
+// reward_kernel of one step, with the lane group the batch size picks
+template <bool ROWS>
+static int launch_reward_kernel(const BcgParams* p, const BcgBatch* b, const BcgStepOut* out, int cap, bool pdl_reward, cudaStream_t s) {
+  const int64_t ns = b->n_envs;
+  if (ns > 16384) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<8, ROWS>, blocks_for(ns * 8, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
+  else if (ns > 2048) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<16, ROWS>, blocks_for(ns * 16, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
+  else BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<32, ROWS>, blocks_for(ns * 32, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
+  return BCG_OK;
+}
+
+extern "C" {
+
 int bcg_step_events(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64,
                     uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream) {
+  return bcg_step_rows(p, b, nullptr, actions, action_is_f64, step_index, out, events, stream);
+}
+
+int bcg_step_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
+                  uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream) {
   if (int rc = check_batch(p, b)) return rc;
+  if (int rc = check_rows(rows)) return rc;
   BCG_REQUIRE(actions && out, "null actions/out");
   const bool ego = out->ego_image || out->goal_n_state;
   if (ego) {
@@ -2853,23 +2950,18 @@ int bcg_step_events(const BcgParams* p, const BcgBatch* b, const void* actions, 
   {
     if (events && events[1]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[1], s));
     const int cap = ego ? ego_capacity(*p, *b) : 0;
-    int sms = 0;
-    if (int rc = sm_count_of_current_device(&sms)) return rc;
-    const int move_blocks = (int)blocks_for(b->n_envs, BCG_MOVE_THREADS);
     // (event records between the kernels are stream operations of their own: the timed form runs without the overlap)
     const bool pdl = !(events && (events[0] || events[1]));          // an event right before a kernel: no overlap for it
     const bool pdl_reward = !(events && events[2]);
-    const int64_t ns = b->n_envs;
-    if (move_blocks <= sms * BCG_MOVE_FEWER_BLOCKS)
-      BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEWER_BLOCKS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap));
-    else if (move_blocks <= sms * BCG_MOVE_FEW_BLOCKS)
-      BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEW_BLOCKS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap));
-    else
-      BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_MIN_BLOCKS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap));
+    if (rows) {
+      if (int rc = launch_move_kernel<true>(p, b, *rows, L, actions, action_is_f64, step_index, out, cap, pdl, s)) return rc;
+    } else {
+      if (int rc = launch_move_kernel<false>(p, b, BcgEnvRows{nullptr, nullptr}, L, actions, action_is_f64, step_index, out, cap, pdl, s))
+        return rc;
+    }
     if (events && events[2]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[2], s));
-    if (ns > 16384) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<8>, blocks_for(ns * 8, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
-    else if (ns > 2048) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<16>, blocks_for(ns * 16, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
-    else BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<32>, blocks_for(ns * 32, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
+    if (int rc = rows ? launch_reward_kernel<true>(p, b, out, cap, pdl_reward, s) : launch_reward_kernel<false>(p, b, out, cap, pdl_reward, s))
+      return rc;
     BCG_CHECK_CUDA(cudaGetLastError());
   }
   if (events && events[3]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[3], s));
@@ -2889,9 +2981,15 @@ int bcg_step(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t
 
 int bcg_rollout(const BcgParams* p, const BcgBatch* b, const float* plan, int32_t horizon, uint64_t step_index,
                 const BcgStepOut* out, void* stream) {
+  return bcg_rollout_rows(p, b, nullptr, plan, horizon, step_index, out, stream);
+}
+
+int bcg_rollout_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
+                     uint64_t step_index, const BcgStepOut* out, void* stream) {
   BCG_REQUIRE(plan && horizon >= 0, "null plan / negative horizon");
   for (int32_t h = 0; h < horizon; ++h)
-    if (int rc = bcg_step(p, b, plan + (int64_t)h * b->n_envs * 2, 0, step_index + (uint64_t)h, out, stream)) return rc;
+    if (int rc = bcg_step_rows(p, b, rows, plan + (int64_t)h * b->n_envs * 2, 0, step_index + (uint64_t)h, out, nullptr, stream))
+      return rc;
   return BCG_OK;
 }
 

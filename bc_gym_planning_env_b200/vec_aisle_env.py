@@ -16,6 +16,7 @@ import numpy as np
 import torch
 
 from bc_gym_planning_env_b200 import _native as nat
+from bc_gym_planning_env_b200 import env_params as envp
 from bc_gym_planning_env_b200.envs.synth_turn_env import TurnParams
 from bc_gym_planning_env_b200.utilities.costmap_2d import CostMap2D
 from bc_gym_planning_env_b200.vec_env import DEFAULT_NOISE, VecPlanEnv, _round_up, footprint_lut_for
@@ -63,8 +64,9 @@ class _VecSlotEnv(VecPlanEnv):
     cell-tile, tile-plane and path arenas, and host accessors that read a world back."""
 
     def _setup_slots(self, params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
-                     footprint_scale, footprint, map_cells, path_points, record_bytes):
-        self._configure(params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego, 'tiles')
+                     footprint_scale, footprint, map_cells, path_points, record_bytes, params_ids=None):
+        self._configure(params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego, 'tiles',
+                        params_ids)
         if not self.params.refine_path:
             raise ValueError("device-side generation always refines the path (EnvParams.refine_path)")
         if max(1, int(0.05 / self.resolution)) != 1:
@@ -150,9 +152,12 @@ class _VecSlotEnv(VecPlanEnv):
 class VecRandomAisleTurnEnv(_VecSlotEnv):
     def __init__(self, n_envs, params=None, draw_new_turn_on_reset=True, seed=0, turn_params=None,
                  noise_parameters=DEFAULT_NOISE, auto_reset=False, device=None, env_id_base=0, with_ego=False,
-                 footprint_scale=1.0, footprint=None, resolution=0.03, max_map_cells=None, max_path_points=None):
+                 footprint_scale=1.0, footprint=None, resolution=0.03, max_map_cells=None, max_path_points=None,
+                 params_ids=None):
         """
         :param n_envs: batch size; env e draws from the Philox stream (seed; env_id_base + e, draw index)
+        :param params, noise_parameters, params_ids: one EnvParams and noise setting for the batch, or a pool of them
+            and the set of every env (see VecPlanEnv); `reset(mask, params_ids=...)` moves envs to other sets
         :param draw_new_turn_on_reset: `reset` draws a new turn for the envs it resets (reference default)
         :param auto_reset: the step's own in-kernel reset.  It restores the initial state of the env's CURRENT world
             (no launch, no host round trip) and does NOT draw a new turn, whatever draw_new_turn_on_reset says: an
@@ -163,12 +168,13 @@ class VecRandomAisleTurnEnv(_VecSlotEnv):
         :param max_map_cells, max_path_points: slot capacities per env (default: worst case of the distribution)
         """
         from bc_gym_planning_env_b200.envs.base.params import EnvParams
-        pd = (params if params is not None else EnvParams()).path_delta
+        first = params[0] if envp.is_pool(params) and len(params) else params
+        pd = (first if first is not None else EnvParams()).path_delta
         cells, points = worst_case_world(float(resolution), pd)
         self._draw_new_turn_on_reset = bool(draw_new_turn_on_reset)
         self._setup_slots(params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
                           footprint_scale, footprint, max_map_cells if max_map_cells is not None else cells,
-                          max_path_points if max_path_points is not None else points, TURN_DTYPE.itemsize)
+                          max_path_points if max_path_points is not None else points, TURN_DTYPE.itemsize, params_ids)
         self._turns = self._records
         self._slots.params_out = self._turns.data_ptr()
         self.generate(turn_params=turn_params)
@@ -186,22 +192,52 @@ class VecRandomAisleTurnEnv(_VecSlotEnv):
             if arr.dtype != TURN_DTYPE or arr.shape != (self.n_envs,):
                 raise ValueError("turn_params must hold one TurnParams per env")
             tp = self._to_device(arr.view(np.uint8).reshape(self.n_envs, TURN_DTYPE.itemsize))
-        nat.check(nat.lib().bcg_generate_aisles(C.byref(self._c_params), C.byref(self._batch), C.byref(self._slots),
-                                                nat.ptr(m), nat.ptr(tp), self._draw_index, float(self.params.path_delta),
-                                                self._stream()))
+        nat.check(nat.lib().bcg_generate_aisles_rows(C.byref(self._c_params), C.byref(self._batch), self._rows,
+                                                     C.byref(self._slots), nat.ptr(m), nat.ptr(tp), self._draw_index,
+                                                     float(self.params.path_delta), self._stream()))
         self._draw_index += 1
         if tp is not None:
             torch.cuda.current_stream(self.device).synchronize()     # tp is released when this returns
 
-    def reset(self, mask=None):
+    def reset(self, mask=None, params_ids=None):
         """RandomAisleTurnEnv.reset (envs/synth_turn_env.py:278-291) for all envs (mask None) or those with
-        mask[e] true: a new turn when draw_new_turn_on_reset, the initial state either way."""
+        mask[e] true: a new turn when draw_new_turn_on_reset, the initial state either way.
+        params_ids (batches built with a pool only): [n_envs] pool indices; the envs being reset move to their entry
+        before their world and initial state are built (the entries of the other envs are ignored) -- domain
+        randomisation at episode boundaries in the same single generation launch.  Without draw_new_turn_on_reset an env
+        whose set changes gets its current world rebuilt from its recorded TurnParams, so that its initial state follows
+        the new goal tolerances."""
+        changed = None
+        if params_ids is not None:
+            changed = self._assign_params(mask, params_ids)
         if not self._draw_new_turn_on_reset:
+            if changed is not None and changed.any():
+                draw_index = self._draw_index
+                self.generate(torch.from_numpy(changed), turn_params=self.turn_params())
+                self._draw_index = draw_index              # (no draw was made)
             return super(VecRandomAisleTurnEnv, self).reset(mask)
         self.generate(mask)
         if self.with_ego:
             self.observe_ego()
         return self.observation()
+
+    def _assign_params(self, mask, params_ids):
+        """Move the masked envs to pool entries params_ids[e] (rows rebuilt and validated on the host, then uploaded);
+        returns the bool [n_envs] host mask of the envs whose set changed."""
+        if self._pool is None:
+            raise ValueError("params_ids needs a batch built with a pool of EnvParams")
+        new = np.asarray(params_ids.cpu() if isinstance(params_ids, torch.Tensor) else params_ids)
+        if new.shape != (self.n_envs,) or not np.issubdtype(new.dtype, np.integer):
+            raise ValueError("params_ids must be %d integers" % self.n_envs)
+        m = np.ones(self.n_envs, dtype=bool) if mask is None else np.asarray(
+            mask.cpu() if isinstance(mask, torch.Tensor) else mask).astype(bool).reshape(-1)
+        ids = np.where(m, new, self._params_ids_host).astype(np.int64)
+        rows = envp.build_env_rows(self._pool, self._noise_pool, ids, self.n_envs)
+        changed = ids != self._params_ids_host
+        self._params_ids_host = ids
+        self.env_rows_f.copy_(torch.from_numpy(rows.f))
+        self.env_rows_i.copy_(torch.from_numpy(rows.i))
+        return changed
 
     # ---- accessors: the worlds live on the device ----------------------------------------------------
     def turn_params(self, e=None):
@@ -248,6 +284,9 @@ class VecRandomMiniEnv(_VecSlotEnv):
         """
         from bc_gym_planning_env_b200.envs.base.params import EnvParams
         from bc_gym_planning_env_b200.envs.mini_env import RandomMiniEnvParams
+        if envp.is_pool(params):
+            # the device sampler's final check uses batch-wide goal tolerances (BcgMiniGenParams)
+            raise ValueError("VecRandomMiniEnv takes one RandomMiniEnvParams; per-env parameter pools are not supported")
         if params is None:
             params = RandomMiniEnvParams(env_params=EnvParams(goal_ang_dist=np.pi / 8., goal_spat_dist=0.2))
         self.gen_params = params

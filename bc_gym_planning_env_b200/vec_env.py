@@ -13,6 +13,7 @@ import numpy as np
 import torch
 
 from bc_gym_planning_env_b200 import _native as nat
+from bc_gym_planning_env_b200 import env_params as envp
 from bc_gym_planning_env_b200.envs.base.params import CONTINUOUS_REWARD, CONTINUOUS_REWARD_PURE_PURSUIT, EnvParams
 from bc_gym_planning_env_b200.footprint_lut import FootprintLut
 from bc_gym_planning_env_b200.robot_models.robot_dimensions import TRICYCLE, get_dimensions_example
@@ -91,13 +92,17 @@ class VecPlanEnv(object):
     def __init__(self, costmaps, paths, params=None, n_envs=None, map_ids=None, path_ids=None,
                  noise_parameters=DEFAULT_NOISE, seed=0, auto_reset=False, device=None, env_id_base=0,
                  private_map_copies=False, with_ego=False, footprint_scale=1.0, use_tma=True, footprint=None,
-                 ego_staging='tiles', ego_sparse=True, compact_ego=False):
+                 ego_staging='tiles', ego_sparse=True, compact_ego=False, params_ids=None):
         """
         :param costmaps: pool of CostMap2D (uint8), one resolution
         :param paths: pool of oriented paths, array(n, 3); refined here when params.refine_path
-        :param params EnvParams: shared by the batch
+        :param params: one EnvParams shared by the batch, or a sequence of them (a pool: env e uses
+            params[params_ids[e]]).  Delays, iteration_timeout, the goal tolerances and the progress multiplier may
+            differ between the sets of a pool; dt, robot, resolution, reward provider, refine_path and path_delta may not
         :param map_ids, path_ids: [n_envs] indices into the pools (default: env e uses entry e % len)
-        :param noise_parameters: dict alpha1..alpha6 or None (noise off); PlanEnv's default is on
+        :param noise_parameters: dict alpha1..alpha6 or None (noise off); PlanEnv's default is on.  With a pool also a
+            sequence of such settings, one per set
+        :param params_ids: [n_envs] indices into the params pool (default e % len(pool)); only with a pool
         :param private_map_copies: give every env its own copy of its costmap in HBM (pool replicated
             on device) instead of sharing pool entries
         :param with_ego: assemble the egocentric observation inside every step
@@ -121,7 +126,7 @@ class VecPlanEnv(object):
             np.count_nonzero(c.get_data()) * 20 > c.get_data().size for c in costmaps)
         self._compact_ego = bool(compact_ego)
         self._configure(params, n, float(costmaps[0].get_resolution()), noise_parameters, seed, auto_reset, device,
-                        env_id_base, with_ego, ego_staging if use_tma else 'spans')   # use_tma=False: older spelling
+                        env_id_base, with_ego, ego_staging if use_tma else 'spans', params_ids)   # use_tma=False: older spelling
         self._map_pool = costmaps
         self._map_ids_host = (np.arange(n) % len(costmaps)) if map_ids is None else np.asarray(map_ids, dtype=np.int64)
         self._path_ids_host = (np.arange(n) % len(paths)) if path_ids is None else np.asarray(path_ids, dtype=np.int64)
@@ -135,7 +140,7 @@ class VecPlanEnv(object):
         nat.check(nat.lib().bcg_build_lethal_tiles(C.byref(self._batch), 0, self._batch.n_maps, s))
         if self.cell_tile_arena is not None:
             nat.check(nat.lib().bcg_build_cell_tiles(C.byref(self._batch), 0, self._batch.n_maps, s))
-        nat.check(nat.lib().bcg_init_state(C.byref(self._c_params), C.byref(self._batch), s))
+        nat.check(nat.lib().bcg_init_state_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, s))
         self.check_status()
         if self._ego_list is not None:
             # bcg_build_lethal_tiles counted the occupied cells of every map: when none is above the library's dense
@@ -146,9 +151,20 @@ class VecPlanEnv(object):
                 self._batch.flags |= nat.BATCH_SPARSE_EGO_ONLY
 
     def _configure(self, params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
-                   ego_staging):
+                   ego_staging, params_ids=None):
         """Everything that does not depend on where the maps and paths come from."""
         nat.require_cuda()
+        self._pool = self._noise_pool = self._env_rows = None
+        if envp.is_pool(params):
+            # a pool: per-env rows (BcgEnvRows); self.params is set 0, whose batch-wide fields every set shares
+            self._pool = envp.check_pool(params)
+            self._noise_pool = envp.normalize_noise(len(self._pool), noise_parameters)
+            self._env_rows = envp.build_env_rows(self._pool, self._noise_pool, params_ids, n_envs)
+            self._params_ids_host = (np.arange(int(n_envs)) % len(self._pool) if params_ids is None
+                                     else np.asarray(params_ids, dtype=np.int64).copy())
+            params, noise_parameters = self._pool[0], self._noise_pool[0]
+        elif params_ids is not None:
+            raise ValueError("params_ids needs a pool of EnvParams (a sequence) as params")
         self.params = params if params is not None else EnvParams()
         self.device = torch.device(device) if device is not None else torch.device('cuda', torch.cuda.current_device())
         if self.device.type != 'cuda':
@@ -167,6 +183,14 @@ class VecPlanEnv(object):
         self._graph = None
         self._plan_graph = None
         self._c_params = self._make_params(noise_parameters, seed, env_id_base)
+        self._rows = None                                  # BcgEnvRows* of the library calls (None: batch-wide params)
+        if self._env_rows is not None:
+            cp = self._c_params
+            cp.delay_control, cp.delay_pose, cp.delay_state = self._env_rows.capacities     # ring capacities
+            self.env_rows_f = self._to_device(self._env_rows.f)
+            self.env_rows_i = self._to_device(self._env_rows.i)
+            self._c_rows = nat.BcgEnvRows(self.env_rows_f.data_ptr(), self.env_rows_i.data_ptr())
+            self._rows = C.byref(self._c_rows)
         self.layout = nat.state_layout(self._c_params)
 
     # ---- setup -------------------------------------------------------------------------------
@@ -460,9 +484,9 @@ class VecPlanEnv(object):
         """One env step for every env.  actions: [N, 2] float32/float64 (tensor or ndarray).
         Returns (VecObservation, reward fp64 [N], done bool [N], {}) -- tensors are reused buffers."""
         a = self._as_actions(actions)
-        nat.check(nat.lib().bcg_step(C.byref(self._c_params), C.byref(self._batch), nat.ptr(a),
-                                     1 if a.dtype == torch.float64 else 0, self._step_index,
-                                     C.byref(self._out), self._stream()))
+        nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
+                                          1 if a.dtype == torch.float64 else 0, self._step_index,
+                                          C.byref(self._out), None, self._stream()))
         self._step_index += 1
         return self.observation(), self.reward, self.done, {}
 
@@ -485,8 +509,9 @@ class VecPlanEnv(object):
             g = torch.cuda.CUDAGraph()
             with torch.cuda.stream(side):
                 with torch.cuda.graph(g, stream=side):
-                    nat.check(nat.lib().bcg_step(C.byref(self._c_params), C.byref(self._batch), nat.ptr(self.actions), 0, 0,
-                                                 C.byref(self._out), C.c_void_p(side.cuda_stream)))
+                    nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows,
+                                                      nat.ptr(self.actions), 0, 0, C.byref(self._out), None,
+                                                      C.c_void_p(side.cuda_stream)))
             torch.cuda.current_stream(self.device).wait_stream(side)
             self._graph = g
         elif actions is not None:
@@ -505,8 +530,8 @@ class VecPlanEnv(object):
             raise ValueError("plan must have shape [H, %d, 2]" % self.n_envs)
         plan = plan.to(torch.float32).contiguous()
         horizon = int(plan.shape[0])
-        nat.check(nat.lib().bcg_rollout(C.byref(self._c_params), C.byref(self._batch), nat.ptr(plan), horizon, self._step_index,
-                                        C.byref(self._out), self._stream()))
+        nat.check(nat.lib().bcg_rollout_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(plan), horizon,
+                                             self._step_index, C.byref(self._out), self._stream()))
         self._step_index += horizon
 
     def rollout_graph(self, plan):
@@ -532,8 +557,9 @@ class VecPlanEnv(object):
             with torch.cuda.stream(side):
                 with torch.cuda.graph(g, stream=side):
                     for h in range(horizon):
-                        nat.check(nat.lib().bcg_step(C.byref(self._c_params), C.byref(self._batch), nat.ptr(buf[h]), 0, 0,
-                                                     C.byref(self._out), C.c_void_p(side.cuda_stream)))
+                        nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows,
+                                                          nat.ptr(buf[h]), 0, 0, C.byref(self._out), None,
+                                                          C.c_void_p(side.cuda_stream)))
             torch.cuda.current_stream(self.device).wait_stream(side)
             self._plan_graph = (horizon, g, buf)
         else:
@@ -555,9 +581,9 @@ class VecPlanEnv(object):
         handles exist; entries may be None) recorded around the kernels; see bcg_step_events."""
         a = self._as_actions(actions)
         handles = (C.c_void_p * 5)(*[C.c_void_p(ev.cuda_event if ev is not None else None) for ev in events])
-        nat.check(nat.lib().bcg_step_events(C.byref(self._c_params), C.byref(self._batch), nat.ptr(a),
-                                            1 if a.dtype == torch.float64 else 0, self._step_index,
-                                            C.byref(self._out), handles, self._stream()))
+        nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
+                                          1 if a.dtype == torch.float64 else 0, self._step_index,
+                                          C.byref(self._out), handles, self._stream()))
         self._step_index += 1
         return self.observation(), self.reward, self.done, {}
 
@@ -774,6 +800,16 @@ class VecPlanEnv(object):
         if tuple(state.f.shape) != (self.layout.n_frows, k) or tuple(state.i.shape) != (self.layout.n_irows, k):
             raise ValueError("snapshot shape does not match the env layout / index count")
         f, i = state.f.to(self.device).contiguous(), state.i.to(self.device).contiguous()
+        if self._env_rows is not None and k:
+            # a column must fit the target env's own rings: queue length <= its delay, head inside it (empty when 0)
+            d = self.env_rows_i[nat.EP_I_DELAY_CONTROL:nat.EP_I_DELAY_STATE + 1][:, idx]
+            q = i[nat.I_QC:nat.I_QS + 1]
+            head, length = q & 0xffff, q >> 16
+            bad = (length > d) | ((head >= d) & (q != 0))
+            if bool(bad.any()):
+                col = int(torch.nonzero(bad.any(dim=0))[0, 0])
+                raise ValueError("set_state: snapshot column %d holds queues (head | len << 16 = %s) that do not fit the "
+                                 "delays %s of env %d" % (col, q[:, col].tolist(), d[:, col].tolist(), int(idx[col])))
         nat.check(nat.lib().bcg_scatter_state(C.byref(self._batch), nat.ptr(idx), k, nat.ptr(f), nat.ptr(i),
                                               1 if load_delayed_robot else 0, self._stream()))
 
@@ -852,9 +888,43 @@ class VecPlanEnv(object):
     def costmap(self, e):
         return self._map_pool[int(self._map_ids_host[e])]
 
-    def queue_rows(self, which):
-        """(first fp64 row, slots, components, int row) of a delay ring: 'control' | 'pose' | 'state'."""
+    def queue_rows(self, which, e=None):
+        """(first fp64 row, slots, components, int row) of a delay ring: 'control' | 'pose' | 'state'.  `slots` is the
+        ring's capacity, or with `e` the delay of env e: the slots its queue uses (the modulus of its head)."""
         L, p = self.layout, self.params
+        if e is not None:
+            p = self.params_of(e)
+        elif self._pool is not None:
+            cp = self._c_params
+            return {'control': (L.ring_control, cp.delay_control, 2, nat.I_QC),
+                    'pose': (L.ring_pose, cp.delay_pose, 3, nat.I_QP),
+                    'state': (L.ring_state, cp.delay_state, 7, nat.I_QS)}[which]
         return {'control': (L.ring_control, p.control_delay, 2, nat.I_QC),
                 'pose': (L.ring_pose, p.pose_delay, 3, nat.I_QP),
                 'state': (L.ring_state, p.state_delay, 7, nat.I_QS)}[which]
+
+    # ---- per-env parameters ----------------------------------------------------------------------
+    def params_of(self, e):
+        """The EnvParams env e steps with."""
+        return self.params if self._pool is None else self._pool[int(self._params_ids_host[int(e)])]
+
+    def noise_of(self, e):
+        """The odometry noise setting (dict alpha1..alpha6, or None for off) env e steps with."""
+        if self._pool is None:
+            cp = self._c_params
+            return dict(('alpha%d' % (k + 1), cp.alpha[k]) for k in range(6)) if cp.noise_on else None
+        return self._noise_pool[int(self._params_ids_host[int(e)])]
+
+    @property
+    def params_ids(self):
+        """int64 [N] host array: the pool entry of every env (None without a pool)"""
+        return None if self._pool is None else self._params_ids_host.copy()
+
+    @property
+    def delays(self):
+        """int32 [N, 3] device tensor: the control, pose and state delay of every env"""
+        if self._pool is not None:
+            return self.env_rows_i[nat.EP_I_DELAY_CONTROL:nat.EP_I_DELAY_STATE + 1].t()
+        p = self.params
+        return torch.tensor([[p.control_delay, p.pose_delay, p.state_delay]], dtype=torch.int32,
+                            device=self.device).expand(self.n_envs, 3)

@@ -268,6 +268,27 @@ typedef struct BcgStateLayout {
   int32_t ring_state;   /* delay_state slots x 7 rows                                        */
 } BcgStateLayout;
 
+/* Per-env parameters of a batch whose envs do not all share one EnvParams / noise setting: structure of arrays like
+ * state_f / state_i, f[row * n_envs + env] (fp64 rows BCG_EP_F_*) and i[row * n_envs + env] (int32 rows BCG_EP_I_*).
+ * They override the same fields of BcgParams for env `env`; everything else stays batch-wide.  The delays in BcgParams
+ * are then the ring capacities (the per-field maxima of the rows: bcg_state_layout sizes the rings from them), and env e
+ * uses the first min(d_e, capacity) slots of each ring.  A NULL BcgEnvRows* means "every env uses BcgParams". */
+#define BCG_EP_F_SP 0       /* RewardParams.spatial_precision                          */
+#define BCG_EP_F_AP 1       /* RewardParams.angular_precision                          */
+#define BCG_EP_F_PM 2       /* RewardParams.spatial_progress_multiplier                */
+#define BCG_EP_F_ALPHA 3    /* 6 rows: odometry noise alpha1..alpha6 (used when noise_on) */
+#define BCG_EP_F_ROWS 9
+#define BCG_EP_I_DELAY_CONTROL 0
+#define BCG_EP_I_DELAY_POSE 1
+#define BCG_EP_I_DELAY_STATE 2
+#define BCG_EP_I_TIMEOUT 3  /* EnvParams.iteration_timeout                             */
+#define BCG_EP_I_NOISE_ON 4 /* 0: the env's robot moves without odometry noise          */
+#define BCG_EP_I_ROWS 5
+typedef struct BcgEnvRows {
+  const double* f;   /* device [BCG_EP_F_ROWS][n_envs] */
+  const int32_t* i;  /* device [BCG_EP_I_ROWS][n_envs] */
+} BcgEnvRows;
+
 /* outputs of one step; any pointer may be NULL to skip that output */
 typedef struct BcgStepOut {
   double* reward;      /* [n] reward of this step (reward.py:214-259)                          */
@@ -293,7 +314,7 @@ int bcg_abi_version(void);
 size_t bcg_last_error(char* buf, size_t cap);
 /* sizeof() of the ABI structs, in declaration order: 0 BcgParams, 1 BcgMapDesc, 2 BcgPathDesc,
  * 3 BcgFootprintLut, 4 BcgBatch, 5 BcgStateLayout, 6 BcgStepOut, 7 BcgTurnParams, 8 BcgAisleSlots, 9 BcgMiniGenParams,
- * 10 BcgMiniParams; -1 for anything else.  Lets a
+ * 10 BcgMiniParams, 11 BcgEnvRows; -1 for anything else.  Lets a
  * binding (ctypes, cffi, ...) verify its struct mirrors before the first call. */
 int64_t bcg_sizeof(int32_t which);
 /* number of CUDA devices visible, <0 on error; makes a missing GPU a loud failure for callers */
@@ -317,6 +338,9 @@ int bcg_encode_map_tensor_maps(const BcgMapDesc* maps_host, int32_t n_maps, cons
 /* make_initial_state (env.py:179-214) + ContinuousRewardProvider.generate_initial_state
  * (reward.py:261-288) for every env: writes init_f/init_i and copies them into state_f/state_i */
 int bcg_init_state(const BcgParams* p, const BcgBatch* b, void* stream);
+/* bcg_init_state with per-env goal tolerances: env e's initial target index uses its own spatial / angular precision
+ * from `rows` (NULL: bcg_init_state) */
+int bcg_init_state_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, void* stream);
 /* PlanEnv.reset (env.py:293-303) for envs with mask[e] != 0 (mask NULL = all) */
 int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream);
 
@@ -329,6 +353,11 @@ int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream);
  * Not available together with TMA tensor maps (map_tmaps), which cannot be re-encoded on the device. */
 int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgAisleSlots* slots, const uint8_t* mask,
                         const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta, void* stream);
+/* bcg_generate_aisles whose initial states use each env's own goal tolerances from `rows` (NULL: bcg_generate_aisles).
+ * Rows changed before the call (a new parameter set at a reset) are what the new worlds' initial states see. */
+int bcg_generate_aisles_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
+                             const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
+                             void* stream);
 
 /* RandomMiniEnv's env construction (envs/mini_env.py:323-389, what its reset repeats) on the device, for envs with
  * mask[e] != 0 (mask NULL = all), in the same per-env slots as bcg_generate_aisles: sample MiniEnvParams (:269-320,
@@ -364,6 +393,13 @@ int bcg_step(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t
  * launched as a programmatic dependent of its predecessor.  events == NULL behaves exactly like bcg_step. */
 int bcg_step_events(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64,
                     uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream);
+
+/* bcg_step_events for a batch with per-env parameters (BcgEnvRows; NULL: bcg_step_events).  move_kernel reads env e's
+ * delays, timeout, noise flag and alphas from the rows with its other top-of-kernel loads and forwards its goal tolerances
+ * and progress multiplier to reward_kernel in the env's work slot.  Ring capacities are p's delays; a row delay above
+ * its capacity is clamped to it (memory safety does not depend on the row contents; the host validates them). */
+int bcg_step_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
+                  uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream);
 
 /* the pieces, individually addressable (used by tests, ncu and the hook seam) */
 /* robot.step (tricycle_model.py:478-538 / differential_drive.py:236-265) into b->cand */
@@ -430,6 +466,9 @@ int bcg_observe_ego_path(const BcgParams* p, const BcgBatch* b, int32_t max_poin
  * step h uses the Philox step index step_index + h (or the device-side counter when BcgBatch.step_counter is set). */
 int bcg_rollout(const BcgParams* p, const BcgBatch* b, const float* plan, int32_t horizon, uint64_t step_index,
                 const BcgStepOut* out, void* stream);
+/* bcg_rollout for a batch with per-env parameters (see bcg_step_rows; rows NULL: bcg_rollout) */
+int bcg_rollout_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
+                     uint64_t step_index, const BcgStepOut* out, void* stream);
 
 /* -- image memory --------------------------------------------------------------------------------
  * Egocentric crops are mostly zeros.  A device allocation with compute-data compression (CUDA virtual memory
