@@ -127,8 +127,8 @@ STATUS_LUT_MISS, STATUS_PATH_EXHAUSTED, STATUS_SLOT_OVERFLOW, STATUS_SAMPLER_EMP
 STAT_NAMES = ("episodes", "return", "length", "collided", "goal", "timeout")
 STATS_WORDS = 8
 ROBOT_TRICYCLE, ROBOT_DIFFDRIVE = 0, 1
-MAP_ONLY_LETHAL = 1
-BATCH_SPARSE_EGO_ONLY = 1
+MAP_ONLY_LETHAL, MAP_CELL_INDEX = 1, 4
+BATCH_SPARSE_EGO_ONLY, BATCH_CELL_INDEX = 1, 2
 REWARD_CONTINUOUS, REWARD_PURE_PURSUIT = 0, 1
 # per-env parameter rows (BcgEnvRows)
 EP_F_SP, EP_F_AP, EP_F_PM, EP_F_ALPHA, EP_F_ROWS = 0, 1, 2, 3, 9

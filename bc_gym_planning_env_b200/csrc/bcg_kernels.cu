@@ -416,7 +416,8 @@ struct __align__(16) EgoTileWork {   // 128 bytes
   int32_t fwd[6];                    // cv::warpAffine's forward matrix (source -> crop) in 16.16 fixed point, translation
                                      // relative to the window origin (X0, Y0): the sparse kernel's candidate pixels
   int32_t dense_map;                 // bit 0: more than 1 cell in 20 of the map is occupied (skip the sparse kernel's
-                                     // scan); bit 1: every occupied cell is 254 (BCG_MAP_ONLY_LETHAL)
+                                     // scan); bit 1: every occupied cell is 254 (BCG_MAP_ONLY_LETHAL); bit 2: the map's
+                                     // cell index is exact (BCG_MAP_CELL_INDEX)
   // what the sparse kernel needs of the map descriptor, so that its loads start from the record alone
   int32_t sum_off;                   // BcgMapDesc.sum_off
   uint32_t tiles_xy;                 // tiles_x | tiles_y << 16
@@ -460,7 +461,8 @@ __device__ __forceinline__ void write_ego_tile_record(const BcgParams& p, const 
   w.X0 = w.Y0 = w.ntx = w.nty = 0;
   w.mode = BCG_EGO_MODE_DIRECT;
   w.map_id = map_id;
-  w.dense_map = (((int64_t)m.occupied * 20 > (int64_t)m.width * m.height) ? 1 : 0) | ((m.flags & BCG_MAP_ONLY_LETHAL) ? 2 : 0);
+  w.dense_map = (((int64_t)m.occupied * 20 > (int64_t)m.width * m.height) ? 1 : 0) | ((m.flags & BCG_MAP_ONLY_LETHAL) ? 2 : 0) |
+                (m.flags & BCG_MAP_CELL_INDEX);
   w.sum_off = m.sum_off;
   w.tiles_xy = (uint32_t)m.tiles_x | ((uint32_t)m.tiles_y << 16);
   w.tile_off16 = (uint32_t)(m.tile_off >> 4);
@@ -1384,10 +1386,70 @@ __global__ void __launch_bounds__(256) zero_occupied_kernel(const BcgBatch b, co
   if (k >= count) return;
   BcgMapDesc* m = const_cast<BcgMapDesc*>(b.maps) + first + k;
   m->occupied = 0;
+  m->flags &= ~BCG_MAP_CELL_INDEX;                      // set again by cell_index_kernel once the index matches the plane
   if (b.occ_tile_arena && b.occ_sum_arena) {            // tiles_kernel only sets summary bits
     uint32_t* sum = const_cast<uint32_t*>(b.occ_sum_arena) + m->sum_off;
     const int words = m->tiles_y * ((m->tiles_x + 31) >> 5);
     for (int i = 0; i < words; ++i) sum[i] = 0u;
+  }
+}
+
+// Cell index of one map per CTA (BCG_BATCH_CELL_INDEX trailer, after tiles_kernel): per 32 x 16 tile of the occupancy
+// plane its cell count, an exclusive block scan of the counts in row-major tile order (prefix), and the cells themselves,
+// row-major inside each tile, at their tile's prefix.  Dense maps get no trailer; a map whose cells exceed the trailer's
+// capacity keeps BCG_MAP_CELL_INDEX clear (nothing is written past the capacity).
+#define BCG_CIX_THREADS 256
+__global__ void __launch_bounds__(BCG_CIX_THREADS) cell_index_kernel(const BcgBatch b, const int first) {
+  __shared__ int warp_sum[BCG_CIX_THREADS / 32];
+  const BcgMapDesc m = b.maps[first + blockIdx.x];
+  if ((int64_t)m.occupied * 20 > (int64_t)m.width * m.height) return;
+  const int ntiles = m.tiles_x * m.tiles_y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t* const occ = b.occ_tile_arena + m.tile_off;
+  uint32_t* const trailer = const_cast<uint32_t*>(b.occ_sum_arena) + m.sum_off + m.tiles_y * ((m.tiles_x + 31) >> 5);
+  uint32_t* const prefix = trailer + 2;
+  uint32_t* const cells = prefix + ntiles + 1;
+  const uint32_t cap = trailer[0];
+  uint32_t running = 0u;
+  for (int t0 = 0; t0 < ntiles; t0 += BCG_CIX_THREADS) {
+    const int t = t0 + tid;
+    int cnt = 0;
+    if (t < ntiles)
+      for (int r = 0; r < 16; ++r) cnt += __popc(occ[t * 16 + r]);
+    int incl = cnt;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int v = __shfl_up_sync(BCG_FULL, incl, d);
+      if (lane >= d) incl += v;
+    }
+    if (lane == 31) warp_sum[warp] = incl;
+    __syncthreads();
+    int before = 0, chunk = 0;
+    for (int w = 0; w < BCG_CIX_THREADS / 32; ++w) {
+      const int s = warp_sum[w];
+      if (w < warp) before += s;
+      chunk += s;
+    }
+    __syncthreads();                        // warp_sum is rewritten by the next chunk
+    if (t < ntiles) {
+      uint32_t at = running + (uint32_t)(before + incl - cnt);
+      prefix[t] = at;
+      const int ty = t / m.tiles_x, tx = t - ty * m.tiles_x;
+      for (int r = 0; r < 16; ++r) {
+        uint32_t w = occ[t * 16 + r];
+        while (w) {
+          const int bit = __ffs((int)w) - 1;
+          w &= w - 1u;
+          if (at < cap) cells[at] = (uint32_t)((tx << 5) + bit) | ((uint32_t)((ty << 4) + r) << 16);
+          ++at;
+        }
+      }
+    }
+    running += (uint32_t)chunk;
+  }
+  if (tid == 0) {
+    prefix[ntiles] = running;
+    trailer[1] = running;
+    if (running <= cap) atomicOr(&const_cast<BcgMapDesc*>(b.maps)[first + blockIdx.x].flags, BCG_MAP_CELL_INDEX);
   }
 }
 
@@ -1848,6 +1910,10 @@ __global__ void __launch_bounds__(BCG_EGT_THREADS, BCG_EGT_CTAS) ego_tiles_kerne
 #define BCG_EGS_DYNAMIC 1            // 1: envs beyond a CTA's first four are drawn from a global counter
 #endif
 #define BCG_EGS_QCAP 64              // ring slots per warp: a push adds <= 32 to <= 31 left over
+#ifndef BCG_EGS_CELL_ROUNDS
+#define BCG_EGS_CELL_ROUNDS 8        // with a cell index: cells loaded per thread before the first is resolved (65 536
+                                     // envs: 2: 0.2884 ms per step, 4: 0.2792, 8: 0.2773; profiles/r3b_notes.md)
+#endif
 #ifndef BCG_EGS_SPANS
 #define BCG_EGS_SPANS 1              // clip the listed cells to the tile spans of the rotated crop (0: to its bounding box)
 #endif
@@ -1943,16 +2009,26 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     if (en < n && tid < BCG_EGO_WORK_BYTES / 16)
       cp_async_16(rec_u32 + slot * BCG_EGO_WORK_BYTES + tid * 16, recs + (int64_t)en * BCG_EGO_WORK_BYTES + tid * 16, 16u);
   };
+  const bool cix_batch = SUM && (b.flags & BCG_BATCH_CELL_INDEX) != 0;
   // Tile-summary words of the window of record `q`, lane <-> band of 16 rows (zero where the band or the word lies
-  // outside the map, or the env will not take the sparse path).  Loaded one env ahead of their use, so that an env's
-  // chain of dependent DRAM round trips is the occupancy words alone.
-  auto summary_words = [&](const EgoTileWork* q, uint32_t& lo, uint32_t& hi) {
+  // outside the map, or the env will not take the sparse path).  With a cell index (BCG_BATCH_CELL_INDEX) they are the
+  // band's prefix counts at the window's first tile column and one past its last instead: the band's cells are
+  // cells[lo .. hi).  Loaded one env ahead of their use, so that an env's chain of dependent DRAM round trips is the
+  // occupancy words (or cells) alone.
+  auto summary_words = [&](const EgoTileWork* q, uint32_t& lo, uint32_t& hi, const bool use_index) {
     lo = hi = 0u;
     if (q->mode != BCG_EGO_MODE_TILES || (q->dense_map & 1)) return;
     const int qby0 = q->Y0 >> 4, qnby = ((q->Y0 + 8 * q->nty - 1) >> 4) - qby0 + 1;
     const int qtx = (int)(q->tiles_xy & 0xffffu), qty = (int)(q->tiles_xy >> 16), sw = (qtx + 31) >> 5;
     const int ty = qby0 + lane, w0 = q->X0 >> 10;                            // X0 >> 5 may be negative: w0 = -1
     if (lane < qnby && (unsigned)ty < (unsigned)qty) {
+      if (use_index && cix_batch && (q->dense_map & 4)) {
+        const uint32_t* const prow = b.occ_sum_arena + q->sum_off + qty * sw + 2 + ty * qtx;
+        const int c0 = min(max(q->X0 >> 5, 0), qtx), c1 = min(max(((q->X0 + 16 * q->ntx - 1) >> 5) + 1, c0), qtx);
+        lo = __ldg(prow + c0);
+        hi = __ldg(prow + c1);
+        return;
+      }
       const uint32_t* const srow = b.occ_sum_arena + q->sum_off + ty * sw;
       if ((unsigned)w0 < (unsigned)sw) lo = __ldg(srow + w0);
       if ((unsigned)(w0 + 1) < (unsigned)sw) hi = __ldg(srow + w0 + 1);
@@ -1988,7 +2064,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
   make_spans(0, 0);
   __syncthreads();
   uint32_t pf_lo = 0u, pf_hi = 0u;              // summary words of the env about to be rendered
-  if (SUM) summary_words(reinterpret_cast<const EgoTileWork*>(rec_s), pf_lo, pf_hi);
+  if (SUM) summary_words(reinterpret_cast<const EgoTileWork*>(rec_s), pf_lo, pf_hi, true);
 #if BCG_EGS_DYNAMIC
   for (int it = 0;; ++it) {
     const int e = ids_s[it & 7];
@@ -2010,7 +2086,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     // record it + 1 has landed (only the newest fetch may still be in flight): start its summary loads now
     const uint32_t cur_lo = pf_lo, cur_hi = pf_hi;
     if (SUM && e_next < n)
-      summary_words(reinterpret_cast<const EgoTileWork*>(rec_s + ((it + 1) & (BCG_EGS_REC_SLOTS - 1)) * BCG_EGO_WORK_BYTES), pf_lo, pf_hi);
+      summary_words(reinterpret_cast<const EgoTileWork*>(rec_s + ((it + 1) & (BCG_EGS_REC_SLOTS - 1)) * BCG_EGO_WORK_BYTES), pf_lo, pf_hi, true);
     if (e_next < n) make_spans((it + 1) & (BCG_EGS_REC_SLOTS - 1), (it + 1) & 1);
     const EgoTileWork* r = reinterpret_cast<const EgoTileWork*>(rec_s + slot * BCG_EGO_WORK_BYTES);
     const int mode = r->mode, X0 = r->X0, Y0 = r->Y0, ntx = r->ntx, nty = r->nty;
@@ -2022,6 +2098,30 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     // almost every window: they go straight to the dense kernel instead of paying for a scan that is thrown away
     const bool dense_map = (r->dense_map & 1) != 0;     // decided by the record writer, which holds the map descriptor
     const bool try_sparse = mode == BCG_EGO_MODE_TILES && ntile <= BCG_EGS_MAX_TILES && !dense_map && (!SUM || (nby <= 32 && nwx <= 32));
+    // With a cell index (BCG_BATCH_CELL_INDEX, map bit in the record) band b's cells are cells[lo_b .. hi_b) (the words
+    // `summary_words` loaded, lane <-> band).  An inclusive warp scan of the band counts numbers the window's cells
+    // 0 .. total - 1, and cell j of band b is cells[j + lo_b - start_b]: the scatter reads them straight from there.
+    // Nothing is listed or staged; the cells of the bands outside the rotated crop fail the scatter's candidate test like
+    // any other.  A window with more than BCG_EGS_LIST cells in its bands (whose cells inside the crop's tile spans may
+    // or may not overflow the list) is listed from the occupancy plane instead, so that the overflow rule -- and with it
+    // which envs report a compact hit list -- stays exactly that of the listing.
+    const bool has_index = SUM && cix_batch && try_sparse && (r->dense_map & 4);
+    int bincl = 0, boff = 0, total = 0;
+    const uint32_t* cells = nullptr;
+    if (has_index) {
+      const int bcnt = (int)(cur_hi - cur_lo);
+      bincl = bcnt;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const int v = __shfl_up_sync(BCG_FULL, bincl, d);
+        if (lane >= d) bincl += v;
+      }
+      total = __shfl_sync(BCG_FULL, bincl, 31);
+      boff = (int)cur_lo - (bincl - bcnt);
+      const int tx_ = (int)(r->tiles_xy & 0xffffu), ty_ = (int)(r->tiles_xy >> 16);
+      cells = b.occ_sum_arena + r->sum_off + ty_ * ((tx_ + 31) >> 5) + 3 + tx_ * ty_;
+    }
+    const bool cix = has_index && total <= BCG_EGS_LIST;
     if (try_sparse) {
       // ---- 1. zero the crop in global memory ----------------------------------------------------------------------
       {
@@ -2141,10 +2241,14 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
           qhead += 32u;
         }
       };
-      if constexpr (SUM) {
+      if (cix) {
+        // cell index: nothing to list, the scatter below reads the window's cells from the index
+      } else if constexpr (SUM) {
+        uint32_t slo = cur_lo, shi = cur_hi;
+        if (has_index) summary_words(r, slo, shi, false);                       // the prefetched words were prefix counts
         // (a) which tiles of the window hold a cell at all: lane <-> band of 16 rows, one or two words of the map's tile
         // summary each, loaded one env ahead (`summary_words`; every warp holds the same words: no barrier)
-        const uint32_t tmask = (uint32_t)((((uint64_t)cur_hi << 32) | cur_lo) >> (wx0 & 31)) & ((1u << nwx) - 1u);
+        const uint32_t tmask = (uint32_t)((((uint64_t)shi << 32) | slo) >> (wx0 & 31)) & ((1u << nwx) - 1u);
         // (b) the list of those tiles (band << 6 | column), in band order: inclusive warp scan of the per-band counts
         int tincl = __popc(tmask);
 #pragma unroll
@@ -2211,7 +2315,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     cp_async_wait_group_1();                  // the record needed next iteration has landed
     __syncthreads();                          // zeros (incl. head / tail bytes), tables, list and count are complete
     const uint32_t count = T.count[par];
-    const bool sparse = try_sparse && count <= BCG_EGS_LIST;
+    const bool sparse = try_sparse && (cix || count <= BCG_EGS_LIST);
     if (sparse) {
       // ---- 3. scatter the listed cells ----------------------------------------------------------------------------
       const bool only_lethal = (r->dense_map & 2) != 0;
@@ -2231,14 +2335,12 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
       asm volatile("" : "+r"(abase), "+r"(bbase), "+r"(lethal_value));
       auto scatter = [&](auto lethal_tag) {
       constexpr bool LETHAL = decltype(lethal_tag)::value;
-      for (uint32_t i = tid; i < count; i += NT) {
-        const uint32_t key = lds_u32(list_u32 + 4u * i);
-        const int xr = (int)(key & 0xffffu), yr = (int)(key >> 16);
+      auto resolve = [&](const int xr, const int yr) {
         // candidates only, in 16.16 integers (no conversions: they run on the quarter-rate unit); the fixed-point test
         // below decides
         const int fu = (m0 * xr + m1 * yr + m2) >> 16;
         const int fv = (m3 * xr + m4 * yr + m5) >> 16;
-        if (fu < -1 || fu >= ego_w || fv < -1 || fv >= ego_h) continue;     // every candidate is outside the crop
+        if (fu < -1 || fu >= ego_w || fv < -1 || fv >= ego_h) return;       // every candidate is outside the crop
         uint32_t val = lethal_value;
         if (!LETHAL) val = __ldg(src + (int64_t)(Y0 + yr) * pitch + (X0 + xr));
         // candidates (fu | fu + 1, fv | fv + 1); fu in [-1, ego_w - 1], fv in [-1, ego_h - 1]: the outer ones are sentinels
@@ -2277,6 +2379,35 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
             if (h01) { if (at < (uint32_t)hit_cap) out[at] = tagged | (uint32_t)(o00 + ego_w); ++at; }
             if (h11) { if (at < (uint32_t)hit_cap) out[at] = tagged | (uint32_t)(o00 + ego_w + 1); ++at; }
           }
+        }
+      };
+      if (cix) {
+        // BCG_EGS_CELL_ROUNDS cells per thread are loaded before the first is resolved; a cell's band is found by a
+        // binary search over the band scan (lanes >= the window's bands hold `total`)
+        constexpr int CR = BCG_EGS_CELL_ROUNDS;
+        for (int base = warp * 32; base < total; base += CR * NT) {
+          uint32_t cell[CR];
+#pragma unroll
+          for (int rd = 0; rd < CR; ++rd) {
+            const int j = base + rd * NT + lane;
+            cell[rd] = 0u;
+            if (base + rd * NT < total) {                                      // warp-uniform
+              int bnd = 0;                                                     // bands whose cells all precede j
+#pragma unroll
+              for (int s = 16; s > 0; s >>= 1)
+                if (__shfl_sync(BCG_FULL, bincl, bnd + s - 1) <= j) bnd += s;
+              const int off = __shfl_sync(BCG_FULL, boff, bnd);
+              if (j < total) cell[rd] = __ldg(cells + j + off);
+            }
+          }
+#pragma unroll
+          for (int rd = 0; rd < CR; ++rd)
+            if (base + rd * NT + lane < total) resolve((int)(cell[rd] & 0xffffu) - X0, (int)(cell[rd] >> 16) - Y0);
+        }
+      } else {
+        for (uint32_t i = tid; i < count; i += NT) {
+          const uint32_t key = lds_u32(list_u32 + 4u * i);
+          resolve((int)(key & 0xffffu), (int)(key >> 16));
         }
       }
       };
@@ -2534,6 +2665,10 @@ int bcg_build_lethal_tiles(const BcgBatch* b, int32_t first, int32_t count, void
   for (int32_t done = 0; done < count; done += 32768) {
     const int32_t chunk = (count - done) < 32768 ? (count - done) : 32768;
     tiles_kernel<<<dim3(8, chunk), 256, 0, s>>>(*b, first + done);
+    BCG_CHECK_CUDA(cudaGetLastError());
+  }
+  if ((b->flags & BCG_BATCH_CELL_INDEX) && b->occ_tile_arena && b->occ_sum_arena && count > 0) {
+    cell_index_kernel<<<count, BCG_CIX_THREADS, 0, s>>>(*b, first);
     BCG_CHECK_CUDA(cudaGetLastError());
   }
   return BCG_OK;

@@ -232,6 +232,7 @@ class VecPlanEnv(object):
     def _upload_maps(self, costmaps, private_copies):
         descs = (nat.BcgMapDesc * len(costmaps))()
         data_off, tile_off, ctile_off, sum_off = 0, 0, 0, 0
+        capacity_at, capacities = [], []
         for k, cm in enumerate(costmaps):
             data = cm.get_data()
             if data.dtype != np.uint8 or data.ndim != 2:
@@ -249,6 +250,12 @@ class VecPlanEnv(object):
             d.ctiles_x, d.ctiles_y = d.pitch // 16, (h + 7) // 8
             d.data_off, d.tile_off, d.cell_tile_off, d.sum_off = data_off, tile_off, ctile_off, sum_off
             sum_off += d.tiles_y * ((d.tiles_x + 31) // 32)
+            # the map's cell index (BCG_BATCH_CELL_INDEX trailer, filled by bcg_build_lethal_tiles): dense maps get none
+            nnz = int(np.count_nonzero(data))
+            if nnz * 20 <= h * w:
+                capacity_at.append(sum_off)
+                capacities.append(nnz)
+                sum_off += 3 + d.tiles_x * d.tiles_y + nnz
             data_off += _round_up(h * d.pitch, 128)
             tile_off += d.tiles_x * d.tiles_y * 16
             ctile_off += d.ctiles_x * d.ctiles_y * 128
@@ -258,6 +265,8 @@ class VecPlanEnv(object):
             view = arena[d.data_off:d.data_off + d.height * d.pitch].reshape(d.height, d.pitch)
             view[:, :d.width] = cm.get_data()
         pool_bytes, pool_words, pool_ctile_bytes, pool_sum_words = data_off, tile_off, ctile_off, sum_off
+        sum_init = np.zeros(max(pool_sum_words, 1), dtype=np.int32)     # tile summaries zero, trailer capacities set
+        sum_init[np.asarray(capacity_at, dtype=np.int64)] = capacities
         map_arena = self._to_device(arena)
         ids = self._map_ids_host
         if private_copies:
@@ -285,6 +294,7 @@ class VecPlanEnv(object):
             pool_words *= copies
             pool_ctile_bytes *= copies
             pool_sum_words *= copies
+            sum_init = np.tile(sum_init, copies)                     # every copy owns its trailers
         self._map_descs_host = descs
         self.map_arena = map_arena
         # TMA tensor maps for the egocentric kernel's source-window staging: three box-width classes
@@ -301,7 +311,8 @@ class VecPlanEnv(object):
         self.occ_tile_arena = torch.zeros(max(pool_words, 1), dtype=torch.int32, device=self.device)
         if pool_sum_words >= 2 ** 31:
             raise ValueError("tile summaries of this batch exceed the 32-bit offsets of BcgMapDesc.sum_off")
-        self.occ_sum_arena = torch.zeros(max(pool_sum_words, 1), dtype=torch.int32, device=self.device)
+        self.occ_sum_arena = self._to_device(sum_init)
+        self._cell_index_trailers = True
         if self.ego_staging == 'tma':
             nat.check(nat.lib().bcg_encode_map_tensor_maps(descs, len(descs), C.c_void_p(map_arena.data_ptr()), widths,
                                                            len(self._tmap_widths), self._tmap_box_h,
@@ -426,6 +437,8 @@ class VecPlanEnv(object):
         # loads every tile under the footprint)
         if os.environ.get("BCG_EGO_SUMMARY", "1") != "0":
             b.occ_sum_arena = self.occ_sum_arena.data_ptr()
+            if getattr(self, '_cell_index_trailers', False):
+                b.flags |= nat.BATCH_CELL_INDEX
         self._ego_list = None
         if self.cell_tile_arena is not None and getattr(self, '_ego_sparse', True):
             self._ego_list = torch.zeros(self.n_envs + 4, dtype=torch.int32, device=self.device)

@@ -118,6 +118,8 @@ typedef struct BcgParams {
  * rows, tile (ty, tx) at cell_tile_off + (ty * ctiles_x + tx) * 128, row r of a tile at + r * 16, zero
  * beyond the map; the egocentric kernel fetches whole HBM lines of a rotated window from it) */
 #define BCG_MAP_ONLY_LETHAL 1
+#define BCG_MAP_CELL_INDEX 4  /* the map's cell index (see BCG_BATCH_CELL_INDEX) is exact; set by bcg_build_lethal_tiles,
+                                 callers leave it clear */
 typedef struct BcgMapDesc {
   int64_t data_off;  /* byte offset of uint8 [H][pitch] in the map arena                      */
   int64_t tile_off;  /* uint32 offset of the lethal tile plane in the tile arena               */
@@ -168,6 +170,18 @@ typedef struct BcgFootprintLut {
                                        host after bcg_build_lethal_tiles; always true for device-generated worlds): the
                                        sparse egocentric kernel renders the rare window that overflows its cell list
                                        itself and the dense kernel is not launched behind it */
+#define BCG_BATCH_CELL_INDEX 2      /* the host reserved a cell-index trailer after the tile summary of every map that is
+                                       not dense (occupied * 20 <= width * height): at uint32 offset
+                                       sum_off + tiles_y * ((tiles_x + 31) / 32) of occ_sum_arena,
+                                         [0] capacity (cells; written by the host), [1] total (cells),
+                                         [2 .. 2 + tiles_y * tiles_x] prefix: exclusive counts of occupied cells per 32 x 16
+                                             tile of the occupancy plane in row-major tile order (tiles_y * tiles_x + 1 words),
+                                         then `capacity` words of cells: every occupied cell as x | y << 16 in map pixels,
+                                             grouped by tile in that order, row-major inside a tile.
+                                       bcg_build_lethal_tiles fills them and sets BCG_MAP_CELL_INDEX on the maps whose cells
+                                       fit; the sparse egocentric kernel then reads a window's cells from there instead of
+                                       listing them from the occupancy plane.  Without this bit no trailer is read or
+                                       written (tile summaries may be packed tightly). */
 
 /* everything a step touches; all pointers are device pointers */
 typedef struct BcgBatch {
@@ -213,8 +227,9 @@ typedef struct BcgBatch {
                             for the sparse path, handed to the dense cell-tile kernel (count at [n_envs]; [n_envs + 1] is
                             the sparse kernel's env counter)                                                 */
   const uint32_t* occ_sum_arena; /* optional: one bit per tile of the occupancy plane (BcgMapDesc.sum_off), filled by
-                            bcg_build_lethal_tiles and kept by the generators; must start out zero.  With it the sparse
-                            egocentric kernel loads only the non-empty tiles of a window                              */
+                            bcg_build_lethal_tiles and kept by the generators; must start out zero (but for the capacity
+                            words of BCG_BATCH_CELL_INDEX trailers).  With it the sparse egocentric kernel loads only
+                            the non-empty tiles of a window, or with a cell index only the window's cells              */
   uint32_t* status; /* [BCG_STATUS_WORDS] */
   double* stats;    /* [BCG_STATS_WORDS]  */
   uint64_t* step_counter; /* optional device [2], zero at start: when set, bcg_step ignores its step_index argument,
