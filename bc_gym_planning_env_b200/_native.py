@@ -117,8 +117,17 @@ class BcgEnvRows(C.Structure):
     _fields_ = [("f", C.c_void_p), ("i", C.c_void_p)]
 
 
+class BcgEpisodeEnds(C.Structure):
+    _fields_ = [
+        ("reason", C.c_void_p), ("final_slot", C.c_void_p), ("final_obs_vec", C.c_void_p), ("final_goal_n_state", C.c_void_p),
+        ("final_return", C.c_void_p), ("final_length", C.c_void_p), ("final_ego_work", C.c_void_p),
+        ("final_ego_image", C.c_void_p), ("final_list", C.c_void_p), ("count", C.c_void_p),
+        ("capacity", C.c_int32), ("reserved", C.c_int32),
+    ]
+
+
 _STRUCTS = [BcgParams, BcgMapDesc, BcgPathDesc, BcgFootprintLut, BcgBatch, BcgStateLayout, BcgStepOut, BcgTurnParams,
-            BcgAisleSlots, BcgMiniGenParams, BcgMiniParams, BcgEnvRows]
+            BcgAisleSlots, BcgMiniGenParams, BcgMiniParams, BcgEnvRows, BcgEpisodeEnds]
 
 # fixed rows / words of include/bcg_b200.h
 F_ROBOT, F_DROBOT, F_DPOSE, F_TIME, F_MIN_DIST, F_EP_RETURN, F_FIXED = 0, 7, 14, 17, 18, 19, 20
@@ -133,6 +142,8 @@ REWARD_CONTINUOUS, REWARD_PURE_PURSUIT = 0, 1
 # per-env parameter rows (BcgEnvRows)
 EP_F_SP, EP_F_AP, EP_F_PM, EP_F_ALPHA, EP_F_ROWS = 0, 1, 2, 3, 9
 EP_I_DELAY_CONTROL, EP_I_DELAY_POSE, EP_I_DELAY_STATE, EP_I_TIMEOUT, EP_I_NOISE_ON, EP_I_ROWS = 0, 1, 2, 3, 4, 5
+# episode-end reason bits (BcgEpisodeEnds.reason)
+END_GOAL, END_COLLIDED, END_TIMEOUT, END_NOW = 1, 2, 4, 8
 
 # every symbol include/bcg_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
@@ -161,6 +172,8 @@ SYMBOLS = {
                                   C.POINTER(BcgStepOut), C.POINTER(C.c_void_p), _P]),
     "bcg_step_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
                                 C.POINTER(BcgStepOut), C.POINTER(C.c_void_p), _P]),
+    "bcg_step_ends": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
+                                C.POINTER(BcgStepOut), C.POINTER(BcgEpisodeEnds), C.POINTER(C.c_void_p), _P]),
     "bcg_kinematic_step": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64, _P]),
     "bcg_collision": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, _P, _P, _P]),
     "bcg_collision_u8": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, _P, _P]),
@@ -178,6 +191,8 @@ SYMBOLS = {
     "bcg_rollout": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64, C.POINTER(BcgStepOut), _P]),
     "bcg_rollout_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
                                    C.POINTER(BcgStepOut), _P]),
+    "bcg_rollout_ends": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
+                                   C.POINTER(BcgStepOut), C.POINTER(BcgEpisodeEnds), _P]),
     "bcg_alloc_image_memory": (C.c_int, [C.c_int64, C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
     "bcg_free_image_memory": (C.c_int, [_P, C.c_int64]),
 }

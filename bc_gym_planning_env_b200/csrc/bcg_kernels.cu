@@ -687,11 +687,14 @@ __device__ __forceinline__ void write_goal_from_transform(const BcgParams& p, co
 // the env's other top-of-kernel loads, and the goal tolerances and the progress multiplier are forwarded to
 // reward_kernel at BCG_SR_ENV_OFF of the work slot.  (The copy is kept in the kernel body, not behind a function call:
 // that way the instantiation without rows compiles to the same instructions as before rows existed.)
-template <int MIN_BLOCKS, bool ROWS>
+// ENDS: the step reports episode ends (BcgEpisodeEnds, appended behind the other parameters so that their offsets, and
+// the instructions of the instantiation without it, stay as they were).  Its counters are zeroed here, after the wait:
+// the previous step's egocentric kernel reads them, and the caller reads them after this step.
+template <int MIN_BLOCKS, bool ROWS, bool ENDS>
 __global__ void __launch_bounds__(BCG_MOVE_THREADS, MIN_BLOCKS)
 move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, const void* __restrict__ actions,
             const int action_is_f64, const uint64_t step_index_arg, const BcgStepOut out, const int ego_cap,
-            const BcgEnvRows rows) {
+            const BcgEnvRows rows, int32_t* const ends_count) {
   pdl_wait();                                            // the previous step's kernels are done with the records and rows
   pdl_launch_next();
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -700,6 +703,7 @@ move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, c
   const int64_t N = b.n_envs;
   const uint64_t step_index = b.step_counter ? *reinterpret_cast<const volatile uint64_t*>(b.step_counter) : step_index_arg;
   if (e == 0 && b.ego_list) b.ego_list[N] = b.ego_list[N + 1] = 0;       // hand-over count, env counter of the sparse kernel
+  if (ENDS && e == 0) ends_count[0] = ends_count[1] = 0;                 // episode ends, their hand-over count
   double* const sf = b.state_f + e;
   int32_t* const si = b.state_i + e;
   // ---- everything that is read from rows (independent loads, issued together) ----------------------------------------
@@ -887,9 +891,11 @@ __device__ __forceinline__ void reset_env_rows(const BcgParams& p, const BcgBatc
 // wants few warps (the straight-line code is paid per warp), a small one a short chain (a chunk in one round).
 // ROWS: the batch has per-env parameters; env e's goal tolerances and progress multiplier come from its work slot, where
 // move_kernel left them (in the kernel body for the reason given at move_kernel)
-template <int G, bool ROWS>
+// ENDS: the step reports episode ends (BcgEpisodeEnds): the reason byte of every env and the final record of every env
+// whose episode ends now, taken before the auto-reset overwrites its rows and its egocentric record
+template <int G, bool ROWS, bool ENDS>
 __global__ void __launch_bounds__(BCG_REWARD_THREADS, BCG_REWARD_RESIDENT / BCG_REWARD_THREADS)
-reward_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStepOut out, const int ego_cap) {
+reward_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStepOut out, const int ego_cap, const BcgEpisodeEnds ends) {
   pdl_wait();                                            // move_kernel's records
   pdl_launch_next();
   const int e = (blockIdx.x * blockDim.x + threadIdx.x) / G;
@@ -965,6 +971,46 @@ reward_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStepOut out, c
         if (collided_after) atomicAdd(b.stats + BCG_STAT_COLLIDED, 1.0);
         if (goal) atomicAdd(b.stats + BCG_STAT_GOAL, 1.0);
         if (timed_out) atomicAdd(b.stats + BCG_STAT_TIMEOUT, 1.0);
+      }
+    }
+    if (ENDS && active) {
+      // (done, and with it `ended`, is uniform over the env's lane group)
+      const bool ended = done && !(rec.flags & BCG_SR_DONE_BEFORE);
+      int slot = -1;
+      if (gl == 0) {
+        const int causes = (goal ? BCG_END_GOAL : 0) | (collided_after ? BCG_END_COLLIDED : 0) | (timed_out ? BCG_END_TIMEOUT : 0);
+        ends.reason[e] = (uint8_t)((done ? causes : 0) | (ended ? BCG_END_NOW : 0));
+        if (ended) {
+          const int k = atomicAdd(ends.count, 1);
+          slot = k < ends.capacity ? k : -1;
+          // the observation as move_kernel left it in the rows (the obs_vec fields) and the post-step target
+          const double* const sf = b.state_f + e;
+          float4* const o = reinterpret_cast<float4*>(ends.final_obs_vec + (int64_t)e * 12);
+          o[0] = make_float4((float)sf[(BCG_F_DPOSE + 0) * N], (float)sf[(BCG_F_DPOSE + 1) * N], (float)sf[(BCG_F_DPOSE + 2) * N],
+                             (float)sf[(BCG_F_DROBOT + 0) * N]);
+          o[1] = make_float4((float)sf[(BCG_F_DROBOT + 1) * N], (float)sf[(BCG_F_DROBOT + 2) * N], (float)sf[(BCG_F_DROBOT + 3) * N],
+                             (float)sf[(BCG_F_DROBOT + 4) * N]);
+          o[2] = make_float4((float)sf[(BCG_F_DROBOT + 5) * N], (float)sf[(BCG_F_DROBOT + 6) * N], (float)sf[BCG_F_TIME * N], (float)target);
+          if (out.goal_n_state)
+            write_goal_from_transform(p, pd.P, pd.pitch, pd.n, target, rec.ct, rec.st, rec.tx, rec.ty, rec.tt, rec.drobot,
+                                      ends.final_goal_n_state + (int64_t)e * 9);
+          ends.final_return[e] = ep_return;
+          ends.final_length[e] = rec.iter_after;
+        }
+        ends.final_slot[e] = slot;
+      }
+      if (ended) {
+        const unsigned gmask = (0xffffffffu >> (32 - G)) << (lane & ~(unsigned)(G - 1));
+        if (out.ego_image) {
+          // the env's egocentric record, 16 bytes per lane, into its slot
+          slot = __shfl_sync(gmask, slot, (int)(lane & ~(unsigned)(G - 1)));
+          if (slot >= 0) {
+            const uint4* const src = reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(b.ego_work) + (int64_t)e * BCG_EGO_WORK_BYTES);
+            uint4* const dst = reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(ends.final_ego_work) + (int64_t)slot * BCG_EGO_WORK_BYTES);
+            for (int k = gl; k < BCG_EGO_WORK_BYTES / 16; k += G) dst[k] = src[k];
+          }
+        }
+        __syncwarp(gmask);                               // the record and the rows are read before the reset rewrites them
       }
     }
     if (active && done && p.auto_reset) {
@@ -1724,11 +1770,14 @@ __device__ __forceinline__ void sts_v4(uint32_t addr, const uint4& v) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
 
-template <int NG>
+// ENDS: after its envs the kernel renders the final crops of the step's episode ends (BcgEpisodeEnds): with env_list the
+// slots the sparse kernel handed over (final_list[0 .. count[1] - 1]), without it every slot in use
+template <int NG, bool ENDS>
 __global__ void __launch_bounds__(BCG_EGT_THREADS, BCG_EGT_CTAS) ego_tiles_kernel(const BcgParams p, const BcgBatch b,
                                                                                   uint8_t* __restrict__ image,
                                                                                   const int win_bytes,
-                                                                                  const int* __restrict__ env_list) {
+                                                                                  const int* __restrict__ env_list,
+                                                                                  const BcgEpisodeEnds ends) {
   extern __shared__ __align__(128) uint8_t egt_smem[];
   constexpr int NT = BCG_EGT_THREADS, NW = NT / 32;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -1737,16 +1786,23 @@ __global__ void __launch_bounds__(BCG_EGT_THREADS, BCG_EGT_CTAS) ego_tiles_kerne
   const uint32_t win_u32 = smem_u32(egt_smem), rec_u32 = smem_u32(rec_s);
   const uint8_t* const recs = reinterpret_cast<const uint8_t*>(b.ego_work);
   // env_list (optional): render only the envs env_list[0 .. env_list[n_envs] - 1] (what the sparse kernel left over)
-  const int n = env_list ? env_list[b.n_envs] : b.n_envs, G = gridDim.x;
+  const int n_env_items = env_list ? env_list[b.n_envs] : b.n_envs, G = gridDim.x;
+  // items n_env_items .. n - 1 are final crops
+  const int n = ENDS ? n_env_items + (env_list ? ends.count[1] : min(ends.count[0], ends.capacity)) : n_env_items;
   const int ego_w = p.ego_w, ego_h = p.ego_h, npx = ego_w * ego_h;
   const int e0 = blockIdx.x;
   if (e0 >= n) return;
   auto env_of = [&](int i) { return env_list ? env_list[i] : i; };
+  auto slot_of = [&](int i) { return env_list ? ends.final_list[i - n_env_items] : i - n_env_items; };
 
-  // record of env `en` -> ring slot `slot` (the first 16 threads move 16 bytes each)
+  // record of item `en` -> ring slot `slot` (the first 16 threads move 16 bytes each)
   auto fetch_record = [&](int en, int slot) {
-    if (en < n && tid < BCG_EGO_WORK_BYTES / 16)
-      cp_async_16(rec_u32 + slot * BCG_EGO_WORK_BYTES + tid * 16, recs + (int64_t)env_of(en) * BCG_EGO_WORK_BYTES + tid * 16, 16u);
+    if (en < n && tid < BCG_EGO_WORK_BYTES / 16) {
+      const uint8_t* const src = ENDS && en >= n_env_items
+                                     ? reinterpret_cast<const uint8_t*>(ends.final_ego_work) + (int64_t)slot_of(en) * BCG_EGO_WORK_BYTES
+                                     : recs + (int64_t)env_of(en) * BCG_EGO_WORK_BYTES;
+      cp_async_16(rec_u32 + slot * BCG_EGO_WORK_BYTES + tid * 16, src + tid * 16, 16u);
+    }
   };
 
   // The newest record fetch may still be in flight after a wait, so records are fetched RD envs ahead.
@@ -1822,7 +1878,7 @@ __global__ void __launch_bounds__(BCG_EGT_THREADS, BCG_EGT_CTAS) ego_tiles_kerne
     const int map_id = r->map_id;
     cp_async_wait_group_1();                  // the record needed next iteration has landed (the newest may not have)
     __syncthreads();                          // window, tables and that record are visible to every warp
-    uint8_t* const dst = image + (int64_t)env_of(e) * npx;
+    uint8_t* const dst = ENDS && e >= n_env_items ? ends.final_ego_image + (int64_t)slot_of(e) * npx : image + (int64_t)env_of(e) * npx;
     if (mode == BCG_EGO_MODE_TILES) {
       // ---- gather: warp w takes crop rows w, w + 8, ...; lane l takes columns l, l + 32, ...  (NG = ceil(ego_w / 32):
       // only the last column group can be partial) -----------------------------------------------------------------
@@ -1959,12 +2015,16 @@ __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.comm
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-template <bool SUM, bool HITS>
+// ENDS: items n_envs .. n_envs + min(count[0], capacity) - 1 are the final crops of the step's episode ends
+// (BcgEpisodeEnds): item n_envs + s renders the record final_ego_work[s] into final_ego_image[s], hands slot s over to the
+// dense kernel through final_list, and records no compact hit list
+template <bool SUM, bool HITS, bool ENDS>
 __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kernel(const BcgParams p, const BcgBatch b,
                                                                                    uint8_t* __restrict__ image,
                                                                                    uint32_t* __restrict__ hit_list,
                                                                                    int32_t* __restrict__ hit_count,
-                                                                                   const int hit_cap, const int evict_from) {
+                                                                                   const int hit_cap, const int evict_from,
+                                                                                   const BcgEpisodeEnds ends) {
   constexpr int NT = BCG_EGS_THREADS;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   // All static shared memory is ONE struct, and its shared-window address is kept in one register (the empty asm hides
@@ -2004,10 +2064,14 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
   const int ego_w = p.ego_w, ego_h = p.ego_h, npx = ego_w * ego_h;
   const int e0 = blockIdx.x;
   if (e0 >= n) return;
+  int n_items = n;                              // + the final crops (ENDS), counted by reward_kernel: set after the wait
 
   auto fetch_record = [&](int en, int slot) {
-    if (en < n && tid < BCG_EGO_WORK_BYTES / 16)
-      cp_async_16(rec_u32 + slot * BCG_EGO_WORK_BYTES + tid * 16, recs + (int64_t)en * BCG_EGO_WORK_BYTES + tid * 16, 16u);
+    if (en < n_items && tid < BCG_EGO_WORK_BYTES / 16) {
+      const uint8_t* const src = ENDS && en >= n ? reinterpret_cast<const uint8_t*>(ends.final_ego_work) + (int64_t)(en - n) * BCG_EGO_WORK_BYTES
+                                                 : recs + (int64_t)en * BCG_EGO_WORK_BYTES;
+      cp_async_16(rec_u32 + slot * BCG_EGO_WORK_BYTES + tid * 16, src + tid * 16, 16u);
+    }
   };
   const bool cix_batch = SUM && (b.flags & BCG_BATCH_CELL_INDEX) != 0;
   // Tile-summary words of the window of record `q`, lane <-> band of 16 rows (zero where the band or the word lies
@@ -2040,6 +2104,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
   if (tid < 2) T.count[tid] = T.hits[tid] = 0;
   pdl_wait();                                 // the records (and, on a reset, the state) are reward_kernel's
   pdl_launch_next();
+  if (ENDS) n_items = n + min(ends.count[0], ends.capacity);
 #pragma unroll
   for (int k = 0; k < RD; ++k) fetch_record(e0 + k * G, k);
   cp_async_commit();
@@ -2068,7 +2133,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
 #if BCG_EGS_DYNAMIC
   for (int it = 0;; ++it) {
     const int e = ids_s[it & 7];
-    if (e >= n) break;
+    if (e >= n_items) break;
     int drawn = 0;
     if (tid == 0) drawn = (RD + 1) * G + atomicAdd(b.ego_list + n + 1, 1);       // stored at the end of the iteration
     const int slot = it & (BCG_EGS_REC_SLOTS - 1), par = it & 1;
@@ -2077,7 +2142,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     const int e_next = ids_s[(it + 1) & 7];
 #else
   int e = e0;
-  for (int it = 0; e < n; e += G, ++it) {
+  for (int it = 0; e < n_items; e += G, ++it) {
     const int slot = it & (BCG_EGS_REC_SLOTS - 1), par = it & 1;
     fetch_record(e + RD * G, (it + RD) & (BCG_EGS_REC_SLOTS - 1));
     cp_async_commit();
@@ -2085,12 +2150,13 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
 #endif
     // record it + 1 has landed (only the newest fetch may still be in flight): start its summary loads now
     const uint32_t cur_lo = pf_lo, cur_hi = pf_hi;
-    if (SUM && e_next < n)
+    if (SUM && e_next < n_items)
       summary_words(reinterpret_cast<const EgoTileWork*>(rec_s + ((it + 1) & (BCG_EGS_REC_SLOTS - 1)) * BCG_EGO_WORK_BYTES), pf_lo, pf_hi, true);
-    if (e_next < n) make_spans((it + 1) & (BCG_EGS_REC_SLOTS - 1), (it + 1) & 1);
+    if (e_next < n_items) make_spans((it + 1) & (BCG_EGS_REC_SLOTS - 1), (it + 1) & 1);
     const EgoTileWork* r = reinterpret_cast<const EgoTileWork*>(rec_s + slot * BCG_EGO_WORK_BYTES);
     const int mode = r->mode, X0 = r->X0, Y0 = r->Y0, ntx = r->ntx, nty = r->nty;
-    uint8_t* const dst = image + (int64_t)e * npx;
+    const bool final_crop = ENDS && e >= n;             // a final crop: no compact hit list, its own image and hand-over
+    uint8_t* const dst = final_crop ? ends.final_ego_image + (int64_t)(e - n) * npx : image + (int64_t)e * npx;
     const int wx0 = X0 >> 5, nwx = ((X0 + 16 * ntx - 1) >> 5) - wx0 + 1;        // <= 9 columns of 32-cell words
     const int by0 = Y0 >> 4, nby = ((Y0 + 8 * nty - 1) >> 4) - by0 + 1;         // bands of 16 rows
     const int ntile = nby * nwx;
@@ -2366,7 +2432,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
 #ifdef BCG_EGS_EXP_NO_HITS
         }
 #endif
-        if (HITS) {
+        if (HITS && !final_crop) {
           // compact observation (BcgStepOut.ego_hits): pixel offset | value << 16 of every non-zero crop pixel.  A crop
           // pixel samples exactly one cell and the four candidates of a cell are distinct pixels: no duplicates.
           const int nh = (int)h00 + (int)h10 + (int)h01 + (int)h11;
@@ -2437,15 +2503,17 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
         if (X >= 0 && X < mw && Y >= 0 && Y < mh) val = __ldg(src + Y * mpitch + X);
         dst[i] = val;
       }
+    } else if (final_crop) {
+      if (tid == 0) ends.final_list[atomicAdd(ends.count + 1, 1)] = e - n;
     } else if (tid == 0) {
       const int at = atomicAdd(b.ego_list + n, 1);
       b.ego_list[at] = e;
     }
     if (tid == 0) T.count[par ^ 1] = 0;         // nobody reads the other counter before the next barrier
     if (HITS) {                                 // (the hit counter of this env is complete after the barrier below)
-      if (!sparse && tid == 0) hit_count[e] = -1;       // rendered densely: the consumer reads the image itself
+      if (!sparse && tid == 0 && !final_crop) hit_count[e] = -1;       // rendered densely: the consumer reads the image itself
       __syncthreads();
-      if (sparse && tid == 0) hit_count[e] = (int32_t)T.hits[par];      // > hit_cap: the list overflowed, read the image
+      if (sparse && tid == 0 && !final_crop) hit_count[e] = (int32_t)T.hits[par];      // > hit_cap: the list overflowed, read the image
       if (tid == 0) T.hits[par ^ 1] = 0;
     }
 #if BCG_EGS_DYNAMIC
@@ -2636,6 +2704,7 @@ int64_t bcg_sizeof(int32_t which) {
     case 9: return sizeof(BcgMiniGenParams);
     case 10: return sizeof(BcgMiniParams);
     case 11: return sizeof(BcgEnvRows);
+    case 12: return sizeof(BcgEpisodeEnds);
     default: return -1;
   }
 }
@@ -2910,33 +2979,43 @@ static int sm_count_of_current_device(int* out) {
   return BCG_OK;
 }
 
-template <int NG>
-static int launch_ego_tiles(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const int* env_list, cudaStream_t s) {
+template <int NG, bool ENDS>
+static int launch_ego_tiles(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const int* env_list, const BcgEpisodeEnds& ends,
+                            cudaStream_t s) {
   const int win = ego_window_capacity(*p);
   const int smem = win + (int)sizeof(EgoTab) + BCG_EGT_REC_SLOTS * BCG_EGO_WORK_BYTES;
   static int configured[64] = {0};    // per template instance and device: the attribute is per function and context
   int dev = 0;
   BCG_CHECK_CUDA(cudaGetDevice(&dev));
   if (dev < 0 || dev >= 64 || configured[dev] < smem) {
-    BCG_CHECK_CUDA(cudaFuncSetAttribute(ego_tiles_kernel<NG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    BCG_CHECK_CUDA(cudaFuncSetAttribute(ego_tiles_kernel<NG, ENDS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     if (dev >= 0 && dev < 64) configured[dev] = smem;
   }
   int sms = 0;
   if (int rc = sm_count_of_current_device(&sms)) return rc;
   const int grid = b->n_envs < BCG_EGT_CTAS * sms ? b->n_envs : BCG_EGT_CTAS * sms;
-  ego_tiles_kernel<NG><<<grid, BCG_EGT_THREADS, smem, s>>>(*p, *b, ego_image, win, env_list);
+  ego_tiles_kernel<NG, ENDS><<<grid, BCG_EGT_THREADS, smem, s>>>(*p, *b, ego_image, win, env_list, ends);
   BCG_CHECK_CUDA(cudaGetLastError());
   return BCG_OK;
 }
 
-static int launch_ego_dense(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const int* env_list, cudaStream_t s) {
+template <bool ENDS>
+static int launch_ego_dense(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const int* env_list, const BcgEpisodeEnds& ends,
+                            cudaStream_t s) {
   switch ((p->ego_w + 31) / 32) {
-    case 1: return launch_ego_tiles<1>(p, b, ego_image, env_list, s);
-    case 2: return launch_ego_tiles<2>(p, b, ego_image, env_list, s);
-    case 3: return launch_ego_tiles<3>(p, b, ego_image, env_list, s);
-    case 4: return launch_ego_tiles<4>(p, b, ego_image, env_list, s);
-    default: return launch_ego_tiles<5>(p, b, ego_image, env_list, s);
+    case 1: return launch_ego_tiles<1, ENDS>(p, b, ego_image, env_list, ends, s);
+    case 2: return launch_ego_tiles<2, ENDS>(p, b, ego_image, env_list, ends, s);
+    case 3: return launch_ego_tiles<3, ENDS>(p, b, ego_image, env_list, ends, s);
+    case 4: return launch_ego_tiles<4, ENDS>(p, b, ego_image, env_list, ends, s);
+    default: return launch_ego_tiles<5, ENDS>(p, b, ego_image, env_list, ends, s);
   }
+}
+
+// the dense kernel, with the final crops of `ends` (may be NULL) behind the envs
+static int launch_ego_dense(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const int* env_list, const BcgEpisodeEnds* ends,
+                            cudaStream_t s) {
+  if (ends) return launch_ego_dense<true>(p, b, ego_image, env_list, *ends, s);
+  return launch_ego_dense<false>(p, b, ego_image, env_list, BcgEpisodeEnds{}, s);
 }
 
 // sparse scatter kernel for every env, then the dense kernel for the envs it handed over (usually none)
@@ -2947,7 +3026,8 @@ struct EgoHits {       // BcgStepOut.ego_hits / ego_hit_count / ego_hit_cap (all
   bool pdl;            // launch the sparse kernel as a programmatic dependent of the kernel before it (the step path)
 };
 
-static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const EgoHits& hits, cudaStream_t s) {
+static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const EgoHits& hits, const BcgEpisodeEnds* ends,
+                             cudaStream_t s) {
   int sms = 0;
   if (int rc = sm_count_of_current_device(&sms)) return rc;
   // (the hand-over count and the env counter in ego_list[n_envs ..] were zeroed by the state / prep kernel)
@@ -2961,8 +3041,8 @@ static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego
   if (dev >= 0 && dev < 64 && per_sm_cache[sum][dev] > 0 && tab_cache[sum][dev] == tab_bytes) {
     per_sm = per_sm_cache[sum][dev];
   } else {
-    if (sum) BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ego_sparse_kernel<true, false>, BCG_EGS_THREADS, tab_bytes));
-    else BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ego_sparse_kernel<false, false>, BCG_EGS_THREADS, tab_bytes));
+    if (sum) BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ego_sparse_kernel<true, false, false>, BCG_EGS_THREADS, tab_bytes));
+    else BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ego_sparse_kernel<false, false, false>, BCG_EGS_THREADS, tab_bytes));
     BCG_REQUIRE(per_sm > 0, "the sparse egocentric kernel does not fit an SM with this crop size");
     if (dev >= 0 && dev < 64) {
       per_sm_cache[sum][dev] = per_sm;
@@ -2983,16 +3063,32 @@ static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego
   const int evict = (long long)b->n_envs * p->ego_w * p->ego_h <= evict_bytes ? 0 : b->n_envs;   // evict_from: envs >= it use the policy
   uint32_t* const no_list = nullptr;
   int32_t* const no_count = nullptr;
+  // (the final crops of episode ends, when asked for, are the items behind the envs)
+  const BcgEpisodeEnds en = ends ? *ends : BcgEpisodeEnds{};
+#define BCG_EGS_LAUNCH(SUM, HITS, ENDS, LIST, COUNT, CAP) \
+  BCG_CHECK_CUDA(launch_step_kernel(ego_sparse_kernel<SUM, HITS, ENDS>, grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b, ego_image, \
+                                    LIST, COUNT, CAP, evict, en))
   if (hits.list) {
-    if (sum) BCG_CHECK_CUDA(launch_step_kernel(ego_sparse_kernel<true, true>, grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b, ego_image, hits.list, hits.count, hits.cap, evict));
-    else BCG_CHECK_CUDA(launch_step_kernel(ego_sparse_kernel<false, true>, grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b, ego_image, hits.list, hits.count, hits.cap, evict));
+    if (ends) {
+      if (sum) BCG_EGS_LAUNCH(true, true, true, hits.list, hits.count, hits.cap);
+      else BCG_EGS_LAUNCH(false, true, true, hits.list, hits.count, hits.cap);
+    } else {
+      if (sum) BCG_EGS_LAUNCH(true, true, false, hits.list, hits.count, hits.cap);
+      else BCG_EGS_LAUNCH(false, true, false, hits.list, hits.count, hits.cap);
+    }
   } else {
-    if (sum) BCG_CHECK_CUDA(launch_step_kernel(ego_sparse_kernel<true, false>, grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b, ego_image, no_list, no_count, 0, evict));
-    else BCG_CHECK_CUDA(launch_step_kernel(ego_sparse_kernel<false, false>, grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b, ego_image, no_list, no_count, 0, evict));
+    if (ends) {
+      if (sum) BCG_EGS_LAUNCH(true, false, true, no_list, no_count, 0);
+      else BCG_EGS_LAUNCH(false, false, true, no_list, no_count, 0);
+    } else {
+      if (sum) BCG_EGS_LAUNCH(true, false, false, no_list, no_count, 0);
+      else BCG_EGS_LAUNCH(false, false, false, no_list, no_count, 0);
+    }
   }
+#undef BCG_EGS_LAUNCH
   BCG_CHECK_CUDA(cudaGetLastError());
   if (b->flags & BCG_BATCH_SPARSE_EGO_ONLY) return BCG_OK;     // the sparse kernel rendered every env itself
-  return launch_ego_dense(p, b, ego_image, b->ego_list, s);
+  return launch_ego_dense(p, b, ego_image, b->ego_list, ends, s);
 }
 
 // BCG_EGO_KERNEL=dense forces the dense cell-tile kernel for every env (A/B timing of the sparse path)
@@ -3004,14 +3100,17 @@ static bool ego_dense_kernel_requested() {
   return dense;
 }
 
-// the image kernel(s); the per-env records must already be in b->ego_work
-static int launch_ego_image(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const EgoHits& hits, cudaStream_t s) {
+// the image kernel(s); the per-env records must already be in b->ego_work (and those of the final crops of `ends`, which
+// may be NULL, in ends->final_ego_work)
+static int launch_ego_image(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const EgoHits& hits, const BcgEpisodeEnds* ends,
+                            cudaStream_t s) {
   if (b->cell_tile_arena) {
-    if (b->occ_tile_arena && b->ego_list && !ego_dense_kernel_requested()) return launch_ego_sparse(p, b, ego_image, hits, s);
+    if (b->occ_tile_arena && b->ego_list && !ego_dense_kernel_requested()) return launch_ego_sparse(p, b, ego_image, hits, ends, s);
     BCG_REQUIRE(!hits.list, "the compact egocentric output (BcgStepOut.ego_hits) comes from the sparse kernel: ego_list is needed");
-    return launch_ego_dense(p, b, ego_image, nullptr, s);
+    return launch_ego_dense(p, b, ego_image, nullptr, ends, s);
   }
   BCG_REQUIRE(!hits.list, "the compact egocentric output (BcgStepOut.ego_hits) needs the cell-tile / occupancy planes");
+  BCG_REQUIRE(!ends, "final crops of episode ends need the cell-tile planes (BcgBatch.cell_tile_arena)");
   const int cap = ego_tile_capacity(*p, *b);
   // alignment slack + the per-row spans of the plain-load path, which live behind the tile
   const int extra = 128 + BCG_EGO_MAX_TILE_ROWS * (int)sizeof(short2);
@@ -3030,36 +3129,61 @@ int bcg_observe_ego(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, f
   ego_prep_kernel<<<blocks_for(b->n_envs, 128), 128, 0, s>>>(*p, *b, ego_image ? 1 : 0, goal_n_state,
                                                             ego_capacity(*p, *b));
   BCG_CHECK_CUDA(cudaGetLastError());
-  if (ego_image) return launch_ego_image(p, b, ego_image, EgoHits{nullptr, nullptr, 0, false}, s);
+  if (ego_image) return launch_ego_image(p, b, ego_image, EgoHits{nullptr, nullptr, 0, false}, nullptr, s);
   return BCG_OK;
 }
 
 }  // extern "C"
 
 // move_kernel of one step, at the register tier the batch size picks
-template <bool ROWS>
+template <bool ROWS, bool ENDS>
 static int launch_move_kernel(const BcgParams* p, const BcgBatch* b, const BcgEnvRows& rows, const BcgStateLayout& L,
                               const void* actions, int32_t action_is_f64, uint64_t step_index, const BcgStepOut* out,
-                              int cap, bool pdl, cudaStream_t s) {
+                              int32_t* ends_count, int cap, bool pdl, cudaStream_t s) {
   int sms = 0;
   if (int rc = sm_count_of_current_device(&sms)) return rc;
   const int move_blocks = (int)blocks_for(b->n_envs, BCG_MOVE_THREADS);
   if (move_blocks <= sms * BCG_MOVE_FEWER_BLOCKS)
-    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEWER_BLOCKS, ROWS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows));
+    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEWER_BLOCKS, ROWS, ENDS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows, ends_count));
   else if (move_blocks <= sms * BCG_MOVE_FEW_BLOCKS)
-    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEW_BLOCKS, ROWS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows));
+    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEW_BLOCKS, ROWS, ENDS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows, ends_count));
   else
-    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_MIN_BLOCKS, ROWS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows));
+    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_MIN_BLOCKS, ROWS, ENDS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows, ends_count));
   return BCG_OK;
 }
 
 // reward_kernel of one step, with the lane group the batch size picks
-template <bool ROWS>
-static int launch_reward_kernel(const BcgParams* p, const BcgBatch* b, const BcgStepOut* out, int cap, bool pdl_reward, cudaStream_t s) {
+template <bool ROWS, bool ENDS>
+static int launch_reward_kernel(const BcgParams* p, const BcgBatch* b, const BcgStepOut* out, const BcgEpisodeEnds& ends, int cap,
+                                bool pdl_reward, cudaStream_t s) {
   const int64_t ns = b->n_envs;
-  if (ns > 16384) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<8, ROWS>, blocks_for(ns * 8, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
-  else if (ns > 2048) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<16, ROWS>, blocks_for(ns * 16, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
-  else BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<32, ROWS>, blocks_for(ns * 32, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap));
+  if (ns > 16384) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<8, ROWS, ENDS>, blocks_for(ns * 8, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, ends));
+  else if (ns > 2048) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<16, ROWS, ENDS>, blocks_for(ns * 16, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, ends));
+  else BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<32, ROWS, ENDS>, blocks_for(ns * 32, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, ends));
+  return BCG_OK;
+}
+
+// the two state kernels of a step (events[2], when set, is recorded between them)
+template <bool ROWS, bool ENDS>
+static int launch_state_kernels(const BcgParams* p, const BcgBatch* b, const BcgEnvRows& rows, const BcgStateLayout& L,
+                                const void* actions, int32_t action_is_f64, uint64_t step_index, const BcgStepOut* out,
+                                const BcgEpisodeEnds& ends, void* const* events, int cap, bool pdl, bool pdl_reward, cudaStream_t s) {
+  if (int rc = launch_move_kernel<ROWS, ENDS>(p, b, rows, L, actions, action_is_f64, step_index, out, ends.count, cap, pdl, s)) return rc;
+  if (events && events[2]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[2], s));
+  return launch_reward_kernel<ROWS, ENDS>(p, b, out, ends, cap, pdl_reward, s);
+}
+
+static int check_ends(const BcgBatch* b, const BcgStepOut* out, const BcgEpisodeEnds* ends) {
+  if (!ends) return BCG_OK;
+  BCG_REQUIRE(ends->capacity >= 1, "BcgEpisodeEnds.capacity must be at least 1");
+  BCG_REQUIRE(ends->reason && ends->final_slot && ends->final_obs_vec && ends->final_return && ends->final_length && ends->count,
+              "BcgEpisodeEnds: reason, final_slot, final_obs_vec, final_return, final_length and count are needed");
+  if (out->goal_n_state) BCG_REQUIRE(ends->final_goal_n_state, "BcgEpisodeEnds.final_goal_n_state is needed with goal_n_state");
+  if (out->ego_image) {
+    BCG_REQUIRE(ends->final_ego_work && ends->final_ego_image && ends->final_list,
+                "BcgEpisodeEnds: final_ego_work, final_ego_image and final_list are needed with ego_image");
+    BCG_REQUIRE(b->cell_tile_arena, "final crops of episode ends need the cell-tile planes (BcgBatch.cell_tile_arena)");
+  }
   return BCG_OK;
 }
 
@@ -3067,14 +3191,20 @@ extern "C" {
 
 int bcg_step_events(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64,
                     uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream) {
-  return bcg_step_rows(p, b, nullptr, actions, action_is_f64, step_index, out, events, stream);
+  return bcg_step_ends(p, b, nullptr, actions, action_is_f64, step_index, out, nullptr, events, stream);
 }
 
 int bcg_step_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
                   uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream) {
+  return bcg_step_ends(p, b, rows, actions, action_is_f64, step_index, out, nullptr, events, stream);
+}
+
+int bcg_step_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
+                  uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* const* events, void* stream) {
   if (int rc = check_batch(p, b)) return rc;
   if (int rc = check_rows(rows)) return rc;
   BCG_REQUIRE(actions && out, "null actions/out");
+  if (int rc = check_ends(b, out, ends)) return rc;
   const bool ego = out->ego_image || out->goal_n_state;
   if (ego) {
     if (int rc = check_ego(p, b, out->ego_image)) return rc;
@@ -3088,22 +3218,23 @@ int bcg_step_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows,
     // (event records between the kernels are stream operations of their own: the timed form runs without the overlap)
     const bool pdl = !(events && (events[0] || events[1]));          // an event right before a kernel: no overlap for it
     const bool pdl_reward = !(events && events[2]);
-    if (rows) {
-      if (int rc = launch_move_kernel<true>(p, b, *rows, L, actions, action_is_f64, step_index, out, cap, pdl, s)) return rc;
-    } else {
-      if (int rc = launch_move_kernel<false>(p, b, BcgEnvRows{nullptr, nullptr}, L, actions, action_is_f64, step_index, out, cap, pdl, s))
-        return rc;
-    }
-    if (events && events[2]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[2], s));
-    if (int rc = rows ? launch_reward_kernel<true>(p, b, out, cap, pdl_reward, s) : launch_reward_kernel<false>(p, b, out, cap, pdl_reward, s))
-      return rc;
+    const BcgEnvRows r = rows ? *rows : BcgEnvRows{nullptr, nullptr};
+    const BcgEpisodeEnds en = ends ? *ends : BcgEpisodeEnds{};
+    int rc;
+    if (rows) rc = ends ? launch_state_kernels<true, true>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s)
+                        : launch_state_kernels<true, false>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s);
+    else rc = ends ? launch_state_kernels<false, true>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s)
+                   : launch_state_kernels<false, false>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s);
+    if (rc) return rc;
     BCG_CHECK_CUDA(cudaGetLastError());
   }
   if (events && events[3]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[3], s));
   if (out->ego_image) {
     BCG_REQUIRE((out->ego_hits != nullptr) == (out->ego_hit_count != nullptr) && (!out->ego_hits || out->ego_hit_cap > 0),
                 "ego_hits, ego_hit_count and ego_hit_cap go together");
-    if (int rc = launch_ego_image(p, b, out->ego_image, EgoHits{out->ego_hits, out->ego_hit_count, out->ego_hit_cap, !(events && events[3])}, s)) return rc;
+    if (int rc = launch_ego_image(p, b, out->ego_image, EgoHits{out->ego_hits, out->ego_hit_count, out->ego_hit_cap, !(events && events[3])},
+                                  ends, s))
+      return rc;
   }
   if (events && events[4]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[4], s));
   return BCG_OK;
@@ -3116,14 +3247,19 @@ int bcg_step(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t
 
 int bcg_rollout(const BcgParams* p, const BcgBatch* b, const float* plan, int32_t horizon, uint64_t step_index,
                 const BcgStepOut* out, void* stream) {
-  return bcg_rollout_rows(p, b, nullptr, plan, horizon, step_index, out, stream);
+  return bcg_rollout_ends(p, b, nullptr, plan, horizon, step_index, out, nullptr, stream);
 }
 
 int bcg_rollout_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
                      uint64_t step_index, const BcgStepOut* out, void* stream) {
+  return bcg_rollout_ends(p, b, rows, plan, horizon, step_index, out, nullptr, stream);
+}
+
+int bcg_rollout_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
+                     uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* stream) {
   BCG_REQUIRE(plan && horizon >= 0, "null plan / negative horizon");
   for (int32_t h = 0; h < horizon; ++h)
-    if (int rc = bcg_step_rows(p, b, rows, plan + (int64_t)h * b->n_envs * 2, 0, step_index + (uint64_t)h, out, nullptr, stream))
+    if (int rc = bcg_step_ends(p, b, rows, plan + (int64_t)h * b->n_envs * 2, 0, step_index + (uint64_t)h, out, ends, nullptr, stream))
       return rc;
   return BCG_OK;
 }

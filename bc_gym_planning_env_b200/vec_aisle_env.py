@@ -64,9 +64,10 @@ class _VecSlotEnv(VecPlanEnv):
     cell-tile, tile-plane and path arenas, and host accessors that read a world back."""
 
     def _setup_slots(self, params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
-                     footprint_scale, footprint, map_cells, path_points, record_bytes, params_ids=None):
+                     footprint_scale, footprint, map_cells, path_points, record_bytes, params_ids=None, episode_ends=False,
+                     episode_end_capacity=None):
         self._configure(params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego, 'tiles',
-                        params_ids)
+                        params_ids, episode_ends, episode_end_capacity)
         if not self.params.refine_path:
             raise ValueError("device-side generation always refines the path (EnvParams.refine_path)")
         if max(1, int(0.05 / self.resolution)) != 1:
@@ -153,7 +154,7 @@ class VecRandomAisleTurnEnv(_VecSlotEnv):
     def __init__(self, n_envs, params=None, draw_new_turn_on_reset=True, seed=0, turn_params=None,
                  noise_parameters=DEFAULT_NOISE, auto_reset=False, device=None, env_id_base=0, with_ego=False,
                  footprint_scale=1.0, footprint=None, resolution=0.03, max_map_cells=None, max_path_points=None,
-                 params_ids=None):
+                 params_ids=None, episode_ends=False, episode_end_capacity=None):
         """
         :param n_envs: batch size; env e draws from the Philox stream (seed; env_id_base + e, draw index)
         :param params, noise_parameters, params_ids: one EnvParams and noise setting for the batch, or a pool of them
@@ -166,6 +167,8 @@ class VecRandomAisleTurnEnv(_VecSlotEnv):
             one generation launch for the envs that finished.
         :param turn_params: optional list of n_envs TurnParams for the first worlds (default: drawn on device)
         :param max_map_cells, max_path_points: slot capacities per env (default: worst case of the distribution)
+        :param episode_ends, episode_end_capacity: see VecPlanEnv.  With auto_reset, `reset(done)` after a step gives the
+            envs that finished a new turn; their final observations (`final_observation()`) are those of the old one
         """
         from bc_gym_planning_env_b200.envs.base.params import EnvParams
         first = params[0] if envp.is_pool(params) and len(params) else params
@@ -174,7 +177,8 @@ class VecRandomAisleTurnEnv(_VecSlotEnv):
         self._draw_new_turn_on_reset = bool(draw_new_turn_on_reset)
         self._setup_slots(params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
                           footprint_scale, footprint, max_map_cells if max_map_cells is not None else cells,
-                          max_path_points if max_path_points is not None else points, TURN_DTYPE.itemsize, params_ids)
+                          max_path_points if max_path_points is not None else points, TURN_DTYPE.itemsize, params_ids,
+                          episode_ends, episode_end_capacity)
         self._turns = self._records
         self._slots.params_out = self._turns.data_ptr()
         self.generate(turn_params=turn_params)
@@ -272,7 +276,7 @@ class VecRandomMiniEnv(_VecSlotEnv):
 
     def __init__(self, n_envs, params=None, draw_new_turn_on_reset=True, seed=0, mini_params=None,
                  noise_parameters=DEFAULT_NOISE, auto_reset=False, device=None, env_id_base=0, with_ego=False,
-                 footprint_scale=1.0, footprint=None):
+                 footprint_scale=1.0, footprint=None, episode_ends=False, episode_end_capacity=None):
         """
         :param params RandomMiniEnvParams: the sampling space and its EnvParams (default: RandomMiniEnv's own,
             goal tolerances 0.2 m / pi/8)
@@ -281,6 +285,7 @@ class VecRandomMiniEnv(_VecSlotEnv):
         :param auto_reset: in-kernel reset to the initial state of the env's CURRENT world; it never samples a new
             world (see VecRandomAisleTurnEnv).  The reference builds a new env per episode (mini_env.py:447-470):
             auto_reset=False + `env.reset(done)` does that here.
+        :param episode_ends, episode_end_capacity: see VecPlanEnv
         """
         from bc_gym_planning_env_b200.envs.base.params import EnvParams
         from bc_gym_planning_env_b200.envs.mini_env import RandomMiniEnvParams
@@ -303,7 +308,8 @@ class VecRandomMiniEnv(_VecSlotEnv):
         side_x, side_y = int(round(h / ep.resolution)) + 33, int(round(w / ep.resolution)) + 9
         diag = np.hypot(params.inner_w + 2 * params.mid_margin, params.inner_h + 2 * params.mid_margin)
         self._setup_slots(ep, n_envs, ep.resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
-                          footprint_scale, footprint, side_x * side_y, int(np.ceil(diag / ep.path_delta)) + 8, MINI_DTYPE.itemsize)
+                          footprint_scale, footprint, side_x * side_y, int(np.ceil(diag / ep.path_delta)) + 8, MINI_DTYPE.itemsize,
+                          episode_ends=episode_ends, episode_end_capacity=episode_end_capacity)
         self.generate(mini_params=mini_params)
         self.check_status()
 

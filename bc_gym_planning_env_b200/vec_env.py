@@ -77,6 +77,24 @@ class VecObservation(object):
         return self._env.costmap(e)
 
 
+class FinalObservation(object):
+    """What the episodes that ended at the last step looked like at their end, before the auto-reset (device tensors,
+    reused buffers that the next step overwrites; nothing here synchronises).  Rows are indexed by env and valid where
+    `ended` is true:
+      ended           bool [N]          the episode of env e ended at the last step
+      obs_vec         float32 [N, 12]   the compact observation (delayed pose, delayed robot state, time, target index)
+      goal_n_state    float32 [N, 9, 1] with the egocentric observation, else None
+      episode_return  float64 [N]       the episode's return, this step's reward included
+      episode_length  int32 [N]         its iterations
+      slot            int32 [N]         env e's row of ego_image, -1 when it did not end or found no free slot
+      ego_image       uint8 [capacity, H, W, 1] final crops by slot (with the egocentric observation, else None)
+      count           int32 scalar      episodes that ended at the last step; more than `capacity` means that some ended
+                                        envs (which ones is unspecified) have no crop: see VecPlanEnv.final_ego"""
+
+    def __init__(self, **fields):
+        self.__dict__.update(fields)
+
+
 class VecState(object):
     """Snapshot of k env columns (reference `State`, envs/base/env.py:52-68): fp64 rows [F, k] and
     int32 rows [I, k].  Costmaps and paths are immutable per env, so a snapshot holds no copy of them."""
@@ -92,7 +110,8 @@ class VecPlanEnv(object):
     def __init__(self, costmaps, paths, params=None, n_envs=None, map_ids=None, path_ids=None,
                  noise_parameters=DEFAULT_NOISE, seed=0, auto_reset=False, device=None, env_id_base=0,
                  private_map_copies=False, with_ego=False, footprint_scale=1.0, use_tma=True, footprint=None,
-                 ego_staging='tiles', ego_sparse=True, compact_ego=False, params_ids=None):
+                 ego_staging='tiles', ego_sparse=True, compact_ego=False, params_ids=None, episode_ends=False,
+                 episode_end_capacity=None):
         """
         :param costmaps: pool of CostMap2D (uint8), one resolution
         :param paths: pool of oriented paths, array(n, 3); refined here when params.refine_path
@@ -114,6 +133,11 @@ class VecPlanEnv(object):
             `step_host(images='compact')` sends to the host instead of whole crops (needs with_ego and the sparse kernel)
         :param ego_sparse: with 'tiles' staging, render crops with the sparse scatter kernel (occupancy plane; the dense
             cell-tile kernel only takes the envs it hands over).  False: the dense kernel renders every env
+        :param episode_ends: report every step why envs are done (`terminated`, `truncated`, `episode_reason`) and keep
+            the final observation of every episode that ends (`final_observation()`), also when `auto_reset` has already
+            replaced it.  Computed in the step's own kernels (no extra launch); with the egocentric observation it needs
+            ego_staging='tiles'
+        :param episode_end_capacity: final crops kept per step (default n_envs, which never overflows; 1 .. n_envs)
         """
         costmaps = list(costmaps)
         paths = list(paths)
@@ -126,7 +150,8 @@ class VecPlanEnv(object):
             np.count_nonzero(c.get_data()) * 20 > c.get_data().size for c in costmaps)
         self._compact_ego = bool(compact_ego)
         self._configure(params, n, float(costmaps[0].get_resolution()), noise_parameters, seed, auto_reset, device,
-                        env_id_base, with_ego, ego_staging if use_tma else 'spans', params_ids)   # use_tma=False: older spelling
+                        env_id_base, with_ego, ego_staging if use_tma else 'spans', params_ids,   # use_tma=False: older spelling
+                        episode_ends, episode_end_capacity)
         self._map_pool = costmaps
         self._map_ids_host = (np.arange(n) % len(costmaps)) if map_ids is None else np.asarray(map_ids, dtype=np.int64)
         self._path_ids_host = (np.arange(n) % len(paths)) if path_ids is None else np.asarray(path_ids, dtype=np.int64)
@@ -151,8 +176,20 @@ class VecPlanEnv(object):
                 self._batch.flags |= nat.BATCH_SPARSE_EGO_ONLY
 
     def _configure(self, params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
-                   ego_staging, params_ids=None):
+                   ego_staging, params_ids=None, episode_ends=False, episode_end_capacity=None):
         """Everything that does not depend on where the maps and paths come from."""
+        self.episode_ends = bool(episode_ends)
+        self.episode_end_capacity = None
+        if self.episode_ends:
+            cap = int(n_envs) if episode_end_capacity is None else int(episode_end_capacity)
+            if not 1 <= cap <= int(n_envs):
+                raise ValueError("episode_end_capacity must be in [1, n_envs=%d], got %d" % (int(n_envs), cap))
+            if with_ego and ego_staging != 'tiles':
+                raise ValueError("episode_ends with the egocentric observation needs ego_staging='tiles' (the final crops are "
+                                 "rendered by the cell-tile kernels), got %r" % (ego_staging,))
+            self.episode_end_capacity = cap
+        elif episode_end_capacity is not None:
+            raise ValueError("episode_end_capacity needs episode_ends=True")
         nat.require_cuda()
         self._pool = self._noise_pool = self._env_rows = None
         if envp.is_pool(params):
@@ -382,6 +419,23 @@ class VecPlanEnv(object):
         self._hit_u8 = torch.zeros(n, dtype=torch.uint8, device=dev)
         self.obs_vec = torch.zeros((n, 12), dtype=torch.float32, device=dev)
         cp = self._c_params
+        if self.episode_ends:
+            cap = self.episode_end_capacity
+            self._end_reason = torch.zeros(n, dtype=torch.uint8, device=dev)
+            self._final_slot = torch.full((n,), -1, dtype=torch.int32, device=dev)
+            self._final_obs_vec = torch.zeros((n, 12), dtype=torch.float32, device=dev)
+            self._final_return = torch.zeros(n, dtype=torch.float64, device=dev)
+            self._final_length = torch.zeros(n, dtype=torch.int32, device=dev)
+            self._ends_count = torch.zeros(2, dtype=torch.int32, device=dev)
+            self._end_flags = torch.zeros((3, n), dtype=torch.bool, device=dev)      # ended, terminated, truncated
+            self._end_scratch = torch.zeros(n, dtype=torch.uint8, device=dev)
+            self._final_goal_n_state = self._final_ego_work = self.final_ego_image = self._final_list = None
+            if self.with_ego:
+                self._final_goal_n_state = torch.zeros((n, 9, 1), dtype=torch.float32, device=dev)
+                self._final_ego_work = torch.zeros((cap, 128), dtype=torch.uint8, device=dev)
+                self._final_list = torch.zeros(cap, dtype=torch.int32, device=dev)
+                # (before the step's crops: _new_image_tensor records whether the step's crops got compressed memory)
+                self.final_ego_image = self._new_image_tensor((cap, cp.ego_h, cp.ego_w, 1))
         if self.with_ego:
             self.ego_image = self._new_image_tensor((n, cp.ego_h, cp.ego_w, 1))
             self.goal_n_state = torch.zeros((n, 9, 1), dtype=torch.float32, device=dev)
@@ -462,6 +516,18 @@ class VecPlanEnv(object):
             self._ego_hit_count = torch.zeros(self.n_envs, dtype=torch.int32, device=self.device)
             # (BcgStepOut.ego_hits is only set for the steps whose lists are wanted: step_host(images='compact'))
         self._out = out
+        self._ends = None                                  # BcgEpisodeEnds* of the step calls (None: episode_ends off)
+        if getattr(self, 'episode_ends', False):
+            en = nat.BcgEpisodeEnds()
+            en.reason, en.final_slot = self._end_reason.data_ptr(), self._final_slot.data_ptr()
+            en.final_obs_vec, en.final_return = self._final_obs_vec.data_ptr(), self._final_return.data_ptr()
+            en.final_length, en.count = self._final_length.data_ptr(), self._ends_count.data_ptr()
+            if self.with_ego:
+                en.final_goal_n_state, en.final_ego_work = self._final_goal_n_state.data_ptr(), self._final_ego_work.data_ptr()
+                en.final_ego_image, en.final_list = self.final_ego_image.data_ptr(), self._final_list.data_ptr()
+            en.capacity = self.episode_end_capacity
+            self._c_ends = en
+            self._ends = C.byref(self._c_ends)
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -474,6 +540,33 @@ class VecPlanEnv(object):
     @property
     def hit(self):
         return self._hit_u8.view(torch.bool)
+
+    def _ends_on(self):
+        if not self.episode_ends:
+            raise ValueError("this batch was built without episode_ends=True")
+
+    @property
+    def episode_reason(self):
+        """uint8 [N] of the last step (needs episode_ends): nat.END_GOAL | END_COLLIDED | END_TIMEOUT, the causes of `done`,
+        set while the env is done; nat.END_NOW, the episode ended at this step"""
+        self._ends_on()
+        return self._end_reason
+
+    @property
+    def terminated(self):
+        """bool [N] (needs episode_ends): done by reaching the goal or by a collision -- no bootstrap from the final
+        observation.  A reused buffer, like `done`."""
+        self._ends_on()
+        torch.bitwise_and(self._end_reason, nat.END_GOAL | nat.END_COLLIDED, out=self._end_scratch)
+        return torch.ne(self._end_scratch, 0, out=self._end_flags[1])
+
+    @property
+    def truncated(self):
+        """bool [N] (needs episode_ends): done by the iteration timeout alone (a goal or a collision on the same step
+        terminates) -- bootstrap from the final observation.  A reused buffer, like `done`."""
+        self._ends_on()
+        torch.bitwise_and(self._end_reason, nat.END_GOAL | nat.END_COLLIDED | nat.END_TIMEOUT, out=self._end_scratch)
+        return torch.eq(self._end_scratch, nat.END_TIMEOUT, out=self._end_flags[2])
 
     def action_bounds(self):
         """low, high of the action Box (reference envs/base/env.py:237-240), float32."""
@@ -497,9 +590,9 @@ class VecPlanEnv(object):
         """One env step for every env.  actions: [N, 2] float32/float64 (tensor or ndarray).
         Returns (VecObservation, reward fp64 [N], done bool [N], {}) -- tensors are reused buffers."""
         a = self._as_actions(actions)
-        nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
+        nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
                                           1 if a.dtype == torch.float64 else 0, self._step_index,
-                                          C.byref(self._out), None, self._stream()))
+                                          C.byref(self._out), self._ends, None, self._stream()))
         self._step_index += 1
         return self.observation(), self.reward, self.done, {}
 
@@ -522,8 +615,8 @@ class VecPlanEnv(object):
             g = torch.cuda.CUDAGraph()
             with torch.cuda.stream(side):
                 with torch.cuda.graph(g, stream=side):
-                    nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows,
-                                                      nat.ptr(self.actions), 0, 0, C.byref(self._out), None,
+                    nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows,
+                                                      nat.ptr(self.actions), 0, 0, C.byref(self._out), self._ends, None,
                                                       C.c_void_p(side.cuda_stream)))
             torch.cuda.current_stream(self.device).wait_stream(side)
             self._graph = g
@@ -543,8 +636,8 @@ class VecPlanEnv(object):
             raise ValueError("plan must have shape [H, %d, 2]" % self.n_envs)
         plan = plan.to(torch.float32).contiguous()
         horizon = int(plan.shape[0])
-        nat.check(nat.lib().bcg_rollout_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(plan), horizon,
-                                             self._step_index, C.byref(self._out), self._stream()))
+        nat.check(nat.lib().bcg_rollout_ends(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(plan), horizon,
+                                             self._step_index, C.byref(self._out), self._ends, self._stream()))
         self._step_index += horizon
 
     def rollout_graph(self, plan):
@@ -570,8 +663,8 @@ class VecPlanEnv(object):
             with torch.cuda.stream(side):
                 with torch.cuda.graph(g, stream=side):
                     for h in range(horizon):
-                        nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows,
-                                                          nat.ptr(buf[h]), 0, 0, C.byref(self._out), None,
+                        nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows,
+                                                          nat.ptr(buf[h]), 0, 0, C.byref(self._out), self._ends, None,
                                                           C.c_void_p(side.cuda_stream)))
             torch.cuda.current_stream(self.device).wait_stream(side)
             self._plan_graph = (horizon, g, buf)
@@ -594,9 +687,9 @@ class VecPlanEnv(object):
         handles exist; entries may be None) recorded around the kernels; see bcg_step_events."""
         a = self._as_actions(actions)
         handles = (C.c_void_p * 5)(*[C.c_void_p(ev.cuda_event if ev is not None else None) for ev in events])
-        nat.check(nat.lib().bcg_step_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
+        nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
                                           1 if a.dtype == torch.float64 else 0, self._step_index,
-                                          C.byref(self._out), handles, self._stream()))
+                                          C.byref(self._out), self._ends, handles, self._stream()))
         self._step_index += 1
         return self.observation(), self.reward, self.done, {}
 
@@ -610,7 +703,9 @@ class VecPlanEnv(object):
         host memory as well, after the egocentric kernel (N x 15.6 KB per step: the PCIe link then sets the pace).
         Returns (reward, done, obs_vec) host tensors -- plus (ego_image, goal_n_state) with `images` --, valid when
         this call returns.  It waits for exactly what it returns: without `images` that is the copies of reward / done /
-        obs, not the egocentric kernel, which finishes in stream order behind them."""
+        obs, not the egocentric kernel, which finishes in stream order behind them.  With episode_ends the episode ends
+        and final observations are computed but stay on the device (`final_observation()`); copying them to the host
+        here is not implemented yet."""
         if getattr(self, '_host_io', None) is None:
             n = self.n_envs
             self._host_io = dict(
@@ -868,6 +963,34 @@ class VecPlanEnv(object):
             self._status.zero_()
             raise nat.BcgError("%d generated worlds did not fit their map / path slots (envs left unchanged)"
                                % st[nat.STATUS_SLOT_OVERFLOW])
+
+    def final_observation(self):
+        """The final observation of every episode that ended at the last step (needs episode_ends), as it was before
+        the auto-reset replaced it: a FinalObservation of device tensors.  Does not synchronise; `ended` and the rows
+        combine with the step's outputs by torch.where."""
+        self._ends_on()
+        torch.bitwise_and(self._end_reason, nat.END_NOW, out=self._end_scratch)
+        ended = torch.ne(self._end_scratch, 0, out=self._end_flags[0])
+        return FinalObservation(ended=ended, obs_vec=self._final_obs_vec, goal_n_state=self._final_goal_n_state,
+                                episode_return=self._final_return, episode_length=self._final_length, slot=self._final_slot,
+                                ego_image=self.final_ego_image, count=self._ends_count[0])
+
+    def final_ego(self, env_ids):
+        """Final crops (uint8 [k, H, W, 1]) of envs `env_ids` whose episodes ended at the last step.  Synchronises; raises
+        when the step had more episode ends than episode_end_capacity (some crops were not kept) or when an env did not
+        end at the last step."""
+        self._ends_on()
+        if not self.with_ego:
+            raise ValueError("this batch was built without the egocentric observation (with_ego=False)")
+        count, cap = int(self._ends_count[0]), self.episode_end_capacity
+        if count > cap:
+            raise nat.BcgError("%d episodes ended at the last step but episode_end_capacity is %d: the final crops of %d "
+                               "of them were not kept" % (count, cap, count - cap))
+        idx = self._indices(env_ids)
+        slots = self._final_slot[idx]
+        if bool((slots < 0).any()):
+            raise ValueError("env %d did not end at the last step" % int(idx[torch.nonzero(slots < 0)[0, 0]]))
+        return self.final_ego_image[slots.to(torch.int64)]
 
     def episode_stats(self, reset=False):
         """Device-accumulated episode statistics as a fp64 tensor [STATS_WORDS] (see STAT_NAMES)."""

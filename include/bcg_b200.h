@@ -304,6 +304,46 @@ typedef struct BcgEnvRows {
   const int32_t* i;  /* device [BCG_EP_I_ROWS][n_envs] */
 } BcgEnvRows;
 
+/* Episode ends of an auto-reset batch (bcg_step_ends / bcg_rollout_ends): why each env is done, and the observation of
+ * every episode that ends at this step as it was before the in-kernel reset overwrote it.
+ *
+ * reason[e] is written for every env at every step:
+ *   BCG_END_GOAL | BCG_END_COLLIDED | BCG_END_TIMEOUT  the causes of `done` (env.py:407-419), set while the env is done
+ *                                                      (without auto-reset they stay set, like done)
+ *   BCG_END_NOW                                        the episode ended at this step (done now, not done before it:
+ *                                                      the condition under which the episode statistics count it)
+ * terminated = done && (GOAL | COLLIDED); truncated = done && TIMEOUT && !terminated (a timeout on the step of a goal or
+ * a collision is a termination).
+ * Every env with BCG_END_NOW gets its final record, with or without auto-reset: final_obs_vec (BcgStepOut.obs_vec's
+ * fields, [11] the post-step target index), final_goal_n_state (needs BcgStepOut.goal_n_state), final_return (the
+ * episode return including this step's reward) and final_length (iterations).  These rows are dense, indexed by env
+ * and valid only where BCG_END_NOW is set.
+ * Final crops (needs BcgStepOut.ego_image and the cell-tile planes) are kept in `capacity` slots: count[0] numbers the
+ * ends of the step in no particular order; end k < capacity gets slot k, final_slot[e] = k (else -1), its egocentric
+ * record is copied to final_ego_work[k] before the reset rewrites it, and the egocentric kernels render it into
+ * final_ego_image[k] in the launches that render the step's crops.  count[0] keeps counting past the capacity:
+ * count[0] > capacity means that count[0] - capacity ended envs (which ones is unspecified) have final_slot -1 and no
+ * crop; nothing is written past the capacity.  move_kernel zeroes count[] at the start of every step, so a captured
+ * CUDA graph of a step replays correctly and the counts describe the last step. */
+#define BCG_END_GOAL 1
+#define BCG_END_COLLIDED 2
+#define BCG_END_TIMEOUT 4
+#define BCG_END_NOW 8
+typedef struct BcgEpisodeEnds {
+  uint8_t* reason;            /* [n]                                                                          */
+  int32_t* final_slot;        /* [n] crop slot of an env that ended at this step, -1 otherwise                */
+  float* final_obs_vec;       /* [n][12]                                                                      */
+  float* final_goal_n_state;  /* [n][9]   (needed with BcgStepOut.goal_n_state)                               */
+  double* final_return;       /* [n]                                                                          */
+  int32_t* final_length;      /* [n]                                                                          */
+  void* final_ego_work;       /* [capacity][128 bytes]          (these three are needed with BcgStepOut.ego_image) */
+  uint8_t* final_ego_image;   /* [capacity][ego_h][ego_w]                                                     */
+  int32_t* final_list;        /* [capacity] scratch: slots the sparse egocentric kernel hands to the dense one */
+  int32_t* count;             /* [2]: [0] episodes that ended at this step, [1] scratch (hand-over count)     */
+  int32_t capacity;           /* >= 1                                                                         */
+  int32_t reserved;
+} BcgEpisodeEnds;
+
 /* outputs of one step; any pointer may be NULL to skip that output */
 typedef struct BcgStepOut {
   double* reward;      /* [n] reward of this step (reward.py:214-259)                          */
@@ -329,7 +369,7 @@ int bcg_abi_version(void);
 size_t bcg_last_error(char* buf, size_t cap);
 /* sizeof() of the ABI structs, in declaration order: 0 BcgParams, 1 BcgMapDesc, 2 BcgPathDesc,
  * 3 BcgFootprintLut, 4 BcgBatch, 5 BcgStateLayout, 6 BcgStepOut, 7 BcgTurnParams, 8 BcgAisleSlots, 9 BcgMiniGenParams,
- * 10 BcgMiniParams, 11 BcgEnvRows; -1 for anything else.  Lets a
+ * 10 BcgMiniParams, 11 BcgEnvRows, 12 BcgEpisodeEnds; -1 for anything else.  Lets a
  * binding (ctypes, cffi, ...) verify its struct mirrors before the first call. */
 int64_t bcg_sizeof(int32_t which);
 /* number of CUDA devices visible, <0 on error; makes a missing GPU a loud failure for callers */
@@ -416,6 +456,13 @@ int bcg_step_events(const BcgParams* p, const BcgBatch* b, const void* actions, 
 int bcg_step_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
                   uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream);
 
+/* bcg_step_rows that also reports episode ends (BcgEpisodeEnds; NULL: bcg_step_rows).  Same launches: move_kernel zeroes
+ * the counters, reward_kernel writes the reasons and final records and copies the egocentric records of the ended envs
+ * before it resets them, and the egocentric kernels render the final crops after the step's own.  Final crops need the
+ * cell-tile planes (BcgBatch.cell_tile_arena). */
+int bcg_step_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
+                  uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* const* events, void* stream);
+
 /* the pieces, individually addressable (used by tests, ncu and the hook seam) */
 /* robot.step (tricycle_model.py:478-538 / differential_drive.py:236-265) into b->cand */
 int bcg_kinematic_step(const BcgParams* p, const BcgBatch* b, const void* actions,
@@ -484,6 +531,9 @@ int bcg_rollout(const BcgParams* p, const BcgBatch* b, const float* plan, int32_
 /* bcg_rollout for a batch with per-env parameters (see bcg_step_rows; rows NULL: bcg_rollout) */
 int bcg_rollout_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
                      uint64_t step_index, const BcgStepOut* out, void* stream);
+/* bcg_rollout_rows with episode ends (see bcg_step_ends; ends NULL: bcg_rollout_rows): `ends` describes the last step */
+int bcg_rollout_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
+                     uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* stream);
 
 /* -- image memory --------------------------------------------------------------------------------
  * Egocentric crops are mostly zeros.  A device allocation with compute-data compression (CUDA virtual memory

@@ -2,10 +2,11 @@
 
     python profiles/probes/sass_compare.py OLD.so NEW.so
 
-Kernels are matched by demangled name, with a `false` rows template argument (`move_kernel<8, false>`) and a trailing
-BcgEnvRows parameter dropped, so that the instantiations without per-env rows line up with the kernels of a build that
-had no rows.  Branch-target addresses are ignored.  Prints `same` or `DIFFERENT` (with the count of changed
-instructions) per kernel; instantiations with rows are listed as new.
+Kernels are matched by demangled name, with trailing `false` template arguments (the per-env rows and episode-ends flags:
+`move_kernel<8, false, false>`) and the trailing BcgEnvRows / episode-ends parameters dropped, so that the instantiations
+without rows or ends line up with the kernels of a build that had neither.  Branch-target addresses are ignored.  Prints
+`same` or `DIFFERENT` (with the count of changed instructions) per kernel; instantiations without a counterpart are
+listed as new.
 """
 import difflib
 import re
@@ -38,7 +39,12 @@ def kernels(so):
 def key(name):
     d = subprocess.run([CUDA + "cu++filt", name], capture_output=True, text=True).stdout.strip()
     d = re.sub(r"^void ", "", d.replace("(anonymous namespace)::", ""))
-    return d.replace("<(bool)0>", "").replace(", (bool)0>", ">").replace(", BcgEnvRows)", ")")
+    d = d.replace(", BcgEpisodeEnds)", ")").replace(", BcgEnvRows, int *)", ")").replace(", BcgEnvRows)", ")")
+    while True:
+        k = d.replace("<(bool)0>", "").replace(", (bool)0>", ">")
+        if k == d:
+            return d
+        d = k
 
 
 def main(old, new):
