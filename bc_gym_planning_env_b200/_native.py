@@ -157,24 +157,14 @@ SYMBOLS = {
     "bcg_build_cell_tiles": (C.c_int, [C.POINTER(BcgBatch), C.c_int32, C.c_int32, _P]),
     "bcg_encode_map_tensor_maps": (C.c_int, [C.POINTER(BcgMapDesc), C.c_int32, _P, C.POINTER(C.c_int32), C.c_int32,
                                              C.c_int32, _P]),
-    "bcg_init_state": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P]),
-    "bcg_init_state_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P]),
-    "bcg_generate_aisles_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows),
-                                           C.POINTER(BcgAisleSlots), _P, _P, C.c_uint64, C.c_double, _P]),
-    "bcg_generate_aisles": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgAisleSlots), _P, _P, C.c_uint64,
-                                      C.c_double, _P]),
+    "bcg_init_state": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P]),
+    "bcg_generate_aisles": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows),
+                                      C.POINTER(BcgAisleSlots), _P, _P, C.c_uint64, C.c_double, _P]),
     "bcg_generate_minis": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgAisleSlots), _P,
                                      C.POINTER(BcgMiniGenParams), _P, _P, C.c_uint64, C.c_double, _P]),
     "bcg_reset_where": (C.c_int, [C.POINTER(BcgBatch), _P, _P]),
-    "bcg_step": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64,
-                           C.POINTER(BcgStepOut), _P]),
-    "bcg_step_events": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64,
-                                  C.POINTER(BcgStepOut), C.POINTER(C.c_void_p), _P]),
-    "bcg_step_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
-                                C.POINTER(BcgStepOut), C.POINTER(C.c_void_p), _P]),
-    "bcg_step_ends": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
-                                C.POINTER(BcgStepOut), C.POINTER(BcgEpisodeEnds), C.POINTER(C.c_void_p), _P]),
-    "bcg_kinematic_step": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64, _P]),
+    "bcg_step": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
+                           C.POINTER(BcgStepOut), C.POINTER(BcgEpisodeEnds), C.POINTER(C.c_void_p), _P]),
     "bcg_collision": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, _P, _P, _P]),
     "bcg_collision_u8": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, _P, _P]),
     "bcg_collision_recheck": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, _P]),
@@ -188,11 +178,8 @@ SYMBOLS = {
     "bcg_inverse_transform": (C.c_int, [_P, C.c_int64, _P, _P]),
     "bcg_project_poses": (C.c_int, [C.POINTER(C.c_double), _P, C.c_int64, _P, _P]),
     "bcg_observe_ego_path": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.c_int32, _P, _P, _P]),
-    "bcg_rollout": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), _P, C.c_int32, C.c_uint64, C.POINTER(BcgStepOut), _P]),
-    "bcg_rollout_rows": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
-                                   C.POINTER(BcgStepOut), _P]),
-    "bcg_rollout_ends": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
-                                   C.POINTER(BcgStepOut), C.POINTER(BcgEpisodeEnds), _P]),
+    "bcg_rollout": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P, C.c_int32, C.c_uint64,
+                              C.POINTER(BcgStepOut), C.POINTER(BcgEpisodeEnds), _P]),
     "bcg_alloc_image_memory": (C.c_int, [C.c_int64, C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
     "bcg_free_image_memory": (C.c_int, [_P, C.c_int64]),
 }

@@ -30,10 +30,6 @@
 #include "bcg_generate.cuh"
 
 using namespace bcg;
-// block size of the stand-alone kinematics kernel (the step kernels have their own macros below)
-#ifndef BCG_KIN_THREADS
-#define BCG_KIN_THREADS 128
-#endif
 namespace {
 
 thread_local std::string g_last_error;
@@ -153,38 +149,21 @@ int check_rows(const BcgEnvRows* rows) {
   return BCG_OK;
 }
 
-// ---- kernels -------------------------------------------------------------------------------------
-
-// robot.step for every env (stand-alone bcg_kinematic_step): envs/base/env.py:371-373 (control delay) + robot model, the
-// proposed robot state into b.cand rows 0..6.  One thread per env: every load and store is a coalesced SoA row.
-__global__ void __launch_bounds__(BCG_KIN_THREADS) kin_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L,
-                                                  const void* __restrict__ actions, const int action_is_f64,
-                                                  const uint64_t step_index) {
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= b.n_envs) return;
-  const int64_t N = b.n_envs;
-  double u[2];
-  if (action_is_f64) {
-    const double2 a = reinterpret_cast<const double2*>(actions)[e];
-    u[0] = a.x;
-    u[1] = a.y;
-  } else {
-    const float2 a = reinterpret_cast<const float2*>(actions)[e];
-    u[0] = (double)a.x;
-    u[1] = (double)a.y;
-  }
-  double s[7];
-#pragma unroll
-  for (int r = 0; r < 7; ++r) s[r] = b.state_f[(BCG_F_ROBOT + r) * N + e];
-  if (p.delay_control > 0) {
-    int q = b.state_i[BCG_I_QC * N + e];
-    delay_line<2>(b.state_f + (int64_t)L.ring_control * N + e, N, q, p.delay_control, u);
-    b.state_i[BCG_I_QC * N + e] = q;
-  }
-  robot_step(s, u[0], u[1], p, p.env_id_base + (uint64_t)e, step_index);
-#pragma unroll
-  for (int r = 0; r < 7; ++r) b.cand[r * N + e] = s[r];
+// the per-env slots of the device-side world generators (`who` names the entry point in the messages)
+int check_slots(const BcgParams* p, const BcgBatch* b, const BcgAisleSlots* slots, double path_delta, const char* who) {
+  BCG_REQUIRE(slots && slots->gen_state, "null slots / gen_state");
+  BCG_REQUIRE(b->cell_tile_arena, std::string(who) + " needs the cell-tile arena");
+  BCG_REQUIRE(!b->map_tmaps, std::string(who) + " cannot re-encode TMA tensor maps; use cell-tile or plain-load staging");
+  BCG_REQUIRE(b->n_maps == b->n_envs && b->n_paths == b->n_envs, "device-generated envs own one map and one path slot each");
+  BCG_REQUIRE(slots->map_slot_bytes > 0 && slots->tile_slot_words > 0 && slots->path_pitch >= 8 && slots->path_pitch % 4 == 0 &&
+                  slots->chunk_pitch * 32 >= slots->path_pitch,
+              "bad slot sizes");
+  BCG_REQUIRE(path_delta > 0, "path_delta must be positive");
+  BCG_REQUIRE((int)(0.05 / p->resolution) <= 1, "walls are drawn one pixel thick: resolution must be above 0.025 m");
+  return BCG_OK;
 }
+
+// ---- kernels -------------------------------------------------------------------------------------
 
 // work records of arbitrary poses [3][n] (stand-alone collision entry points)
 __global__ void __launch_bounds__(128) pose_prep_kernel(const BcgParams p, const BcgBatch b,
@@ -2865,7 +2844,7 @@ int bcg_encode_map_tensor_maps(const BcgMapDesc* maps_host, int32_t n_maps, cons
   return BCG_OK;
 }
 
-int bcg_init_state_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, void* stream) {
+int bcg_init_state(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, void* stream) {
   if (int rc = check_batch(p, b)) return rc;
   if (int rc = check_rows(rows)) return rc;
   const int64_t grid = blocks_for((int64_t)b->n_envs * 32, 256);
@@ -2877,27 +2856,12 @@ int bcg_init_state_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows*
   return BCG_OK;
 }
 
-int bcg_init_state(const BcgParams* p, const BcgBatch* b, void* stream) { return bcg_init_state_rows(p, b, nullptr, stream); }
-
-int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgAisleSlots* slots, const uint8_t* mask,
-                        const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta, void* stream) {
-  return bcg_generate_aisles_rows(p, b, nullptr, slots, mask, turn_params, draw_index, path_delta, stream);
-}
-
-int bcg_generate_aisles_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
-                             const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
-                             void* stream) {
+int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
+                        const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
+                        void* stream) {
   if (int rc = check_batch(p, b)) return rc;
   if (int rc = check_rows(rows)) return rc;
-  BCG_REQUIRE(slots && slots->gen_state, "null slots / gen_state");
-  BCG_REQUIRE(b->cell_tile_arena, "bcg_generate_aisles needs the cell-tile arena");
-  BCG_REQUIRE(!b->map_tmaps, "bcg_generate_aisles cannot re-encode TMA tensor maps; use cell-tile or plain-load staging");
-  BCG_REQUIRE(b->n_maps == b->n_envs && b->n_paths == b->n_envs, "device-generated envs own one map and one path slot each");
-  BCG_REQUIRE(slots->map_slot_bytes > 0 && slots->tile_slot_words > 0 && slots->path_pitch >= 8 && slots->path_pitch % 4 == 0 &&
-                  slots->chunk_pitch * 32 >= slots->path_pitch,
-              "bad slot sizes");
-  BCG_REQUIRE(path_delta > 0, "path_delta must be positive");
-  BCG_REQUIRE((int)(0.05 / p->resolution) <= 1, "walls are drawn one pixel thick: resolution must be above 0.025 m");
+  if (int rc = check_slots(p, b, slots, path_delta, "bcg_generate_aisles")) return rc;
   if (rows)
     generate_aisles_kernel<true><<<b->n_envs, 256, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p), *slots, mask, turn_params,
                                                                            draw_index, path_delta, *rows);
@@ -2912,16 +2876,8 @@ int bcg_generate_minis(const BcgParams* p, const BcgBatch* b, const BcgAisleSlot
                        const BcgMiniGenParams* gen, const BcgMiniParams* mini_params, BcgMiniParams* params_out,
                        uint64_t draw_index, double path_delta, void* stream) {
   if (int rc = check_batch(p, b)) return rc;
-  BCG_REQUIRE(slots && slots->gen_state, "null slots / gen_state");
+  if (int rc = check_slots(p, b, slots, path_delta, "bcg_generate_minis")) return rc;
   BCG_REQUIRE(gen || mini_params, "need the sampling space (gen) or explicit MiniEnvParams");
-  BCG_REQUIRE(b->cell_tile_arena, "bcg_generate_minis needs the cell-tile arena");
-  BCG_REQUIRE(!b->map_tmaps, "bcg_generate_minis cannot re-encode TMA tensor maps; use cell-tile or plain-load staging");
-  BCG_REQUIRE(b->n_maps == b->n_envs && b->n_paths == b->n_envs, "device-generated envs own one map and one path slot each");
-  BCG_REQUIRE(slots->map_slot_bytes > 0 && slots->tile_slot_words > 0 && slots->path_pitch >= 8 && slots->path_pitch % 4 == 0 &&
-                  slots->chunk_pitch * 32 >= slots->path_pitch,
-              "bad slot sizes");
-  BCG_REQUIRE(path_delta > 0, "path_delta must be positive");
-  BCG_REQUIRE((int)(0.05 / p->resolution) <= 1, "walls are drawn one pixel thick: resolution must be above 0.025 m");
   BcgMiniGenParams g;
   memset(&g, 0, sizeof(g));
   if (gen) g = *gen;
@@ -2934,16 +2890,6 @@ int bcg_generate_minis(const BcgParams* p, const BcgBatch* b, const BcgAisleSlot
 int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream) {
   BCG_REQUIRE(b && b->state_f && b->init_f && b->state_i && b->init_i && b->n_envs > 0, "bad batch");
   reset_kernel<<<blocks_for(b->n_envs, 256), 256, 0, (cudaStream_t)stream>>>(*b, mask);
-  BCG_CHECK_CUDA(cudaGetLastError());
-  return BCG_OK;
-}
-
-int bcg_kinematic_step(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64,
-                       uint64_t step_index, void* stream) {
-  if (int rc = check_batch(p, b)) return rc;
-  BCG_REQUIRE(actions, "null actions");
-  kin_kernel<<<blocks_for(b->n_envs, BCG_KIN_THREADS), BCG_KIN_THREADS, 0, (cudaStream_t)stream>>>(*p, *b, make_layout(*p), actions,
-                                                                                              action_is_f64, step_index);
   BCG_CHECK_CUDA(cudaGetLastError());
   return BCG_OK;
 }
@@ -3034,6 +2980,12 @@ static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego
   // persistent CTAs, as many per SM as fit with this crop's tables (18 for the 117 x 133 crop)
   const int tab_bytes = (p->ego_w + p->ego_h + 4) * (int)sizeof(int2);     // + a sentinel before and after each table
   const bool sum = b->occ_sum_arena != nullptr;
+  using SparseKernel = decltype(&ego_sparse_kernel<false, false, false>);
+  static const SparseKernel kernels[2][2][2] = {      // [SUM][HITS][ENDS]
+      {{ego_sparse_kernel<false, false, false>, ego_sparse_kernel<false, false, true>},
+       {ego_sparse_kernel<false, true, false>, ego_sparse_kernel<false, true, true>}},
+      {{ego_sparse_kernel<true, false, false>, ego_sparse_kernel<true, false, true>},
+       {ego_sparse_kernel<true, true, false>, ego_sparse_kernel<true, true, true>}}};
   static int per_sm_cache[2][64] = {{0}}, tab_cache[2][64] = {{0}};
   int dev = 0;
   BCG_CHECK_CUDA(cudaGetDevice(&dev));
@@ -3041,8 +2993,7 @@ static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego
   if (dev >= 0 && dev < 64 && per_sm_cache[sum][dev] > 0 && tab_cache[sum][dev] == tab_bytes) {
     per_sm = per_sm_cache[sum][dev];
   } else {
-    if (sum) BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ego_sparse_kernel<true, false, false>, BCG_EGS_THREADS, tab_bytes));
-    else BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ego_sparse_kernel<false, false, false>, BCG_EGS_THREADS, tab_bytes));
+    BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernels[sum][0][0], BCG_EGS_THREADS, tab_bytes));
     BCG_REQUIRE(per_sm > 0, "the sparse egocentric kernel does not fit an SM with this crop size");
     if (dev >= 0 && dev < 64) {
       per_sm_cache[sum][dev] = per_sm;
@@ -3061,31 +3012,11 @@ static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego
     return v ? atoll(v) : 160ll << 20;
   }();
   const int evict = (long long)b->n_envs * p->ego_w * p->ego_h <= evict_bytes ? 0 : b->n_envs;   // evict_from: envs >= it use the policy
-  uint32_t* const no_list = nullptr;
-  int32_t* const no_count = nullptr;
+  const bool with_hits = hits.list != nullptr;
   // (the final crops of episode ends, when asked for, are the items behind the envs)
   const BcgEpisodeEnds en = ends ? *ends : BcgEpisodeEnds{};
-#define BCG_EGS_LAUNCH(SUM, HITS, ENDS, LIST, COUNT, CAP) \
-  BCG_CHECK_CUDA(launch_step_kernel(ego_sparse_kernel<SUM, HITS, ENDS>, grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b, ego_image, \
-                                    LIST, COUNT, CAP, evict, en))
-  if (hits.list) {
-    if (ends) {
-      if (sum) BCG_EGS_LAUNCH(true, true, true, hits.list, hits.count, hits.cap);
-      else BCG_EGS_LAUNCH(false, true, true, hits.list, hits.count, hits.cap);
-    } else {
-      if (sum) BCG_EGS_LAUNCH(true, true, false, hits.list, hits.count, hits.cap);
-      else BCG_EGS_LAUNCH(false, true, false, hits.list, hits.count, hits.cap);
-    }
-  } else {
-    if (ends) {
-      if (sum) BCG_EGS_LAUNCH(true, false, true, no_list, no_count, 0);
-      else BCG_EGS_LAUNCH(false, false, true, no_list, no_count, 0);
-    } else {
-      if (sum) BCG_EGS_LAUNCH(true, false, false, no_list, no_count, 0);
-      else BCG_EGS_LAUNCH(false, false, false, no_list, no_count, 0);
-    }
-  }
-#undef BCG_EGS_LAUNCH
+  BCG_CHECK_CUDA(launch_step_kernel(kernels[sum][with_hits][ends != nullptr], grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b,
+                                    ego_image, hits.list, with_hits ? hits.count : nullptr, with_hits ? hits.cap : 0, evict, en));
   BCG_CHECK_CUDA(cudaGetLastError());
   if (b->flags & BCG_BATCH_SPARSE_EGO_ONLY) return BCG_OK;     // the sparse kernel rendered every env itself
   return launch_ego_dense(p, b, ego_image, b->ego_list, ends, s);
@@ -3135,44 +3066,6 @@ int bcg_observe_ego(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, f
 
 }  // extern "C"
 
-// move_kernel of one step, at the register tier the batch size picks
-template <bool ROWS, bool ENDS>
-static int launch_move_kernel(const BcgParams* p, const BcgBatch* b, const BcgEnvRows& rows, const BcgStateLayout& L,
-                              const void* actions, int32_t action_is_f64, uint64_t step_index, const BcgStepOut* out,
-                              int32_t* ends_count, int cap, bool pdl, cudaStream_t s) {
-  int sms = 0;
-  if (int rc = sm_count_of_current_device(&sms)) return rc;
-  const int move_blocks = (int)blocks_for(b->n_envs, BCG_MOVE_THREADS);
-  if (move_blocks <= sms * BCG_MOVE_FEWER_BLOCKS)
-    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEWER_BLOCKS, ROWS, ENDS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows, ends_count));
-  else if (move_blocks <= sms * BCG_MOVE_FEW_BLOCKS)
-    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_FEW_BLOCKS, ROWS, ENDS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows, ends_count));
-  else
-    BCG_CHECK_CUDA(launch_step_kernel(move_kernel<BCG_MOVE_MIN_BLOCKS, ROWS, ENDS>, move_blocks, BCG_MOVE_THREADS, 0, s, pdl, *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, rows, ends_count));
-  return BCG_OK;
-}
-
-// reward_kernel of one step, with the lane group the batch size picks
-template <bool ROWS, bool ENDS>
-static int launch_reward_kernel(const BcgParams* p, const BcgBatch* b, const BcgStepOut* out, const BcgEpisodeEnds& ends, int cap,
-                                bool pdl_reward, cudaStream_t s) {
-  const int64_t ns = b->n_envs;
-  if (ns > 16384) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<8, ROWS, ENDS>, blocks_for(ns * 8, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, ends));
-  else if (ns > 2048) BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<16, ROWS, ENDS>, blocks_for(ns * 16, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, ends));
-  else BCG_CHECK_CUDA(launch_step_kernel(reward_kernel<32, ROWS, ENDS>, blocks_for(ns * 32, BCG_REWARD_THREADS), BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, ends));
-  return BCG_OK;
-}
-
-// the two state kernels of a step (events[2], when set, is recorded between them)
-template <bool ROWS, bool ENDS>
-static int launch_state_kernels(const BcgParams* p, const BcgBatch* b, const BcgEnvRows& rows, const BcgStateLayout& L,
-                                const void* actions, int32_t action_is_f64, uint64_t step_index, const BcgStepOut* out,
-                                const BcgEpisodeEnds& ends, void* const* events, int cap, bool pdl, bool pdl_reward, cudaStream_t s) {
-  if (int rc = launch_move_kernel<ROWS, ENDS>(p, b, rows, L, actions, action_is_f64, step_index, out, ends.count, cap, pdl, s)) return rc;
-  if (events && events[2]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[2], s));
-  return launch_reward_kernel<ROWS, ENDS>(p, b, out, ends, cap, pdl_reward, s);
-}
-
 static int check_ends(const BcgBatch* b, const BcgStepOut* out, const BcgEpisodeEnds* ends) {
   if (!ends) return BCG_OK;
   BCG_REQUIRE(ends->capacity >= 1, "BcgEpisodeEnds.capacity must be at least 1");
@@ -3189,18 +3082,8 @@ static int check_ends(const BcgBatch* b, const BcgStepOut* out, const BcgEpisode
 
 extern "C" {
 
-int bcg_step_events(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64,
-                    uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream) {
-  return bcg_step_ends(p, b, nullptr, actions, action_is_f64, step_index, out, nullptr, events, stream);
-}
-
-int bcg_step_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
-                  uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream) {
-  return bcg_step_ends(p, b, rows, actions, action_is_f64, step_index, out, nullptr, events, stream);
-}
-
-int bcg_step_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
-                  uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* const* events, void* stream) {
+int bcg_step(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
+             uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* const* events, void* stream) {
   if (int rc = check_batch(p, b)) return rc;
   if (int rc = check_rows(rows)) return rc;
   BCG_REQUIRE(actions && out, "null actions/out");
@@ -3220,12 +3103,32 @@ int bcg_step_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows,
     const bool pdl_reward = !(events && events[2]);
     const BcgEnvRows r = rows ? *rows : BcgEnvRows{nullptr, nullptr};
     const BcgEpisodeEnds en = ends ? *ends : BcgEpisodeEnds{};
-    int rc;
-    if (rows) rc = ends ? launch_state_kernels<true, true>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s)
-                        : launch_state_kernels<true, false>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s);
-    else rc = ends ? launch_state_kernels<false, true>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s)
-                   : launch_state_kernels<false, false>(p, b, r, L, actions, action_is_f64, step_index, out, en, events, cap, pdl, pdl_reward, s);
-    if (rc) return rc;
+    // move_kernel at the register tier the batch size picks
+    using MoveKernel = decltype(&move_kernel<BCG_MOVE_MIN_BLOCKS, false, false>);
+    static const MoveKernel moves[3][2][2] = {      // [tier][ROWS][ENDS]
+        {{move_kernel<BCG_MOVE_FEWER_BLOCKS, false, false>, move_kernel<BCG_MOVE_FEWER_BLOCKS, false, true>},
+         {move_kernel<BCG_MOVE_FEWER_BLOCKS, true, false>, move_kernel<BCG_MOVE_FEWER_BLOCKS, true, true>}},
+        {{move_kernel<BCG_MOVE_FEW_BLOCKS, false, false>, move_kernel<BCG_MOVE_FEW_BLOCKS, false, true>},
+         {move_kernel<BCG_MOVE_FEW_BLOCKS, true, false>, move_kernel<BCG_MOVE_FEW_BLOCKS, true, true>}},
+        {{move_kernel<BCG_MOVE_MIN_BLOCKS, false, false>, move_kernel<BCG_MOVE_MIN_BLOCKS, false, true>},
+         {move_kernel<BCG_MOVE_MIN_BLOCKS, true, false>, move_kernel<BCG_MOVE_MIN_BLOCKS, true, true>}}};
+    int sms = 0;
+    if (int rc = sm_count_of_current_device(&sms)) return rc;
+    const int move_blocks = (int)blocks_for(b->n_envs, BCG_MOVE_THREADS);
+    const int tier = move_blocks <= sms * BCG_MOVE_FEWER_BLOCKS ? 0 : move_blocks <= sms * BCG_MOVE_FEW_BLOCKS ? 1 : 2;
+    BCG_CHECK_CUDA(launch_step_kernel(moves[tier][rows != nullptr][ends != nullptr], move_blocks, BCG_MOVE_THREADS, 0, s, pdl,
+                                      *p, *b, L, actions, (int)action_is_f64, step_index, *out, cap, r, en.count));
+    if (events && events[2]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[2], s));
+    // reward_kernel with the lane group the batch size picks
+    using RewardKernel = decltype(&reward_kernel<8, false, false>);
+    static const RewardKernel rewards[3][2][2] = {  // [group 8, 16, 32][ROWS][ENDS]
+        {{reward_kernel<8, false, false>, reward_kernel<8, false, true>}, {reward_kernel<8, true, false>, reward_kernel<8, true, true>}},
+        {{reward_kernel<16, false, false>, reward_kernel<16, false, true>}, {reward_kernel<16, true, false>, reward_kernel<16, true, true>}},
+        {{reward_kernel<32, false, false>, reward_kernel<32, false, true>}, {reward_kernel<32, true, false>, reward_kernel<32, true, true>}}};
+    const int64_t ns = b->n_envs;
+    const int group = ns > 16384 ? 0 : ns > 2048 ? 1 : 2;
+    BCG_CHECK_CUDA(launch_step_kernel(rewards[group][rows != nullptr][ends != nullptr], blocks_for(ns * (8 << group), BCG_REWARD_THREADS),
+                                      BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, en));
     BCG_CHECK_CUDA(cudaGetLastError());
   }
   if (events && events[3]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[3], s));
@@ -3240,26 +3143,12 @@ int bcg_step_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows,
   return BCG_OK;
 }
 
-int bcg_step(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64, uint64_t step_index,
-             const BcgStepOut* out, void* stream) {
-  return bcg_step_events(p, b, actions, action_is_f64, step_index, out, nullptr, stream);
-}
-
-int bcg_rollout(const BcgParams* p, const BcgBatch* b, const float* plan, int32_t horizon, uint64_t step_index,
-                const BcgStepOut* out, void* stream) {
-  return bcg_rollout_ends(p, b, nullptr, plan, horizon, step_index, out, nullptr, stream);
-}
-
-int bcg_rollout_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
-                     uint64_t step_index, const BcgStepOut* out, void* stream) {
-  return bcg_rollout_ends(p, b, rows, plan, horizon, step_index, out, nullptr, stream);
-}
-
-int bcg_rollout_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
-                     uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* stream) {
+int bcg_rollout(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
+                uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* stream) {
+  if (int rc = check_batch(p, b)) return rc;
   BCG_REQUIRE(plan && horizon >= 0, "null plan / negative horizon");
   for (int32_t h = 0; h < horizon; ++h)
-    if (int rc = bcg_step_ends(p, b, rows, plan + (int64_t)h * b->n_envs * 2, 0, step_index + (uint64_t)h, out, ends, nullptr, stream))
+    if (int rc = bcg_step(p, b, rows, plan + (int64_t)h * b->n_envs * 2, 0, step_index + (uint64_t)h, out, ends, nullptr, stream))
       return rc;
   return BCG_OK;
 }

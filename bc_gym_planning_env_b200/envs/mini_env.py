@@ -165,7 +165,7 @@ def _poses_collide(costmaps, poses, env_params):
     # a far-apart dummy path keeps the initial-state kernel happy; only the collision kernel is used
     dummy = [np.array([[0., 0., 0.], [100., 0., 0.]]) for _ in costmaps]
     checker = VecPlanEnv(costmaps, dummy, attr.evolve(env_params, refine_path=False), noise_parameters=None,
-                         use_tma=False)
+                         ego_staging='spans')
     return checker.pose_collides(np.asarray(poses, dtype=np.float64)).cpu().numpy()
 
 

@@ -196,9 +196,9 @@ class VecRandomAisleTurnEnv(_VecSlotEnv):
             if arr.dtype != TURN_DTYPE or arr.shape != (self.n_envs,):
                 raise ValueError("turn_params must hold one TurnParams per env")
             tp = self._to_device(arr.view(np.uint8).reshape(self.n_envs, TURN_DTYPE.itemsize))
-        nat.check(nat.lib().bcg_generate_aisles_rows(C.byref(self._c_params), C.byref(self._batch), self._rows,
-                                                     C.byref(self._slots), nat.ptr(m), nat.ptr(tp), self._draw_index,
-                                                     float(self.params.path_delta), self._stream()))
+        nat.check(nat.lib().bcg_generate_aisles(C.byref(self._c_params), C.byref(self._batch), self._rows,
+                                                C.byref(self._slots), nat.ptr(m), nat.ptr(tp), self._draw_index,
+                                                float(self.params.path_delta), self._stream()))
         self._draw_index += 1
         if tp is not None:
             torch.cuda.current_stream(self.device).synchronize()     # tp is released when this returns

@@ -109,7 +109,7 @@ class VecState(object):
 class VecPlanEnv(object):
     def __init__(self, costmaps, paths, params=None, n_envs=None, map_ids=None, path_ids=None,
                  noise_parameters=DEFAULT_NOISE, seed=0, auto_reset=False, device=None, env_id_base=0,
-                 private_map_copies=False, with_ego=False, footprint_scale=1.0, use_tma=True, footprint=None,
+                 private_map_copies=False, with_ego=False, footprint_scale=1.0, footprint=None,
                  ego_staging='tiles', ego_sparse=True, compact_ego=False, params_ids=None, episode_ends=False,
                  episode_end_capacity=None):
         """
@@ -150,8 +150,7 @@ class VecPlanEnv(object):
             np.count_nonzero(c.get_data()) * 20 > c.get_data().size for c in costmaps)
         self._compact_ego = bool(compact_ego)
         self._configure(params, n, float(costmaps[0].get_resolution()), noise_parameters, seed, auto_reset, device,
-                        env_id_base, with_ego, ego_staging if use_tma else 'spans', params_ids,   # use_tma=False: older spelling
-                        episode_ends, episode_end_capacity)
+                        env_id_base, with_ego, ego_staging, params_ids, episode_ends, episode_end_capacity)
         self._map_pool = costmaps
         self._map_ids_host = (np.arange(n) % len(costmaps)) if map_ids is None else np.asarray(map_ids, dtype=np.int64)
         self._path_ids_host = (np.arange(n) % len(paths)) if path_ids is None else np.asarray(path_ids, dtype=np.int64)
@@ -165,7 +164,7 @@ class VecPlanEnv(object):
         nat.check(nat.lib().bcg_build_lethal_tiles(C.byref(self._batch), 0, self._batch.n_maps, s))
         if self.cell_tile_arena is not None:
             nat.check(nat.lib().bcg_build_cell_tiles(C.byref(self._batch), 0, self._batch.n_maps, s))
-        nat.check(nat.lib().bcg_init_state_rows(C.byref(self._c_params), C.byref(self._batch), self._rows, s))
+        nat.check(nat.lib().bcg_init_state(C.byref(self._c_params), C.byref(self._batch), self._rows, s))
         self.check_status()
         if self._ego_list is not None:
             # bcg_build_lethal_tiles counted the occupied cells of every map: when none is above the library's dense
@@ -215,7 +214,6 @@ class VecPlanEnv(object):
         if ego_staging not in ('tiles', 'tma', 'spans'):
             raise ValueError("ego_staging must be 'tiles', 'tma' or 'spans'")
         self.ego_staging = ego_staging
-        self.use_tma = ego_staging == 'tma'
         self._step_index = 0
         self._graph = None
         self._plan_graph = None
@@ -407,7 +405,7 @@ class VecPlanEnv(object):
         self.state_i = torch.zeros((L.n_irows, n), dtype=torch.int32, device=dev)
         self.init_f = torch.zeros_like(self.state_f)
         self.init_i = torch.zeros_like(self.state_i)
-        self._cand = torch.zeros((9, n), dtype=torch.float64, device=dev)
+        self._cand = torch.zeros((3, n), dtype=torch.float64, device=dev)
         self._cand_i = torch.zeros((2, n), dtype=torch.int32, device=dev)
         self._work = torch.zeros((n, 192), dtype=torch.uint8, device=dev)
         self._ego_work = torch.zeros((n, 128), dtype=torch.uint8, device=dev)
@@ -497,7 +495,7 @@ class VecPlanEnv(object):
         if self.cell_tile_arena is not None and getattr(self, '_ego_sparse', True):
             self._ego_list = torch.zeros(self.n_envs + 4, dtype=torch.int32, device=self.device)
             b.ego_list = self._ego_list.data_ptr()
-        if self.use_tma:
+        if self.ego_staging == 'tma':
             b.map_tmaps, b.tmap_n_widths, b.tmap_box_h = self.map_tmaps.data_ptr(), len(self._tmap_widths), self._tmap_box_h
             for j, w in enumerate(self._tmap_widths):
                 b.tmap_box_w[j] = w
@@ -589,12 +587,16 @@ class VecPlanEnv(object):
     def step(self, actions):
         """One env step for every env.  actions: [N, 2] float32/float64 (tensor or ndarray).
         Returns (VecObservation, reward fp64 [N], done bool [N], {}) -- tensors are reused buffers."""
-        a = self._as_actions(actions)
-        nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
-                                          1 if a.dtype == torch.float64 else 0, self._step_index,
-                                          C.byref(self._out), self._ends, None, self._stream()))
+        self._bcg_step(self._as_actions(actions), self._step_index, self._stream())
         self._step_index += 1
         return self.observation(), self.reward, self.done, {}
+
+    def _bcg_step(self, actions, step_index, stream, events=None):
+        """One bcg_step call on this batch: actions a float32 / float64 [N, 2] device tensor, stream a c_void_p,
+        events None or the five cudaEvent_t handles."""
+        nat.check(nat.lib().bcg_step(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(actions),
+                                     1 if actions.dtype == torch.float64 else 0, step_index, C.byref(self._out), self._ends,
+                                     events, stream))
 
     def step_graph(self, actions=None):
         """`step` as ONE CUDA-graph launch: the first call captures the step's kernels (reading `self.actions`, a
@@ -615,9 +617,7 @@ class VecPlanEnv(object):
             g = torch.cuda.CUDAGraph()
             with torch.cuda.stream(side):
                 with torch.cuda.graph(g, stream=side):
-                    nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows,
-                                                      nat.ptr(self.actions), 0, 0, C.byref(self._out), self._ends, None,
-                                                      C.c_void_p(side.cuda_stream)))
+                    self._bcg_step(self.actions, 0, C.c_void_p(side.cuda_stream))
             torch.cuda.current_stream(self.device).wait_stream(side)
             self._graph = g
         elif actions is not None:
@@ -636,8 +636,8 @@ class VecPlanEnv(object):
             raise ValueError("plan must have shape [H, %d, 2]" % self.n_envs)
         plan = plan.to(torch.float32).contiguous()
         horizon = int(plan.shape[0])
-        nat.check(nat.lib().bcg_rollout_ends(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(plan), horizon,
-                                             self._step_index, C.byref(self._out), self._ends, self._stream()))
+        nat.check(nat.lib().bcg_rollout(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(plan), horizon,
+                                        self._step_index, C.byref(self._out), self._ends, self._stream()))
         self._step_index += horizon
 
     def rollout_graph(self, plan):
@@ -663,9 +663,7 @@ class VecPlanEnv(object):
             with torch.cuda.stream(side):
                 with torch.cuda.graph(g, stream=side):
                     for h in range(horizon):
-                        nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows,
-                                                          nat.ptr(buf[h]), 0, 0, C.byref(self._out), self._ends, None,
-                                                          C.c_void_p(side.cuda_stream)))
+                        self._bcg_step(buf[h], 0, C.c_void_p(side.cuda_stream))
             torch.cuda.current_stream(self.device).wait_stream(side)
             self._plan_graph = (horizon, g, buf)
         else:
@@ -684,12 +682,9 @@ class VecPlanEnv(object):
 
     def step_timed(self, actions, events):
         """`step` with five torch.cuda.Event (enable_timing=True, already recorded once so that their
-        handles exist; entries may be None) recorded around the kernels; see bcg_step_events."""
-        a = self._as_actions(actions)
+        handles exist; entries may be None) recorded around the kernels; see the `events` of bcg_step."""
         handles = (C.c_void_p * 5)(*[C.c_void_p(ev.cuda_event if ev is not None else None) for ev in events])
-        nat.check(nat.lib().bcg_step_ends(C.byref(self._c_params), C.byref(self._batch), self._rows, nat.ptr(a),
-                                          1 if a.dtype == torch.float64 else 0, self._step_index,
-                                          C.byref(self._out), self._ends, handles, self._stream()))
+        self._bcg_step(self._as_actions(actions), self._step_index, self._stream(), handles)
         self._step_index += 1
         return self.observation(), self.reward, self.done, {}
 
@@ -717,7 +712,7 @@ class VecPlanEnv(object):
                 upload=torch.cuda.Stream(device=self.device), uploaded=torch.cuda.Event(enable_timing=False),
                 events=[torch.cuda.Event(enable_timing=False) for _ in range(5)])
             for ev in self._host_io['events']:
-                ev.record()                                   # creates the handles bcg_step_events records into
+                ev.record()                                   # creates the handles bcg_step records into
         io = self._host_io
         if tuple(actions_host.shape) != (self.n_envs, 2) or actions_host.dtype != torch.float32:
             raise ValueError("actions_host must be a float32 tensor of shape (%d, 2)" % self.n_envs)

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define BCG_ABI_VERSION 11
+#define BCG_ABI_VERSION 12
 
 /* error codes */
 #define BCG_OK 0
@@ -193,8 +193,8 @@ typedef struct BcgBatch {
   int32_t* state_i;
   double* init_f;  /* the state reset() restores (env.py:247,302) */
   int32_t* init_i;
-  double* cand;    /* scratch [9][n_envs]: rows 0..2 = the pose the last step proposed (before the collision
-                      verdict); bcg_kinematic_step writes rows 0..6 (the proposed robot state)              */
+  double* cand;    /* scratch [3][n_envs]: the pose the last step proposed (before the collision verdict), written by
+                      move_kernel                                                                           */
   int32_t* cand_i; /* scratch [2][n_envs] (reserved; must be allocated)                                      */
   void* ego_work;  /* scratch [n_envs][128 bytes]: per-env affine map + source window of the egocentric crop,
                       written by move_kernel / reward_kernel (or bcg_observe_ego) for the egocentric kernel; may
@@ -304,7 +304,7 @@ typedef struct BcgEnvRows {
   const int32_t* i;  /* device [BCG_EP_I_ROWS][n_envs] */
 } BcgEnvRows;
 
-/* Episode ends of an auto-reset batch (bcg_step_ends / bcg_rollout_ends): why each env is done, and the observation of
+/* Episode ends of an auto-reset batch (bcg_step / bcg_rollout): why each env is done, and the observation of
  * every episode that ends at this step as it was before the in-kernel reset overwrote it.
  *
  * reason[e] is written for every env at every step:
@@ -391,11 +391,9 @@ int bcg_build_cell_tiles(const BcgBatch* b, int32_t first, int32_t count, void* 
 int bcg_encode_map_tensor_maps(const BcgMapDesc* maps_host, int32_t n_maps, const void* map_arena_dev,
                                const int32_t* box_w, int32_t n_widths, int32_t box_h, void* out_host);
 /* make_initial_state (env.py:179-214) + ContinuousRewardProvider.generate_initial_state
- * (reward.py:261-288) for every env: writes init_f/init_i and copies them into state_f/state_i */
-int bcg_init_state(const BcgParams* p, const BcgBatch* b, void* stream);
-/* bcg_init_state with per-env goal tolerances: env e's initial target index uses its own spatial / angular precision
- * from `rows` (NULL: bcg_init_state) */
-int bcg_init_state_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, void* stream);
+ * (reward.py:261-288) for every env: writes init_f/init_i and copies them into state_f/state_i.  With `rows` env e's
+ * initial target index uses its own spatial / angular precision (NULL: those of p). */
+int bcg_init_state(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, void* stream);
 /* PlanEnv.reset (env.py:293-303) for envs with mask[e] != 0 (mask NULL = all) */
 int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream);
 
@@ -405,14 +403,12 @@ int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream);
  * (path_and_costmap_from_config :110-192), refine the path (utilities/path_tools.py:178-240, spacing
  * `path_delta`), derive both tile planes, and make the initial state (env.py:179-214, reward.py:261-288).
  * The previous walls of the slot are erased pixel by pixel, so a reset costs O(wall pixels), not O(map).
+ * With `rows` the initial states use each env's own goal tolerances (NULL: those of p); rows changed before the call (a
+ * new parameter set at a reset) are what the new worlds' initial states see.
  * Not available together with TMA tensor maps (map_tmaps), which cannot be re-encoded on the device. */
-int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgAisleSlots* slots, const uint8_t* mask,
-                        const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta, void* stream);
-/* bcg_generate_aisles whose initial states use each env's own goal tolerances from `rows` (NULL: bcg_generate_aisles).
- * Rows changed before the call (a new parameter set at a reset) are what the new worlds' initial states see. */
-int bcg_generate_aisles_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
-                             const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
-                             void* stream);
+int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
+                        const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
+                        void* stream);
 
 /* RandomMiniEnv's env construction (envs/mini_env.py:323-389, what its reset repeats) on the device, for envs with
  * mask[e] != 0 (mask NULL = all), in the same per-env slots as bcg_generate_aisles: sample MiniEnvParams (:269-320,
@@ -437,40 +433,31 @@ int bcg_generate_minis(const BcgParams* p, const BcgBatch* b, const BcgAisleSlot
  * envs it hands over unless BCG_BATCH_SPARSE_EGO_ONLY, else one dense kernel.  Each kernel is launched as a programmatic
  * dependent of the one before it on `stream`.  step_index is the caller's global step counter (ignored when
  * BcgBatch.step_counter is set): odometry noise is Philox4x32-10 keyed by p->seed at counter (env id, step_index, draw),
- * replacing the reference's global np.random (differential_drive.py:50). */
-int bcg_step(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64,
-             uint64_t step_index, const BcgStepOut* out, void* stream);
-
-/* bcg_step with per-kernel hooks: events[0..4] are caller-created cudaEvent_t handles recorded on `stream`: [0], [1]
- * before move_kernel, [2] between move_kernel and reward_kernel, [3] after reward_kernel (reward / done / compact
- * observation are final: a host consumer's copies can start here while the egocentric kernel runs), [4] after the
- * egocentric kernels.  Any entry may be NULL (not recorded).  A kernel with an event recorded right before it is not
- * launched as a programmatic dependent of its predecessor.  events == NULL behaves exactly like bcg_step. */
-int bcg_step_events(const BcgParams* p, const BcgBatch* b, const void* actions, int32_t action_is_f64,
-                    uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream);
-
-/* bcg_step_events for a batch with per-env parameters (BcgEnvRows; NULL: bcg_step_events).  move_kernel reads env e's
- * delays, timeout, noise flag and alphas from the rows with its other top-of-kernel loads and forwards its goal tolerances
- * and progress multiplier to reward_kernel in the env's work slot.  Ring capacities are p's delays; a row delay above
- * its capacity is clamped to it (memory safety does not depend on the row contents; the host validates them). */
-int bcg_step_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
-                  uint64_t step_index, const BcgStepOut* out, void* const* events, void* stream);
-
-/* bcg_step_rows that also reports episode ends (BcgEpisodeEnds; NULL: bcg_step_rows).  Same launches: move_kernel zeroes
- * the counters, reward_kernel writes the reasons and final records and copies the egocentric records of the ended envs
- * before it resets them, and the egocentric kernels render the final crops after the step's own.  Final crops need the
- * cell-tile planes (BcgBatch.cell_tile_arena). */
-int bcg_step_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
-                  uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* const* events, void* stream);
+ * replacing the reference's global np.random (differential_drive.py:50).
+ *
+ * rows (BcgEnvRows; NULL: every env uses p): per-env parameters.  move_kernel reads env e's delays, timeout, noise flag
+ * and alphas from the rows with its other top-of-kernel loads and forwards its goal tolerances and progress multiplier
+ * to reward_kernel in the env's work slot.  Ring capacities are p's delays; a row delay above its capacity is clamped to
+ * it (memory safety does not depend on the row contents; the host validates them).
+ *
+ * ends (BcgEpisodeEnds; NULL: no episode ends are reported): the same launches also report episode ends.  move_kernel
+ * zeroes the counters, reward_kernel writes the reasons and final records and copies the egocentric records of the
+ * ended envs before it resets them, and the egocentric kernels render the final crops after the step's own.  Final
+ * crops need the cell-tile planes (BcgBatch.cell_tile_arena).
+ *
+ * events (NULL: none are recorded): per-kernel hooks, events[0..4] are caller-created cudaEvent_t handles recorded on
+ * `stream`: [0], [1] before move_kernel, [2] between move_kernel and reward_kernel, [3] after reward_kernel (reward /
+ * done / compact observation are final: a host consumer's copies can start here while the egocentric kernel runs), [4]
+ * after the egocentric kernels.  Any entry may be NULL (not recorded).  A kernel with an event recorded right before it
+ * is not launched as a programmatic dependent of its predecessor. */
+int bcg_step(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
+             uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* const* events, void* stream);
 
 /* the pieces, individually addressable (used by tests, ncu and the hook seam) */
-/* robot.step (tricycle_model.py:478-538 / differential_drive.py:236-265) into b->cand */
-int bcg_kinematic_step(const BcgParams* p, const BcgBatch* b, const void* actions,
-                       int32_t action_is_f64, uint64_t step_index, void* stream);
 /* pose_collides (env.py:464-489) of poses [3][n] (rows x,y,th) against each env's map, using the
  * lethal tile plane; flags_out [n].  pixels_out (optional, [n]) = in-map footprint pixel count (warp-per-env
  * kernel; without it the thread-per-env kernel the step itself uses).  poses == NULL checks the poses the last
- * bcg_step / bcg_kinematic_step proposed (rows 0..2 of b->cand).  Two launches: per-env work records (footprint
+ * bcg_step proposed (b->cand).  Two launches: per-env work records (footprint
  * angle bin, mask box, map references) into b->work, then the collision kernel. */
 int bcg_collision(const BcgParams* p, const BcgBatch* b, const double* poses, uint8_t* flags_out,
                   int32_t* pixels_out, void* stream);
@@ -525,15 +512,10 @@ int bcg_observe_ego_path(const BcgParams* p, const BcgBatch* b, int32_t max_poin
 /* H steps of a fixed action plan (Monte-Carlo fan-outs: the reference steps a copied env through a candidate plan,
  * README.md:45-61): bcg_step for plan[h], h = 0 .. horizon - 1, launched back to back from one call -- every kernel a
  * programmatic dependent of the one before, no host work in between.  plan: device float32 [horizon][n_envs][2];
- * step h uses the Philox step index step_index + h (or the device-side counter when BcgBatch.step_counter is set). */
-int bcg_rollout(const BcgParams* p, const BcgBatch* b, const float* plan, int32_t horizon, uint64_t step_index,
-                const BcgStepOut* out, void* stream);
-/* bcg_rollout for a batch with per-env parameters (see bcg_step_rows; rows NULL: bcg_rollout) */
-int bcg_rollout_rows(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
-                     uint64_t step_index, const BcgStepOut* out, void* stream);
-/* bcg_rollout_rows with episode ends (see bcg_step_ends; ends NULL: bcg_rollout_rows): `ends` describes the last step */
-int bcg_rollout_ends(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
-                     uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* stream);
+ * step h uses the Philox step index step_index + h (or the device-side counter when BcgBatch.step_counter is set).
+ * rows and ends as for bcg_step (either may be NULL); `ends` describes the last step. */
+int bcg_rollout(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const float* plan, int32_t horizon,
+                uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* stream);
 
 /* -- image memory --------------------------------------------------------------------------------
  * Egocentric crops are mostly zeros.  A device allocation with compute-data compression (CUDA virtual memory

@@ -113,7 +113,7 @@ def test_two_point_path_and_stepping_after_the_goal():
     env.check_status()
 
 
-def test_malformed_calls_return_error_codes():
+def test_malformed_step_calls_return_error_codes():
     """The C entry points report bad arguments through their return code and bcg_last_error -- nothing is thrown,
     nothing is launched."""
     env, _ = _build(_tiny_worlds())
@@ -121,8 +121,8 @@ def test_malformed_calls_return_error_codes():
     s = env._stream()
     a = torch.zeros((env.n_envs, 2), dtype=torch.float32, device="cuda")
     before = env.state_f.clone()
-    assert lib.bcg_step(C.byref(env._c_params), C.byref(env._batch), None, 0, 0, C.byref(env._out), s) < 0
-    assert lib.bcg_step(C.byref(env._c_params), C.byref(env._batch), nat.ptr(a), 0, 0, None, s) < 0
+    assert lib.bcg_step(C.byref(env._c_params), C.byref(env._batch), None, None, 0, 0, C.byref(env._out), None, None, s) < 0
+    assert lib.bcg_step(C.byref(env._c_params), C.byref(env._batch), None, nat.ptr(a), 0, 0, None, None, None, s) < 0
     assert "null" in nat.last_error()
     assert lib.bcg_observe_ego(C.byref(env._c_params), C.byref(env._batch), None, None, s) < 0
     torch.cuda.synchronize()

@@ -17,14 +17,24 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(bcg_[a-z0-9_]+)\s*\(", text)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_the_declared_abi():
     lib = nat.lib()
     declared = _declared_symbols()
     assert len(declared) >= 18
     for name in declared:
         assert hasattr(lib, name), "libbcg_b200.so does not export %s" % name
     assert sorted(nat.SYMBOLS) == declared, "ctypes binding and header disagree"
-    assert lib.bcg_abi_version() == 11
+    assert lib.bcg_abi_version() == 12
+
+
+def test_one_entry_point_per_operation():
+    # bcg_step, bcg_rollout, bcg_init_state and bcg_generate_aisles take NULL rows / ends / events themselves: no
+    # suffixed variant of them is exported, and no stand-alone kinematics step
+    lib = nat.lib()
+    for name in ("bcg_init_state_rows", "bcg_generate_aisles_rows", "bcg_step_events", "bcg_step_rows", "bcg_step_ends",
+                 "bcg_rollout_rows", "bcg_rollout_ends", "bcg_kinematic_step"):
+        assert not hasattr(lib, name), "libbcg_b200.so still exports %s" % name
+        assert name not in nat.SYMBOLS
 
 
 def test_struct_mirrors_match_library():
@@ -44,13 +54,13 @@ def test_state_layout_follows_delays():
         nat.state_layout(nat.BcgParams(delay_pose=-1))
 
 
-def test_errors_are_reported_not_thrown():
+def test_bad_arguments_return_error_codes():
     lib = nat.lib()
-    assert lib.bcg_step(None, None, None, 0, 0, None, None) < 0
+    assert lib.bcg_step(None, None, None, None, 0, 0, None, None, None, None) < 0
     assert "null" in nat.last_error()
     assert lib.bcg_world_to_pixel(None, 4, 0.0, 0.0, 0.05, None, None) < 0
     p, b = nat.BcgParams(), nat.BcgBatch()
-    assert lib.bcg_step(C.byref(p), C.byref(b), None, 0, 0, None, None) < 0
+    assert lib.bcg_step(C.byref(p), C.byref(b), None, None, 0, 0, None, None, None, None) < 0
     assert "n_envs" in nat.last_error()
 
 
