@@ -64,8 +64,6 @@ class BcgBatch(C.Structure):
         ("maps", C.c_void_p), ("paths", C.c_void_p),
         ("map_arena", C.c_void_p), ("tile_arena", C.c_void_p), ("path_arena", C.c_void_p),
         ("lut", BcgFootprintLut),
-        ("map_tmaps", C.c_void_p), ("tmap_n_widths", C.c_int32), ("tmap_box_h", C.c_int32),
-        ("tmap_box_w", C.c_int32 * 4),
         ("cell_tile_arena", C.c_void_p), ("occ_tile_arena", C.c_void_p), ("ego_list", C.c_void_p),
         ("occ_sum_arena", C.c_void_p), ("status", C.c_void_p), ("stats", C.c_void_p), ("step_counter", C.c_void_p),
     ]
@@ -155,8 +153,6 @@ SYMBOLS = {
     "bcg_state_layout": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgStateLayout)]),
     "bcg_build_lethal_tiles": (C.c_int, [C.POINTER(BcgBatch), C.c_int32, C.c_int32, _P]),
     "bcg_build_cell_tiles": (C.c_int, [C.POINTER(BcgBatch), C.c_int32, C.c_int32, _P]),
-    "bcg_encode_map_tensor_maps": (C.c_int, [C.POINTER(BcgMapDesc), C.c_int32, _P, C.POINTER(C.c_int32), C.c_int32,
-                                             C.c_int32, _P]),
     "bcg_init_state": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows), _P]),
     "bcg_generate_aisles": (C.c_int, [C.POINTER(BcgParams), C.POINTER(BcgBatch), C.POINTER(BcgEnvRows),
                                       C.POINTER(BcgAisleSlots), _P, _P, C.c_uint64, C.c_double, _P]),

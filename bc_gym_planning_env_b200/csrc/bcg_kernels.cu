@@ -15,7 +15,6 @@
 // the stand-alone entry points of the hook seam.
 // No tensor cores: nothing here is a dense contraction.
 #include <cuda.h>
-#include <cudaTypedefs.h>
 #include <cuda_runtime.h>
 
 #include <cstddef>
@@ -153,7 +152,6 @@ int check_rows(const BcgEnvRows* rows) {
 int check_slots(const BcgParams* p, const BcgBatch* b, const BcgAisleSlots* slots, double path_delta, const char* who) {
   BCG_REQUIRE(slots && slots->gen_state, "null slots / gen_state");
   BCG_REQUIRE(b->cell_tile_arena, std::string(who) + " needs the cell-tile arena");
-  BCG_REQUIRE(!b->map_tmaps, std::string(who) + " cannot re-encode TMA tensor maps; use cell-tile or plain-load staging");
   BCG_REQUIRE(b->n_maps == b->n_envs && b->n_paths == b->n_envs, "device-generated envs own one map and one path slot each");
   BCG_REQUIRE(slots->map_slot_bytes > 0 && slots->tile_slot_words > 0 && slots->path_pitch >= 8 && slots->path_pitch % 4 == 0 &&
                   slots->chunk_pitch * 32 >= slots->path_pitch,
@@ -175,17 +173,7 @@ __global__ void __launch_bounds__(128) pose_prep_kernel(const BcgParams p, const
   *reinterpret_cast<WorkCollide*>(rec) = make_work_collide(p, b, b.map_id[e], poses[e], poses[N + e], poses[2 * N + e]);
 }
 
-// cv2::saturate_cast<int>(double) == cvRound with saturation
-__device__ __forceinline__ int cv_round_sat(double v) {
-  const double r = rint(v);
-  if (r >= 2147483647.0) return 2147483647;
-  if (r <= -2147483648.0) return (-2147483647 - 1);
-  return (int)r;
-}
-
 #define BCG_EGO_MAX 256
-#define BCG_EGO_THREADS 256
-#define BCG_EGO_MAX_TILE_ROWS 384
 
 struct EgoAffine {
   double a11, a12, b1, a21, a22, b2;   // source = A * (u, v) + b, cv::warpAffine's inverted map
@@ -270,115 +258,9 @@ __device__ __forceinline__ void write_goal_n_state(const BcgParams& p, const Bcg
   g[8] = (float)drobot[6];
 }
 
-// Per-env record the egocentric kernel starts from, resolved one thread per env (commit / prep kernel):
-// the inverted affine map, the source window and how to stage it.
-struct __align__(16) EgoWork {       // 128 bytes
-  EgoAffine aff;                     // 48
-  int32_t x0, x1, y0, y1;            // source window, not clipped to the map (x0 floored to 16 px for TMA)
-  int32_t cls, mode;                 // TMA box-width class; 0 direct, 1 TMA, 2 plain-load spans
-  int64_t data_off;                  // uint8 cells of the env's map
-  int32_t map_w, map_h, map_pitch, map_id;
-  int32_t pad[8];
-};
-static_assert(sizeof(EgoWork) == 128, "EgoWork records are 128 bytes");
 #define BCG_EGO_MODE_DIRECT 0
-#define BCG_EGO_MODE_TMA 1
-#define BCG_EGO_MODE_SPANS 2
 #define BCG_EGO_MODE_TILES 3
-#define BCG_EGO_WORK_BYTES 128        // stride of the per-env records in BcgBatch.ego_work (EgoWork / EgoTileWork)
-
-__device__ __forceinline__ EgoWork make_ego_work(const BcgParams& p, const BcgBatch& b, int map_id, const BcgMapDesc& m,
-                                                 double px, double py, double pth, int tile_capacity) {
-  EgoWork w;
-  w.aff = ego_affine(p, m, px, py, pth);
-  w.data_off = m.data_off;
-  w.map_w = m.width;
-  w.map_h = m.height;
-  w.map_pitch = m.pitch;
-  w.map_id = map_id;
-  w.cls = 0;
-  w.mode = BCG_EGO_MODE_DIRECT;
-  w.x0 = w.x1 = w.y0 = w.y1 = 0;
-
-  // Source window: every sample is X = floor(x + 0.5 + d), |d| <= 2^-10, of a point x of the rotated crop
-  // rectangle, so the rectangle's corners grown by 0.51 px bound all samples.
-  const EgoAffine& A = w.aff;
-  const double uw = (double)(p.ego_w - 1), vh = (double)(p.ego_h - 1);
-  const double cx[4] = {A.b1, A.a11 * uw + A.b1, A.a11 * uw + A.a12 * vh + A.b1, A.a12 * vh + A.b1};
-  const double cy[4] = {A.b2, A.a21 * uw + A.b2, A.a21 * uw + A.a22 * vh + A.b2, A.a22 * vh + A.b2};
-  const double lim = 1048576.0;
-  const double xlo = fmin(fmin(cx[0], cx[1]), fmin(cx[2], cx[3])), xhi = fmax(fmax(cx[0], cx[1]), fmax(cx[2], cx[3]));
-  const double ylo = fmin(fmin(cy[0], cy[1]), fmin(cy[2], cy[3])), yhi = fmax(fmax(cy[0], cy[1]), fmax(cy[2], cy[3]));
-  const bool sane = p.ego_w <= 128 && xlo > -lim && xhi < lim && ylo > -lim && yhi < lim;   // false for NaN too
-  if (!sane) return w;
-  w.x0 = (int)floor(xlo - 0.51);
-  w.x1 = (int)ceil(xhi + 0.51);
-  w.y0 = (int)floor(ylo - 0.51);
-  w.y1 = (int)ceil(yhi + 0.51);
-  const int bh = w.y1 - w.y0 + 1;
-  w.mode = BCG_EGO_MODE_SPANS;
-  if (b.map_tmaps) {
-    // the innermost start coordinate of a box must land on a 16-byte boundary (misaligned starts raise
-    // an illegal-instruction fault on sm_100a), so the window's left edge is floored to 16 pixels
-    const int x0a = w.x0 & ~15;
-    const int bw = w.x1 - x0a + 1;
-    int cls = 0;
-    while (cls < b.tmap_n_widths && b.tmap_box_w[cls] < bw) ++cls;
-    const int nops = (bh + b.tmap_box_h - 1) / b.tmap_box_h;
-    if (cls < b.tmap_n_widths && nops * b.tmap_box_h * b.tmap_box_w[cls] <= tile_capacity) {
-      w.mode = BCG_EGO_MODE_TMA;
-      w.cls = cls;
-      w.x0 = x0a;
-    }
-  }
-  if (w.mode == BCG_EGO_MODE_SPANS) {
-    const int x0w = w.x0 & ~3;                        // left edge on a 4-byte word
-    const int pitch_w = ((w.x1 - x0w + 1 + 3) >> 2) | 1;
-    if (bh <= BCG_EGO_MAX_TILE_ROWS && (long long)pitch_w * 4 * bh <= tile_capacity) w.x0 = x0w;
-    else w.mode = BCG_EGO_MODE_DIRECT;
-  }
-  return w;
-}
-
-// shared-memory tile the egocentric kernel is launched with (bytes): worst-case source window of the crop
-__host__ __device__ inline int ego_tile_capacity(const BcgParams& p, const BcgBatch& b) {
-  const int side = (int)ceil(sqrt((double)p.ego_w * p.ego_w + (double)p.ego_h * p.ego_h)) + 2;
-  int cap = (side + 1) * ((((side + 3) + 3) / 4) | 1) * 4;
-  if (b.map_tmaps && b.tmap_n_widths >= 1 && b.tmap_box_h > 0) {
-    const int rows = ((side + 1 + b.tmap_box_h - 1) / b.tmap_box_h) * b.tmap_box_h;
-    const int tma_cap = rows * b.tmap_box_w[b.tmap_n_widths - 1];
-    if (tma_cap > cap) cap = tma_cap;
-  }
-  cap = (cap + 127) / 128 * 128;
-  if (cap > 42 * 1024) cap = 42 * 1024;   // larger crops fall back to the direct global gather per CTA
-  return cap;
-}
-
-// x-extent of a convex quad within the horizontal band [ylo, yhi]; extremes lie on the boundary
-__device__ __forceinline__ void quad_band_extent(const double qx[4], const double qy[4], double ylo, double yhi,
-                                                 double& xmin, double& xmax) {
-  xmin = 1e300;
-  xmax = -1e300;
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const double xa = qx[k], ya = qy[k], xb = qx[(k + 1) & 3], yb = qy[(k + 1) & 3];
-    double t0 = 0.0, t1 = 1.0;
-    const double dy = yb - ya;
-    if (dy == 0.0) {
-      if (ya < ylo || ya > yhi) continue;
-    } else {
-      double ta = (ylo - ya) / dy, tb = (yhi - ya) / dy;
-      if (ta > tb) { const double t = ta; ta = tb; tb = t; }
-      t0 = fmax(ta, 0.0);
-      t1 = fmin(tb, 1.0);
-      if (t0 > t1) continue;
-    }
-    const double x0 = xa + (xb - xa) * t0, x1 = xa + (xb - xa) * t1;
-    xmin = fmin(xmin, fmin(x0, x1));
-    xmax = fmax(xmax, fmax(x0, x1));
-  }
-}
-
+#define BCG_EGO_WORK_BYTES 128        // stride of the per-env records in BcgBatch.ego_work (EgoTileWork)
 
 // Record of the persistent cell-tile egocentric kernel (ego_tiles_kernel), resolved one thread per env: the
 // inverted affine map, the tile-aligned source window and, per row of cell tiles, which tiles the rotated crop
@@ -529,17 +411,6 @@ __device__ __forceinline__ uint32_t ego_band_span(const EgoAffine& A, int ego_w,
     te = min((int)ceilf(xmax + M) >> 4, ntx - 1);
   }
   return (uint32_t)(ts | (te << 8));
-}
-
-// the per-env record of whichever egocentric kernel the batch is set up for
-__device__ __forceinline__ void write_ego_record(const BcgParams& p, const BcgBatch& b, int e, int map_id,
-                                                 const BcgMapDesc& m, double px, double py, double pth, int cap) {
-  if (b.cell_tile_arena) {
-    write_ego_tile_record(p, b, e, map_id, m, px, py, pth, cap);
-  } else {
-    *reinterpret_cast<EgoWork*>(reinterpret_cast<uint8_t*>(b.ego_work) + (int64_t)e * BCG_EGO_WORK_BYTES) =
-        make_ego_work(p, b, map_id, m, px, py, pth, cap);
-  }
 }
 
 // ---- the two state kernels of a step --------------------------------------------------------------------------------
@@ -792,7 +663,7 @@ move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, c
   // ---- what reward_kernel starts from ----------------------------------------------------------------------------------------
   const bool true_pose = p.ego_variant == 1;             // observation about the true robot pose vs the observed (delayed) pose
   const double opx = true_pose ? s[0] : dpose[0], opy = true_pose ? s[1] : dpose[1], opth = true_pose ? s[2] : dpose[2];
-  if (out.ego_image) write_ego_record(p, b, e, map_id, m, opx, opy, opth, ego_cap);
+  if (out.ego_image) write_ego_tile_record(p, b, e, map_id, m, opx, opy, opth, ego_cap);
   rec.ct = rec.st = rec.tx = rec.ty = rec.tt = 0.0;
   if (out.goal_n_state) inverse_transform(opx, opy, opth, rec.ct, rec.st, rec.tx, rec.ty, rec.tt);
 #pragma unroll
@@ -859,7 +730,7 @@ __device__ __forceinline__ void reset_env_rows(const BcgParams& p, const BcgBatc
     const double opx = true_pose ? c[0] : dpose[0], opy = true_pose ? c[1] : dpose[1], opth = true_pose ? c[2] : dpose[2];
     if (out.ego_image) {
       const int map_id = b.map_id[e];
-      write_ego_record(p, b, e, map_id, b.maps[map_id], opx, opy, opth, ego_cap);
+      write_ego_tile_record(p, b, e, map_id, b.maps[map_id], opx, opy, opth, ego_cap);
     }
     if (out.goal_n_state) write_goal_n_state(p, b, e, b.paths[b.path_id[e]], opx, opy, opth, target, dstate, out.goal_n_state);
   }
@@ -1539,40 +1410,8 @@ __global__ void __launch_bounds__(64) collision_thread_kernel(const BcgBatch b, 
 #endif
 }
 
-// ---- TMA / mbarrier primitives (sm_90+ PTX; SASS: UTMALDG, SYNCS) ------------------------------------
+// ---- shared-memory and cp.async primitives ----------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t mbar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(mbar), "r"(count) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-
-__device__ __forceinline__ void mbar_expect_tx(uint32_t mbar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(bytes) : "memory");
-}
-
-__device__ __forceinline__ void mbar_wait(uint32_t mbar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "BCG_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra BCG_DONE;\n"
-      "bra BCG_WAIT;\n"
-      "BCG_DONE:\n"
-      "}\n" ::"r"(mbar),
-      "r"(parity)
-      : "memory");
-}
-
-// one 2-D box of a uint8 costmap -> shared memory; out-of-map elements arrive as 0
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const void* tmap, int x, int y, uint32_t mbar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
-      "l"(tmap), "r"(x), "r"(y), "r"(mbar)
-      : "memory");
-}
 
 // 16 bytes global -> shared without passing through registers (SASS: LDGSTS); src_bytes 0 writes zeros
 __device__ __forceinline__ void cp_async_16(uint32_t dst, const void* src, uint32_t src_bytes) {
@@ -1588,142 +1427,12 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t addr) {
   return v;
 }
 
-// EgocentricCostmap.observation (envs/egocentric.py:125-160): extract_egocentric_costmap
-// (utilities/costmap_utils.py:25-75) = cv2.getRotationMatrix2D composed in float32 with the crop
-// shift, then cv2.warpAffine(INTER_NEAREST, borderValue=0): fp64 inverse and 10-bit fixed-point source
-// coordinates X = (rint(A11 u 2^10) + rint((A12 v + b1) 2^10) + 512) >> 10 (SURVEY.md A.9).
-//
-// One CTA per env, starting from the env's EgoWork record (affine map + source window, resolved one
-// thread per env by the commit / prep kernel).  The source pixels of the crop lie in a rotated rectangle
-// whose bounding box is staged into shared memory, zero outside the map (= borderValue); the rotated
-// gather then runs out of shared memory with no bounds checks.  Two ways to stage:
-//   * TMA (b.map_tmaps set): thread 0 issues ceil(rows / box_h) cp.async.bulk.tensor.2d box loads on an
-//     mbarrier right away; the copy engine does the address generation and the out-of-map zero fill
-//     while the CTA builds its fixed-point tables;
-//   * plain loads: per source row only the span of the rotated rectangle (grown by the 0.501 px the
-//     fixed-point rounding can move a sample) is loaded with coalesced 4-byte words.
-// Tile pitches: 144/176/208 B for TMA boxes, 4 * odd otherwise -- all measured at < 2 shared-memory
-// wavefronts per gather averaged over crop angles.
-__global__ void __launch_bounds__(BCG_EGO_THREADS, 5) ego_kernel(const BcgParams p, const BcgBatch b,
-                                                                 uint8_t* __restrict__ image,
-                                                                 const int tile_capacity) {
-  extern __shared__ __align__(128) uint8_t tile_raw[];
-  // TMA destinations must be 128-byte aligned; the launch reserves the slack
-  uint8_t* const tile = tile_raw + ((128u - (smem_u32(tile_raw) & 127u)) & 127u);
-  __shared__ int adx[BCG_EGO_MAX], ady[BCG_EGO_MAX], bdx[BCG_EGO_MAX], bdy[BCG_EGO_MAX];
-  // per-row spans of the plain-load path live behind the tile (that path never needs the whole capacity)
-  short2* const span = reinterpret_cast<short2*>(tile + tile_capacity);
-  __shared__ __align__(8) uint64_t mbar_s;
-  const int e = blockIdx.x;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarp = blockDim.x >> 5;
-  const uint32_t mbar = smem_u32(&mbar_s);
-  const EgoWork w = *reinterpret_cast<const EgoWork*>(reinterpret_cast<const uint8_t*>(b.ego_work) + (int64_t)e * BCG_EGO_WORK_BYTES);   // warp-uniform 128-byte read
-  const EgoAffine A = w.aff;
-  int mode = w.mode;
-  const int X0 = w.x0, Y0 = w.y0;
-  const int bh = w.y1 - Y0 + 1;
-  int pitch_b = 0;
-
-  if (mode == BCG_EGO_MODE_TMA) {
-    pitch_b = b.tmap_box_w[w.cls];
-    if (threadIdx.x == 0) {
-      const int nops = (bh + b.tmap_box_h - 1) / b.tmap_box_h;
-      const int box_bytes = pitch_b * b.tmap_box_h;
-      const uint8_t* tmap = reinterpret_cast<const uint8_t*>(b.map_tmaps) + ((int64_t)w.map_id * b.tmap_n_widths + w.cls) * 128;
-      mbar_init(mbar, 1);
-      mbar_expect_tx(mbar, (uint32_t)(nops * box_bytes));
-      const uint32_t t0 = smem_u32(tile);
-      for (int k = 0; k < nops; ++k) tma_load_2d(t0 + k * box_bytes, tmap, X0, Y0 + k * b.tmap_box_h, mbar);
-    }
-  }
-  // the copy engine is now filling the tile; meanwhile every thread builds the fixed-point tables
-  for (int t = threadIdx.x; t < p.ego_w; t += blockDim.x) {
-    adx[t] = cv_round_sat(A.a11 * t * 1024);
-    ady[t] = cv_round_sat(A.a21 * t * 1024);
-  }
-  for (int t = threadIdx.x; t < p.ego_h; t += blockDim.x) {
-    bdx[t] = cv_round_sat((A.a12 * t + A.b1) * 1024) + 512;
-    bdy[t] = cv_round_sat((A.a22 * t + A.b2) * 1024) + 512;
-  }
-  const uint8_t* src = b.map_arena + w.data_off;
-  const int npx = p.ego_w * p.ego_h;
-  uint8_t* dst = image + (int64_t)e * npx;
-  if (mode == BCG_EGO_MODE_SPANS) {
-    // ---- plain-load staging: per-row span of the rotated crop rectangle ------------------------------------
-    const int bw = w.x1 - X0 + 1;                     // X0 is a multiple of 4 here
-    const int pitch_w = ((bw + 3) >> 2) | 1;          // words per tile row, odd
-    pitch_b = pitch_w * 4;
-    const double uw = (double)(p.ego_w - 1), vh = (double)(p.ego_h - 1);
-    const double qx[4] = {A.b1, A.a11 * uw + A.b1, A.a11 * uw + A.a12 * vh + A.b1, A.a12 * vh + A.b1};
-    const double qy[4] = {A.b2, A.a21 * uw + A.b2, A.a21 * uw + A.a22 * vh + A.b2, A.a22 * vh + A.b2};
-    for (int y = threadIdx.x; y < bh; y += blockDim.x) {
-      double xmin, xmax;
-      quad_band_extent(qx, qy, (double)(Y0 + y) - 0.51, (double)(Y0 + y) + 0.51, xmin, xmax);
-      int xs = 1, xe = 0;
-      if (xmin <= xmax) {
-        xs = max((int)floor(xmin - 0.51) - X0, 0);
-        xe = min((int)ceil(xmax + 0.51) - X0, bw - 1);
-      }
-      span[y] = make_short2((short)xs, (short)xe);
-    }
-    __syncthreads();
-    uint32_t* tw = reinterpret_cast<uint32_t*>(tile);
-    for (int y = warp; y < bh; y += nwarp) {
-      const short2 sp = span[y];
-      if (sp.x > sp.y) continue;
-      const int Ys = Y0 + y;
-      const bool row_in = Ys >= 0 && Ys < w.map_h;
-      // X0 is a multiple of 4 and the row pitch of 32: word loads are aligned and never straddle the map edge
-      const uint32_t* srow = reinterpret_cast<const uint32_t*>(src + (int64_t)(row_in ? Ys : 0) * w.map_pitch);
-      for (int xw = (sp.x >> 2) + lane; xw <= (sp.y >> 2); xw += 32) {
-        const int Xs = X0 + (xw << 2);
-        uint32_t word = 0u;
-        if (row_in && Xs >= 0 && Xs < w.map_pitch) word = __ldg(srow + (Xs >> 2));
-        tw[y * pitch_w + xw] = word;
-      }
-    }
-  }
-  __syncthreads();                       // tables (and the plain-load tile) are complete, the mbarrier is initialised
-  if (mode == BCG_EGO_MODE_TMA) mbar_wait(mbar, 0);
-  if (mode != BCG_EGO_MODE_DIRECT) {
-    // ---- gather: warp w takes crop rows w, w+8, ...; lane l takes columns l, l+32, l+64, l+96 -----------
-    int ax[4], ay[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int u = min(lane + 32 * k, p.ego_w - 1);
-      ax[k] = adx[u] - (X0 << 10);
-      ay[k] = ady[u] - (Y0 << 10);
-    }
-    const uint32_t tbase = smem_u32(tile);
-    const int n_full = p.ego_w >> 5;                 // column groups in which every lane is live
-    uint8_t* drow = dst + (int64_t)warp * p.ego_w + lane;
-    const int row_step = nwarp * p.ego_w;
-    for (int v = warp; v < p.ego_h; v += nwarp, drow += row_step) {
-      const int bx = bdx[v], by = bdy[v];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const int Xr = (ax[k] + bx) >> 10, Yr = (ay[k] + by) >> 10;
-        const uint32_t val = lds_u8(tbase + Yr * pitch_b + Xr);
-        if (k < n_full || lane + 32 * k < p.ego_w) drow[32 * k] = (uint8_t)val;
-      }
-    }
-  } else {
-    // generic path (huge crops / poses far outside any sane range): direct, bounds-checked global gather
-    for (int i = threadIdx.x; i < npx; i += blockDim.x) {
-      const int v = i / p.ego_w, u = i - v * p.ego_w;
-      const long long X = ((long long)adx[u] + bdx[v]) >> 10, Y = ((long long)ady[u] + bdy[v]) >> 10;
-      uint8_t val = 0;
-      if (X >= 0 && X < w.map_w && Y >= 0 && Y < w.map_h) val = __ldg(src + Y * w.map_pitch + X);
-      dst[i] = val;
-    }
-  }
-}
-
 // ---- cell-tile egocentric kernel ----------------------------------------------------------------------------
-// Same observation as ego_kernel (EgocentricCostmap.observation, envs/egocentric.py:125-160 ->
-// extract_egocentric_costmap, utilities/costmap_utils.py:25-75 -> cv2.warpAffine INTER_NEAREST), half the HBM
-// traffic: the source window is staged from the cell tiles (BcgMapDesc), and only the 128-byte tiles the rotated
-// crop rectangle touches are read (the per-row tile spans come with the env's EgoTileWork record).
+// EgocentricCostmap.observation (envs/egocentric.py:125-160): extract_egocentric_costmap (utilities/costmap_utils.py:25-75)
+// = cv2.getRotationMatrix2D composed in float32 with the crop shift, then cv2.warpAffine(INTER_NEAREST, borderValue=0):
+// fp64 inverse and 10-bit fixed-point source coordinates X = (rint(A11 u 2^10) + rint((A12 v + b1) 2^10) + 512) >> 10
+// (SURVEY.md A.9).  The source window is staged from the cell tiles (BcgMapDesc), and only the 128-byte tiles the
+// rotated crop rectangle touches are read (the per-row tile spans come with the env's EgoTileWork record).
 // Persistent CTAs, 5 per SM for the 133 x 117 crop (one 39 KB window each), walking envs blockIdx.x, + gridDim.x, ...;
 // the CTAs of an SM overlap each other's load and gather phases.  Per env: 16-byte pieces of the tiles -> registers ->
 // the row-major shared-memory window (zeros outside the map = borderValue), fixed-point tables, barrier, rotated
@@ -1846,7 +1555,7 @@ __global__ void __launch_bounds__(BCG_EGT_THREADS, BCG_EGT_CTAS) ego_tiles_kerne
     // ---- fixed-point tables of the crop (cv::warpAffine: saturate_cast<int> == cvt.rni with saturation) -------------
     {
       const EgoAffine A = r->aff;
-      for (int t = tid; t < ego_w; t += NT) {
+      for (int t = tid; t < min(ego_w, BCG_EGT_MAX_W); t += NT) {     // wider crops: direct mode, which needs no column table
         T.adx[t] = __double2int_rn(A.a11 * t * 1024);
         T.ady[t] = __double2int_rn(A.a21 * t * 1024);
       }
@@ -1882,13 +1591,16 @@ __global__ void __launch_bounds__(BCG_EGT_THREADS, BCG_EGT_CTAS) ego_tiles_kerne
         if (last_live) d0[32 * (NG - 1)] = (uint8_t)v0[NG - 1];
       }
     } else {
-      // crops too large for the window / poses far outside any sane range: bounds-checked global gather
+      // crops too large for the window / poses far outside any sane range: bounds-checked global gather, with the column
+      // terms computed in place (crops wider than the column table come this way)
       const BcgMapDesc m = b.maps[map_id];
       const uint8_t* src = b.map_arena + m.data_off;
+      const double a11 = r->aff.a11, a21 = r->aff.a21;
       for (int i = tid; i < npx; i += NT) {
         const int vv = i / ego_w, u = i - vv * ego_w;
         const int2 bb = T.bxy[vv];
-        const long long X = ((long long)T.adx[u] + bb.x) >> 10, Y = ((long long)T.ady[u] + bb.y) >> 10;
+        const long long X = ((long long)__double2int_rn(a11 * u * 1024) + bb.x) >> 10;
+        const long long Y = ((long long)__double2int_rn(a21 * u * 1024) + bb.y) >> 10;
         uint8_t val = 0;
         if (X >= 0 && X < m.width && Y >= 0 && Y < m.height) val = __ldg(src + Y * m.pitch + X);
         dst[i] = val;
@@ -2502,7 +2214,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
   }
 }
 
-// EgoWork records and / or goal_n_state from the current state (stand-alone bcg_observe_ego): one thread per env
+// egocentric records and / or goal_n_state from the current state (stand-alone bcg_observe_ego): one thread per env
 __global__ void __launch_bounds__(128) ego_prep_kernel(const BcgParams p, const BcgBatch b, const int want_image,
                                                        float* __restrict__ goal_n_state, const int ego_cap) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -2513,7 +2225,7 @@ __global__ void __launch_bounds__(128) ego_prep_kernel(const BcgParams p, const 
   const double px = sf[(prow + 0) * N], py = sf[(prow + 1) * N], pth = sf[(prow + 2) * N];
   if (want_image) {
     const int map_id = b.map_id[e];
-    write_ego_record(p, b, e, map_id, b.maps[map_id], px, py, pth, ego_cap);
+    write_ego_tile_record(p, b, e, map_id, b.maps[map_id], px, py, pth, ego_cap);
   }
   if (e == 0 && b.ego_list) b.ego_list[N] = b.ego_list[N + 1] = 0;       // hand-over count, env counter of the sparse kernel
   if (goal_n_state) {
@@ -2807,43 +2519,6 @@ int bcg_free_image_memory(void* dptr, int64_t mapped_bytes) {
   return BCG_OK;
 }
 
-int bcg_encode_map_tensor_maps(const BcgMapDesc* maps_host, int32_t n_maps, const void* map_arena_dev,
-                               const int32_t* box_w, int32_t n_widths, int32_t box_h, void* out_host) {
-  BCG_REQUIRE(maps_host && map_arena_dev && out_host && box_w && n_maps >= 0, "null argument");
-  BCG_REQUIRE(n_widths >= 1 && n_widths <= 4 && box_h > 0 && box_h <= 256, "bad TMA box");
-  for (int j = 0; j < n_widths; ++j)
-    BCG_REQUIRE(box_w[j] > 0 && box_w[j] <= 256 && box_w[j] % 16 == 0 && (j == 0 || box_w[j] > box_w[j - 1]),
-                "TMA box widths must be ascending multiples of 16, at most 256");
-  static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    BCG_CHECK_CUDA(cudaGetDriverEntryPointByVersion("cuTensorMapEncodeTiled", &fn, 12000, cudaEnableDefault, &qres));
-    if (!fn || qres != cudaDriverEntryPointSuccess) return fail(BCG_ERR_CUDA, "cuTensorMapEncodeTiled not available");
-    encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-  }
-  CUtensorMap* out = reinterpret_cast<CUtensorMap*>(out_host);
-  static_assert(sizeof(CUtensorMap) == 128, "tensor maps are 128 bytes");
-  for (int32_t k = 0; k < n_maps; ++k) {
-    const BcgMapDesc& m = maps_host[k];
-    const cuuint64_t dims[2] = {(cuuint64_t)m.width, (cuuint64_t)m.height};
-    const cuuint64_t strides[1] = {(cuuint64_t)m.pitch};
-    const cuuint32_t estr[2] = {1, 1};
-    for (int j = 0; j < n_widths; ++j) {
-      const cuuint32_t boxd[2] = {(cuuint32_t)box_w[j], (cuuint32_t)box_h};
-      alignas(64) CUtensorMap tm;
-      const CUresult r = encode(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2,
-                                const_cast<uint8_t*>(reinterpret_cast<const uint8_t*>(map_arena_dev)) + m.data_off, dims,
-                                strides, boxd, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS)
-        return fail(BCG_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult " + std::to_string((int)r));
-      memcpy(out + (int64_t)k * n_widths + j, &tm, sizeof(tm));
-    }
-  }
-  return BCG_OK;
-}
-
 int bcg_init_state(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, void* stream) {
   if (int rc = check_batch(p, b)) return rc;
   if (int rc = check_rows(rows)) return rc;
@@ -2897,17 +2572,19 @@ int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream) {
 static int check_ego(const BcgParams* p, const BcgBatch* b, const uint8_t* ego_image) {
   BCG_REQUIRE(p->ego_w > 0 && p->ego_h > 0 && p->ego_w <= BCG_EGO_MAX && p->ego_h <= BCG_EGO_MAX,
               "egocentric crop must be 1..256 pixels per side");
-  if (ego_image) BCG_REQUIRE(b->ego_work, "BcgBatch.ego_work is needed for the egocentric image");
-  if (ego_image && b->cell_tile_arena) BCG_REQUIRE(p->ego_w <= BCG_EGT_MAX_W, "the cell-tile egocentric kernel handles crops up to 160 pixels wide");
-  if (b->map_tmaps) BCG_REQUIRE(b->tmap_n_widths >= 1 && b->tmap_n_widths <= 4 && b->tmap_box_h > 0, "tensor-map boxes not set");
+  if (ego_image) {
+    BCG_REQUIRE(b->ego_work, "BcgBatch.ego_work is needed for the egocentric image");
+    BCG_REQUIRE(b->cell_tile_arena, "the egocentric image needs the cell-tile planes (BcgBatch.cell_tile_arena)");
+  }
   return BCG_OK;
 }
 
 }  // extern "C"
 
-// capacity handed to the record writers: window buffer of the tile kernel, or shared-memory tile of ego_kernel
-static int ego_capacity(const BcgParams& p, const BcgBatch& b) {
-  return b.cell_tile_arena ? ego_window_capacity(p) : ego_tile_capacity(p, b);
+// window capacity handed to the record writers.  Crops wider than the dense kernel's column table get 0: every record is
+// then in direct mode, and the crop is rendered by the bounds-checked global gather
+static int ego_capacity(const BcgParams& p) {
+  return p.ego_w <= BCG_EGT_MAX_W ? ego_window_capacity(p) : 0;
 }
 
 static int sm_count_of_current_device(int* out) {
@@ -3035,19 +2712,9 @@ static bool ego_dense_kernel_requested() {
 // may be NULL, in ends->final_ego_work)
 static int launch_ego_image(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const EgoHits& hits, const BcgEpisodeEnds* ends,
                             cudaStream_t s) {
-  if (b->cell_tile_arena) {
-    if (b->occ_tile_arena && b->ego_list && !ego_dense_kernel_requested()) return launch_ego_sparse(p, b, ego_image, hits, ends, s);
-    BCG_REQUIRE(!hits.list, "the compact egocentric output (BcgStepOut.ego_hits) comes from the sparse kernel: ego_list is needed");
-    return launch_ego_dense(p, b, ego_image, nullptr, ends, s);
-  }
-  BCG_REQUIRE(!hits.list, "the compact egocentric output (BcgStepOut.ego_hits) needs the cell-tile / occupancy planes");
-  BCG_REQUIRE(!ends, "final crops of episode ends need the cell-tile planes (BcgBatch.cell_tile_arena)");
-  const int cap = ego_tile_capacity(*p, *b);
-  // alignment slack + the per-row spans of the plain-load path, which live behind the tile
-  const int extra = 128 + BCG_EGO_MAX_TILE_ROWS * (int)sizeof(short2);
-  ego_kernel<<<b->n_envs, BCG_EGO_THREADS, cap + extra, s>>>(*p, *b, ego_image, cap);
-  BCG_CHECK_CUDA(cudaGetLastError());
-  return BCG_OK;
+  if (b->occ_tile_arena && b->ego_list && !ego_dense_kernel_requested()) return launch_ego_sparse(p, b, ego_image, hits, ends, s);
+  BCG_REQUIRE(!hits.list, "the compact egocentric output (BcgStepOut.ego_hits) comes from the sparse kernel: ego_list is needed");
+  return launch_ego_dense(p, b, ego_image, nullptr, ends, s);
 }
 
 extern "C" {
@@ -3058,7 +2725,7 @@ int bcg_observe_ego(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, f
   if (int rc = check_ego(p, b, ego_image)) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   ego_prep_kernel<<<blocks_for(b->n_envs, 128), 128, 0, s>>>(*p, *b, ego_image ? 1 : 0, goal_n_state,
-                                                            ego_capacity(*p, *b));
+                                                            ego_capacity(*p));
   BCG_CHECK_CUDA(cudaGetLastError());
   if (ego_image) return launch_ego_image(p, b, ego_image, EgoHits{nullptr, nullptr, 0, false}, nullptr, s);
   return BCG_OK;
@@ -3066,17 +2733,15 @@ int bcg_observe_ego(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, f
 
 }  // extern "C"
 
-static int check_ends(const BcgBatch* b, const BcgStepOut* out, const BcgEpisodeEnds* ends) {
+static int check_ends(const BcgStepOut* out, const BcgEpisodeEnds* ends) {
   if (!ends) return BCG_OK;
   BCG_REQUIRE(ends->capacity >= 1, "BcgEpisodeEnds.capacity must be at least 1");
   BCG_REQUIRE(ends->reason && ends->final_slot && ends->final_obs_vec && ends->final_return && ends->final_length && ends->count,
               "BcgEpisodeEnds: reason, final_slot, final_obs_vec, final_return, final_length and count are needed");
   if (out->goal_n_state) BCG_REQUIRE(ends->final_goal_n_state, "BcgEpisodeEnds.final_goal_n_state is needed with goal_n_state");
-  if (out->ego_image) {
+  if (out->ego_image)
     BCG_REQUIRE(ends->final_ego_work && ends->final_ego_image && ends->final_list,
                 "BcgEpisodeEnds: final_ego_work, final_ego_image and final_list are needed with ego_image");
-    BCG_REQUIRE(b->cell_tile_arena, "final crops of episode ends need the cell-tile planes (BcgBatch.cell_tile_arena)");
-  }
   return BCG_OK;
 }
 
@@ -3087,7 +2752,7 @@ int bcg_step(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, cons
   if (int rc = check_batch(p, b)) return rc;
   if (int rc = check_rows(rows)) return rc;
   BCG_REQUIRE(actions && out, "null actions/out");
-  if (int rc = check_ends(b, out, ends)) return rc;
+  if (int rc = check_ends(out, ends)) return rc;
   const bool ego = out->ego_image || out->goal_n_state;
   if (ego) {
     if (int rc = check_ego(p, b, out->ego_image)) return rc;
@@ -3097,7 +2762,7 @@ int bcg_step(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, cons
   if (events && events[0]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[0], s));
   {
     if (events && events[1]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[1], s));
-    const int cap = ego ? ego_capacity(*p, *b) : 0;
+    const int cap = ego ? ego_capacity(*p) : 0;
     // (event records between the kernels are stream operations of their own: the timed form runs without the overlap)
     const bool pdl = !(events && (events[0] || events[1]));          // an event right before a kernel: no overlap for it
     const bool pdl_reward = !(events && events[2]);

@@ -164,8 +164,7 @@ def _poses_collide(costmaps, poses, env_params):
     from bc_gym_planning_env_b200.vec_env import VecPlanEnv
     # a far-apart dummy path keeps the initial-state kernel happy; only the collision kernel is used
     dummy = [np.array([[0., 0., 0.], [100., 0., 0.]]) for _ in costmaps]
-    checker = VecPlanEnv(costmaps, dummy, attr.evolve(env_params, refine_path=False), noise_parameters=None,
-                         ego_staging='spans')
+    checker = VecPlanEnv(costmaps, dummy, attr.evolve(env_params, refine_path=False), noise_parameters=None)
     return checker.pose_collides(np.asarray(poses, dtype=np.float64)).cpu().numpy()
 
 

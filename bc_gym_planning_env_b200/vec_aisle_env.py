@@ -111,7 +111,6 @@ class _VecSlotEnv(VecPlanEnv):
         self.path_descs = self._to_device(np.frombuffer(bytes(pdescs), dtype=np.uint8).copy())
         self.map_id = torch.arange(n, dtype=torch.int32, device=dev)
         self.path_id = torch.arange(n, dtype=torch.int32, device=dev)
-        self.map_tmaps = None
         self._n_maps = self._n_paths = n
         self._gen_state = torch.zeros((n, 128), dtype=torch.uint8, device=dev)
         self._records = torch.zeros((n, record_bytes), dtype=torch.uint8, device=dev)     # the parameters each world has

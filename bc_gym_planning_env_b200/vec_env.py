@@ -126,17 +126,15 @@ class VecPlanEnv(object):
             on device) instead of sharing pool entries
         :param with_ego: assemble the egocentric observation inside every step
         :param footprint: explicit footprint polygon array(n, 2) in metres (default: the robot's own)
-        :param ego_staging: how the egocentric kernel stages its source window: 'tiles' (default; a derived
-            copy of every costmap in 128-byte cell tiles, only the tiles the rotated window touches are read),
-            'tma' (box loads of the window's bounding box from the uint8 rows) or 'spans' (plain loads)
+        :param ego_staging: how the egocentric kernels stage the source window; 'tiles' is the only value: a derived
+            copy of every costmap in 128-byte cell tiles, of which only the tiles the rotated window touches are read
         :param compact_ego: also keep, per env, the list of non-zero crop pixels (BcgStepOut.ego_hits): what
             `step_host(images='compact')` sends to the host instead of whole crops (needs with_ego and the sparse kernel)
-        :param ego_sparse: with 'tiles' staging, render crops with the sparse scatter kernel (occupancy plane; the dense
+        :param ego_sparse: render crops with the sparse scatter kernel (occupancy plane; the dense
             cell-tile kernel only takes the envs it hands over).  False: the dense kernel renders every env
         :param episode_ends: report every step why envs are done (`terminated`, `truncated`, `episode_reason`) and keep
             the final observation of every episode that ends (`final_observation()`), also when `auto_reset` has already
-            replaced it.  Computed in the step's own kernels (no extra launch); with the egocentric observation it needs
-            ego_staging='tiles'
+            replaced it.  Computed in the step's own kernels (no extra launch)
         :param episode_end_capacity: final crops kept per step (default n_envs, which never overflows; 1 .. n_envs)
         """
         costmaps = list(costmaps)
@@ -162,8 +160,7 @@ class VecPlanEnv(object):
         self._make_batch()
         s = self._stream()
         nat.check(nat.lib().bcg_build_lethal_tiles(C.byref(self._batch), 0, self._batch.n_maps, s))
-        if self.cell_tile_arena is not None:
-            nat.check(nat.lib().bcg_build_cell_tiles(C.byref(self._batch), 0, self._batch.n_maps, s))
+        nat.check(nat.lib().bcg_build_cell_tiles(C.byref(self._batch), 0, self._batch.n_maps, s))
         nat.check(nat.lib().bcg_init_state(C.byref(self._c_params), C.byref(self._batch), self._rows, s))
         self.check_status()
         if self._ego_list is not None:
@@ -183,9 +180,6 @@ class VecPlanEnv(object):
             cap = int(n_envs) if episode_end_capacity is None else int(episode_end_capacity)
             if not 1 <= cap <= int(n_envs):
                 raise ValueError("episode_end_capacity must be in [1, n_envs=%d], got %d" % (int(n_envs), cap))
-            if with_ego and ego_staging != 'tiles':
-                raise ValueError("episode_ends with the egocentric observation needs ego_staging='tiles' (the final crops are "
-                                 "rendered by the cell-tile kernels), got %r" % (ego_staging,))
             self.episode_end_capacity = cap
         elif episode_end_capacity is not None:
             raise ValueError("episode_end_capacity needs episode_ends=True")
@@ -211,8 +205,8 @@ class VecPlanEnv(object):
         self.robot_kind = nat.ROBOT_TRICYCLE if self.dims.drive_type == TRICYCLE else nat.ROBOT_DIFFDRIVE
         self.auto_reset = bool(auto_reset)
         self.with_ego = bool(with_ego)
-        if ego_staging not in ('tiles', 'tma', 'spans'):
-            raise ValueError("ego_staging must be 'tiles', 'tma' or 'spans'")
+        if ego_staging != 'tiles':
+            raise ValueError("ego_staging must be 'tiles' (the TMA and span staging were removed), got %r" % (ego_staging,))
         self.ego_staging = ego_staging
         self._step_index = 0
         self._graph = None
@@ -332,15 +326,8 @@ class VecPlanEnv(object):
             sum_init = np.tile(sum_init, copies)                     # every copy owns its trailers
         self._map_descs_host = descs
         self.map_arena = map_arena
-        # TMA tensor maps for the egocentric kernel's source-window staging: three box-width classes
-        # (dense pitches that keep the rotated shared-memory gather under 2 wavefronts on average) x 8 rows
-        self._tmap_widths, self._tmap_box_h = (144, 176, 208), 8
-        widths = (C.c_int32 * len(self._tmap_widths))(*self._tmap_widths)
-        tm = np.zeros(len(descs) * len(self._tmap_widths) * 128, dtype=np.uint8)
         self.tile_arena = torch.zeros(max(pool_words, 1), dtype=torch.int32, device=self.device)
-        self.cell_tile_arena = None
-        if self.ego_staging == 'tiles':
-            self.cell_tile_arena = torch.empty(max(pool_ctile_bytes, 128), dtype=torch.uint8, device=self.device)
+        self.cell_tile_arena = torch.empty(max(pool_ctile_bytes, 128), dtype=torch.uint8, device=self.device)
         # occupancy plane (cell != 0; same layout as the lethal plane) and its tile summary (one bit per 32 x 16 tile):
         # the sparse egocentric kernel scans them, and the collision check uses the summary to skip empty tiles
         self.occ_tile_arena = torch.zeros(max(pool_words, 1), dtype=torch.int32, device=self.device)
@@ -348,11 +335,6 @@ class VecPlanEnv(object):
             raise ValueError("tile summaries of this batch exceed the 32-bit offsets of BcgMapDesc.sum_off")
         self.occ_sum_arena = self._to_device(sum_init)
         self._cell_index_trailers = True
-        if self.ego_staging == 'tma':
-            nat.check(nat.lib().bcg_encode_map_tensor_maps(descs, len(descs), C.c_void_p(map_arena.data_ptr()), widths,
-                                                           len(self._tmap_widths), self._tmap_box_h,
-                                                           C.c_void_p(tm.ctypes.data)))
-        self.map_tmaps = self._to_device(tm)
         self.map_descs = self._to_device(np.frombuffer(bytes(descs), dtype=np.uint8).copy())
         self.map_id = self._to_device(ids.astype(np.int32))
         self._n_maps = len(descs)
@@ -482,8 +464,7 @@ class VecPlanEnv(object):
         b.lut.bucket_scale = self.lut.bucket_scale
         b.lut.n_bins, b.lut.n_verts, b.lut.max_rows, b.lut.wpr = self.lut.n_bins, self.lut.n_verts, self.lut.max_rows, self.lut.wpr
         b.status, b.stats = self._status.data_ptr(), self._stats.data_ptr()
-        if self.cell_tile_arena is not None:
-            b.cell_tile_arena = self.cell_tile_arena.data_ptr()
+        b.cell_tile_arena = self.cell_tile_arena.data_ptr()
         b.occ_tile_arena = self.occ_tile_arena.data_ptr()
         # BCG_EGO_SUMMARY=0: A/B switch, the sparse kernel then scans every tile of a window (and the collision check
         # loads every tile under the footprint)
@@ -492,13 +473,9 @@ class VecPlanEnv(object):
             if getattr(self, '_cell_index_trailers', False):
                 b.flags |= nat.BATCH_CELL_INDEX
         self._ego_list = None
-        if self.cell_tile_arena is not None and getattr(self, '_ego_sparse', True):
+        if getattr(self, '_ego_sparse', True):
             self._ego_list = torch.zeros(self.n_envs + 4, dtype=torch.int32, device=self.device)
             b.ego_list = self._ego_list.data_ptr()
-        if self.ego_staging == 'tma':
-            b.map_tmaps, b.tmap_n_widths, b.tmap_box_h = self.map_tmaps.data_ptr(), len(self._tmap_widths), self._tmap_box_h
-            for j, w in enumerate(self._tmap_widths):
-                b.tmap_box_w[j] = w
         self._batch = b
         out = nat.BcgStepOut()
         out.reward, out.done, out.hit = self.reward.data_ptr(), self._done_u8.data_ptr(), self._hit_u8.data_ptr()
@@ -508,7 +485,7 @@ class VecPlanEnv(object):
         self._ego_hits = self._ego_hit_count = None
         if getattr(self, '_compact_ego', False):
             if not self.with_ego or self._ego_list is None:
-                raise ValueError("compact_ego needs with_ego=True and the sparse egocentric kernel (ego_staging='tiles', sparse maps)")
+                raise ValueError("compact_ego needs with_ego=True and the sparse egocentric kernel (ego_sparse, sparse maps)")
             self.EGO_HIT_CAP = 1024
             self._ego_hits = torch.zeros((self.n_envs, self.EGO_HIT_CAP), dtype=torch.int32, device=self.device)
             self._ego_hit_count = torch.zeros(self.n_envs, dtype=torch.int32, device=self.device)

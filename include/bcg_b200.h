@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define BCG_ABI_VERSION 12
+#define BCG_ABI_VERSION 13
 
 /* error codes */
 #define BCG_OK 0
@@ -209,16 +209,10 @@ typedef struct BcgBatch {
   const uint32_t* tile_arena;
   const double* path_arena;
   BcgFootprintLut lut;
-  const void* map_tmaps; /* optional: [n_maps][tmap_n_widths] 128-byte TMA tensor maps from
-                            bcg_encode_map_tensor_maps; NULL = the egocentric kernel stages its source
-                            window with plain coalesced loads                                             */
-  int32_t tmap_n_widths;  /* 1..4 box-width classes, ascending                                           */
-  int32_t tmap_box_h;     /* rows per box                                                                */
-  int32_t tmap_box_w[4];  /* box widths (multiples of 16) the tensor maps were encoded with              */
-  const uint8_t* cell_tile_arena; /* optional: cell tiles of every map (bcg_build_cell_tiles); when set the
-                            egocentric kernel stages only the 128-byte tiles its rotated source window
-                            touches (16-byte cp.async pieces, zero fill outside the map) and map_tmaps is
-                            not used                                                                      */
+  const uint8_t* cell_tile_arena; /* cell tiles of every map (bcg_build_cell_tiles); needed for the egocentric image
+                            (and by the world generators): the egocentric kernels stage only the 128-byte tiles
+                            the rotated source window touches (zero fill outside the map); may be NULL when no
+                            egocentric image is ever requested                                                */
   const uint32_t* occ_tile_arena; /* optional: the occupancy plane (1 bit per cell, value != 0), laid out exactly
                             like the lethal tile plane (same tile_off); filled by bcg_build_lethal_tiles.
                             With it, cell_tile_arena and ego_list the egocentric observation takes the sparse
@@ -383,13 +377,6 @@ int bcg_build_lethal_tiles(const BcgBatch* b, int32_t first, int32_t count, void
 /* derive the cell tiles (see BcgMapDesc) of maps [first, first+count) from the uint8 rows (CostMap2D.get_data,
  * costmap_2d.py:91-96: the bytes extract_egocentric_costmap samples, costmap_utils.py:25-75) */
 int bcg_build_cell_tiles(const BcgBatch* b, int32_t first, int32_t count, void* stream);
-/* Host-side: encode n_widths CUtensorMaps (128 B each, cuTensorMapEncodeTiled) per costmap -- uint8
- * [H][pitch] tensor, boxes (box_w[j], box_h), zero fill outside the map (= cv2.warpAffine's
- * borderValue 0, utilities/costmap_utils.py:72) -- into out_host [n_maps][n_widths][128 bytes].  The
- * caller uploads the buffer and points BcgBatch.map_tmaps at it.  Widths must be ascending multiples
- * of 16, and widths and box_h <= 256. */
-int bcg_encode_map_tensor_maps(const BcgMapDesc* maps_host, int32_t n_maps, const void* map_arena_dev,
-                               const int32_t* box_w, int32_t n_widths, int32_t box_h, void* out_host);
 /* make_initial_state (env.py:179-214) + ContinuousRewardProvider.generate_initial_state
  * (reward.py:261-288) for every env: writes init_f/init_i and copies them into state_f/state_i.  With `rows` env e's
  * initial target index uses its own spatial / angular precision (NULL: those of p). */
@@ -404,8 +391,7 @@ int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream);
  * `path_delta`), derive both tile planes, and make the initial state (env.py:179-214, reward.py:261-288).
  * The previous walls of the slot are erased pixel by pixel, so a reset costs O(wall pixels), not O(map).
  * With `rows` the initial states use each env's own goal tolerances (NULL: those of p); rows changed before the call (a
- * new parameter set at a reset) are what the new worlds' initial states see.
- * Not available together with TMA tensor maps (map_tmaps), which cannot be re-encoded on the device. */
+ * new parameter set at a reset) are what the new worlds' initial states see.  Needs BcgBatch.cell_tile_arena. */
 int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
                         const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
                         void* stream);

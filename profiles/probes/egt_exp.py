@@ -1,19 +1,18 @@
 """A/B of the egocentric kernels on the bench workload (run on the GPU box):
     python profiles/probes/egt_exp.py
-sparse = ego_sparse_kernel (default); dense = ego_tiles_kernel for every env (BCG_EGO_KERNEL=dense); tma / spans = the
-first dense kernel with TMA box loads / plain loads of the window's bounding box."""
+sparse = ego_sparse_kernel (default); dense = ego_tiles_kernel for every env (BCG_EGO_KERNEL=dense)."""
 import json
 import os
 import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-for name, staging, kernel in (("sparse", "tiles", None), ("dense", "tiles", "dense"), ("tma", "tma", None), ("spans", "spans", None)):
+for name, kernel in (("sparse", None), ("dense", "dense")):
     env = dict(os.environ)
     if kernel:
         env["BCG_EGO_KERNEL"] = kernel
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "50", "--warmup", "5", "--e2e-steps", "2",
-                          "--cpu-seconds", "0.1", "--gen-envs", "0", "--ego-staging", staging], env=env, capture_output=True, text=True)
+                          "--cpu-seconds", "0.1", "--gen-envs", "0"], env=env, capture_output=True, text=True)
     try:
         d = json.loads(out.stdout.strip().splitlines()[-1])
         ego = [v for k, v in d["kernels_ms"].items() if k.startswith("ego_")][0]

@@ -9,14 +9,14 @@ from tests import common
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("staging,name", [("tiles", "aisle_ego"), ("tma", "aisle_ego"), ("spans", "aisle_ego"),
-                                          ("tiles", "edge_worlds"), ("spans", "edge_worlds"),
-                                          ("tiles", "aisle_goal_reached")])
-def test_ego_observation_matches_reference(staging, name):
-    """All ways of staging the source window (cell tiles via cp.async, TMA box loads, plain span loads) against cv2;
-    `edge_worlds`: crops that lie partly or wholly outside tiny maps (the reference pads with zeros)."""
+@pytest.mark.parametrize("kernel,name", [("tiles", "aisle_ego"), ("dense", "aisle_ego"), ("tiles", "edge_worlds"),
+                                         ("dense", "edge_worlds"), ("tiles", "aisle_goal_reached"), ("dense", "aisle_goal_reached")])
+def test_ego_observation_matches_reference(kernel, name):
+    """Both egocentric kernels against cv2: `tiles` is the default (the sparse scatter kernel, the dense cell-tile kernel
+    for the envs it hands over), `dense` the dense cell-tile kernel for every env (ego_sparse=False); `edge_worlds`: crops
+    that lie partly or wholly outside tiny maps (the reference pads with zeros)."""
     d = common.load(name)
-    env = common.make_vec_env(d, with_ego=True, ego_staging=staging)
+    env = common.make_vec_env(d, with_ego=True, ego_sparse=(kernel == "tiles"))
     actions = torch.from_numpy(d["actions"]).cuda()
     every = int(d["every"])
     k = 0

@@ -381,10 +381,10 @@ def test_validation():
     for cap in (0, 7):
         with pytest.raises(ValueError, match="episode_end_capacity"):
             VecPlanEnv(costmaps, paths, n_envs=6, with_ego=True, episode_ends=True, episode_end_capacity=cap)
-    for staging in ("tma", "spans"):
-        with pytest.raises(ValueError, match="ego_staging"):
-            VecPlanEnv(costmaps, paths, n_envs=6, with_ego=True, episode_ends=True, ego_staging=staging)
-    VecPlanEnv(costmaps, paths, n_envs=6, with_ego=False, episode_ends=True, ego_staging="spans")    # no crops: fine
+    for with_ego in (True, False):                      # 'tiles' is the only staging of the egocentric window
+        for staging in ("tma", "spans"):
+            with pytest.raises(ValueError, match="ego_staging"):
+                VecPlanEnv(costmaps, paths, n_envs=6, with_ego=with_ego, episode_ends=True, ego_staging=staging)
     env = VecPlanEnv(costmaps, paths, n_envs=6)
     with pytest.raises(ValueError, match="episode_ends"):
         env.final_observation()

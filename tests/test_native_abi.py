@@ -24,15 +24,16 @@ def test_library_exports_the_declared_abi():
     for name in declared:
         assert hasattr(lib, name), "libbcg_b200.so does not export %s" % name
     assert sorted(nat.SYMBOLS) == declared, "ctypes binding and header disagree"
-    assert lib.bcg_abi_version() == 12
+    assert lib.bcg_abi_version() == 13
 
 
 def test_one_entry_point_per_operation():
     # bcg_step, bcg_rollout, bcg_init_state and bcg_generate_aisles take NULL rows / ends / events themselves: no
-    # suffixed variant of them is exported, and no stand-alone kinematics step
+    # suffixed variant of them is exported, no stand-alone kinematics step and no tensor-map encoder (the egocentric
+    # kernels stage their windows from the cell tiles only)
     lib = nat.lib()
     for name in ("bcg_init_state_rows", "bcg_generate_aisles_rows", "bcg_step_events", "bcg_step_rows", "bcg_step_ends",
-                 "bcg_rollout_rows", "bcg_rollout_ends", "bcg_kinematic_step"):
+                 "bcg_rollout_rows", "bcg_rollout_ends", "bcg_kinematic_step", "bcg_encode_map_tensor_maps"):
         assert not hasattr(lib, name), "libbcg_b200.so still exports %s" % name
         assert name not in nat.SYMBOLS
 
