@@ -525,14 +525,11 @@ __device__ __forceinline__ bool collide_thread(const BcgFootprintLut& lut, const
     for (int k = 0; k < MAXB; ++k) {
       tm[k] = 0u;
       if (tyb + k <= ty1) {
-        tm[k] = colmask;
-        if (sum) {
-          const uint32_t* srow = sum + (tyb + k) * sw;
-          const int w0 = tx0 >> 5;
-          uint64_t two = __ldg(srow + w0);
-          if ((tx1 >> 5) != w0) two |= (uint64_t)__ldg(srow + w0 + 1) << 32;
-          tm[k] = (uint32_t)(two >> (tx0 & 31)) & colmask;
-        }
+        const uint32_t* srow = sum + (tyb + k) * sw;
+        const int w0 = tx0 >> 5;
+        uint64_t two = __ldg(srow + w0);
+        if ((tx1 >> 5) != w0) two |= (uint64_t)__ldg(srow + w0 + 1) << 32;
+        tm[k] = (uint32_t)(two >> (tx0 & 31)) & colmask;
       }
     }
     // Non-empty tiles of all bands as ONE per-thread list (4 bits per band: a 64-column mask spans <= 3 tiles), so that
@@ -672,14 +669,11 @@ __device__ __forceinline__ bool collide_warp_balanced(const BcgFootprintLut& lut
     for (int k = 0; k < MAXB; ++k) {
       tm[k] = 0u;
       if (ty0 + k <= ty1) {
-        tm[k] = colmask;
-        if (sum) {
-          const uint32_t* srow = sum + (ty0 + k) * sw;
-          const int w0 = tx0 >> 5;
-          uint64_t two = __ldg(srow + w0);
-          if ((tx1 >> 5) != w0) two |= (uint64_t)__ldg(srow + w0 + 1) << 32;
-          tm[k] = (uint32_t)(two >> (tx0 & 31)) & colmask;
-        }
+        const uint32_t* srow = sum + (ty0 + k) * sw;
+        const int w0 = tx0 >> 5;
+        uint64_t two = __ldg(srow + w0);
+        if ((tx1 >> 5) != w0) two |= (uint64_t)__ldg(srow + w0 + 1) << 32;
+        tm[k] = (uint32_t)(two >> (tx0 & 31)) & colmask;
       }
     }
 #pragma unroll

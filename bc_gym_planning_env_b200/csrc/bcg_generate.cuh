@@ -94,8 +94,8 @@ __device__ __forceinline__ AisleGeometry aisle_geometry(const BcgTurnParams& tp,
 struct MapLayout {
   uint8_t* data;       // uint8 rows
   uint32_t* tiles;     // lethal tile plane
-  uint32_t* occ;       // occupancy plane (same layout; may be null)
-  uint32_t* sum;       // tile summary of the occupancy plane: [tiles_y][(tiles_x + 31) / 32] words (may be null)
+  uint32_t* occ;       // occupancy plane (same layout)
+  uint32_t* sum;       // tile summary of the occupancy plane: [tiles_y][(tiles_x + 31) / 32] words
   uint8_t* ctiles;     // cell tiles
   int pitch, rows, tiles_x, ctiles_x;
 };
@@ -130,16 +130,16 @@ __device__ __forceinline__ void draw_wall(const MapLayout& m, int x0, int y0, in
     // Only the pixel with which the line enters a tile touches the summary (x grows along the line, y moves by sy:
     // a tile is entered through its column 0, its row 0 / 15, the map's last row, or at the line's first pixel).
     const bool enters = j == 0 || (x & 31) == 0 || (y & 15) == (sy > 0 ? 0 : 15) || y == m.rows - 1;
-    uint32_t* const sword = (m.sum && enters) ? m.sum + (y >> 4) * ((m.tiles_x + 31) >> 5) + (x >> 10) : nullptr;
+    uint32_t* const sword = m.sum + (y >> 4) * ((m.tiles_x + 31) >> 5) + (x >> 10);
     const uint32_t sbit = 1u << ((x >> 5) & 31);
     if (value == 254) {
       atomicOr(m.tiles + widx, 1u << (x & 31));
-      if (m.occ) atomicOr(m.occ + widx, 1u << (x & 31));
-      if (sword) atomicOr(sword, sbit);                  // result unused: a fire-and-forget reduction
+      atomicOr(m.occ + widx, 1u << (x & 31));
+      if (enters) atomicOr(sword, sbit);                 // result unused: a fire-and-forget reduction
     } else {
       atomicAnd(m.tiles + widx, ~(1u << (x & 31)));
-      if (m.occ) atomicAnd(m.occ + widx, ~(1u << (x & 31)));
-      if (sword) atomicAnd(sword, ~sbit);
+      atomicAnd(m.occ + widx, ~(1u << (x & 31)));
+      if (enters) atomicAnd(sword, ~sbit);
     }
   }
 }

@@ -70,17 +70,9 @@ static int driver_fn(const char* name, F* out) {
 // Programmatic dependent launch: a step kernel launched with the attribute may start while its predecessor in the stream
 // is still draining (launch latency and its own prologue overlap that tail); it calls pdl_wait() before it touches
 // anything the predecessor wrote -- the wait returns when the predecessor grid has completed and its writes are visible.
-// Kernels that call pdl_launch_next() let their successor's CTAs be scheduled once every CTA of theirs has started.
+// No kernel triggers its successor early (griddepcontrol.launch_dependents): successor CTAs waiting in pdl_wait() would
+// hold the slots of the kernel they wait for, so the trigger is left to CTA exit (DESIGN.md section 3).
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_next() {
-#if BCG_PDL_EARLY_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-
-#ifndef BCG_PDL_EARLY_TRIGGER
-#define BCG_PDL_EARLY_TRIGGER 0
-#endif
 
 bool g_pdl_refused = false;       // the driver turned a dependent launch down once: classic launches from then on
 bool pdl_enabled() {
@@ -133,6 +125,8 @@ int check_batch(const BcgParams* p, const BcgBatch* b) {
   BCG_REQUIRE(b->state_f && b->state_i && b->init_f && b->init_i && b->cand && b->cand_i && b->work, "null state pointers");
   BCG_REQUIRE(b->map_id && b->path_id && b->maps && b->paths && b->map_arena && b->tile_arena && b->path_arena,
               "null arena pointers");
+  BCG_REQUIRE(b->occ_tile_arena, "null occupancy plane (BcgBatch.occ_tile_arena)");
+  BCG_REQUIRE(b->occ_sum_arena, "null tile summary (BcgBatch.occ_sum_arena)");
   BCG_REQUIRE(b->lut.edges && b->lut.verts && b->lut.header && b->lut.rows && b->lut.fp_pix && b->lut.bucket_first,
               "null footprint table");
   BCG_REQUIRE(b->lut.n_buckets > 0 && b->lut.bucket_scale > 0, "empty footprint bucket table");
@@ -466,9 +460,6 @@ __device__ __forceinline__ BcgParams with_slot_precision(const BcgParams& p, con
 #define BCG_SR_DONE_BEFORE 8
 #define BCG_SR_GOAL_BEFORE 16
 
-#ifndef BCG_COLLIDE_BALANCED
-#define BCG_COLLIDE_BALANCED 1        // the tiles under a warp's 32 footprints dealt out evenly (collide_warp_balanced)
-#endif
 #ifndef BCG_MOVE_THREADS
 #define BCG_MOVE_THREADS 64
 #endif
@@ -546,7 +537,6 @@ move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, c
             const int action_is_f64, const uint64_t step_index_arg, const BcgStepOut out, const int ego_cap,
             const BcgEnvRows rows, int32_t* const ends_count) {
   pdl_wait();                                            // the previous step's kernels are done with the records and rows
-  pdl_launch_next();
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= b.n_envs) return;
   const BcgParams p = ROWS ? with_env_rows(p_batch, rows, b.n_envs, e) : p_batch;
@@ -615,14 +605,8 @@ move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, c
     fb.nrows = h.z;
     fb.fwidth = h.w;
   }
-#if BCG_COLLIDE_BALANCED
-  const bool hit = collide_warp_balanced(b.lut, b.tile_arena, m.tile_off, b.occ_sum_arena ? b.occ_sum_arena + m.sum_off : nullptr,
-                                         m.tiles_x, m.width, m.height, fb, warp_item_mask(e - (int)(threadIdx.x & 31), b.n_envs),
-                                         threadIdx.x & 31);
-#else
-  const bool hit = collide_thread(b.lut, b.tile_arena + m.tile_off, b.occ_sum_arena ? b.occ_sum_arena + m.sum_off : nullptr,
-                                  m.tiles_x, m.width, m.height, fb);
-#endif
+  const bool hit = collide_warp_balanced(b.lut, b.tile_arena, m.tile_off, b.occ_sum_arena + m.sum_off, m.tiles_x, m.width,
+                                         m.height, fb, warp_item_mask(e - (int)(threadIdx.x & 31), b.n_envs), threadIdx.x & 31);
   if (hit) {  // env.py:458-459 + tricycle_model.py:471-476: pose restored, v = w = 0, wheel / steer command kept
     s[0] = old_pose[0];
     s[1] = old_pose[1];
@@ -747,7 +731,6 @@ template <int G, bool ROWS, bool ENDS>
 __global__ void __launch_bounds__(BCG_REWARD_THREADS, BCG_REWARD_RESIDENT / BCG_REWARD_THREADS)
 reward_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStepOut out, const int ego_cap, const BcgEpisodeEnds ends) {
   pdl_wait();                                            // move_kernel's records
-  pdl_launch_next();
   const int e = (blockIdx.x * blockDim.x + threadIdx.x) / G;
   const unsigned lane = threadIdx.x & 31, gl = lane & (G - 1);
   const bool active = e < b.n_envs;
@@ -969,8 +952,8 @@ __global__ void __launch_bounds__(256) generate_aisles_kernel(const BcgParams p,
   MapLayout m;
   m.data = const_cast<uint8_t*>(b.map_arena) + md->data_off;
   m.tiles = const_cast<uint32_t*>(b.tile_arena) + md->tile_off;
-  m.occ = b.occ_tile_arena ? const_cast<uint32_t*>(b.occ_tile_arena) + md->tile_off : nullptr;
-  m.sum = (b.occ_tile_arena && b.occ_sum_arena) ? const_cast<uint32_t*>(b.occ_sum_arena) + md->sum_off : nullptr;
+  m.occ = const_cast<uint32_t*>(b.occ_tile_arena) + md->tile_off;
+  m.sum = const_cast<uint32_t*>(b.occ_sum_arena) + md->sum_off;
   m.ctiles = const_cast<uint8_t*>(b.cell_tile_arena) + md->cell_tile_off;
   // ---- erase what the slot holds (with the layout it was drawn in) -------------------------------------------
   if (gs->valid) {
@@ -1070,8 +1053,8 @@ __global__ void __launch_bounds__(128) generate_minis_kernel(const BcgParams p, 
   MapLayout m;
   m.data = const_cast<uint8_t*>(b.map_arena) + md->data_off;
   m.tiles = const_cast<uint32_t*>(b.tile_arena) + md->tile_off;
-  m.occ = b.occ_tile_arena ? const_cast<uint32_t*>(b.occ_tile_arena) + md->tile_off : nullptr;
-  m.sum = (b.occ_tile_arena && b.occ_sum_arena) ? const_cast<uint32_t*>(b.occ_sum_arena) + md->sum_off : nullptr;
+  m.occ = const_cast<uint32_t*>(b.occ_tile_arena) + md->tile_off;
+  m.sum = const_cast<uint32_t*>(b.occ_sum_arena) + md->sum_off;
   m.ctiles = const_cast<uint8_t*>(b.cell_tile_arena) + md->cell_tile_off;
   MiniRng rng = {p.seed, p.env_id_base + (uint64_t)e, draw_index, 0u};
   bool accepted = false;
@@ -1228,8 +1211,8 @@ __global__ void __launch_bounds__(256) tiles_kernel(const BcgBatch b, const int 
   const BcgMapDesc m = b.maps[first + blockIdx.y];
   const int words = m.tiles_x * m.tiles_y * 16;
   uint32_t* dst = const_cast<uint32_t*>(b.tile_arena) + m.tile_off;
-  uint32_t* occ = b.occ_tile_arena ? const_cast<uint32_t*>(b.occ_tile_arena) + m.tile_off : nullptr;
-  uint32_t* sum = (occ && b.occ_sum_arena) ? const_cast<uint32_t*>(b.occ_sum_arena) + m.sum_off : nullptr;
+  uint32_t* occ = const_cast<uint32_t*>(b.occ_tile_arena) + m.tile_off;
+  uint32_t* sum = const_cast<uint32_t*>(b.occ_sum_arena) + m.sum_off;
   const uint8_t* src = b.map_arena + m.data_off;
   bool other = false;                      // a cell that is neither free (0) nor lethal (254)
   int occupied = 0;
@@ -1264,8 +1247,8 @@ __global__ void __launch_bounds__(256) tiles_kernel(const BcgBatch b, const int 
       occupied += __popc(obits);
     }
     dst[w] = bits;
-    if (occ) occ[w] = obits;
-    if (sum && obits) {                      // the tile holds a cell (rows race for the same bit: test before the atomic)
+    occ[w] = obits;
+    if (obits) {                             // the tile holds a cell (rows race for the same bit: test before the atomic)
       uint32_t* const sw = sum + ty * ((m.tiles_x + 31) >> 5) + (tx >> 5);
       if ((*(volatile uint32_t*)sw & (1u << (tx & 31))) == 0u) atomicOr(sw, 1u << (tx & 31));
     }
@@ -1283,11 +1266,9 @@ __global__ void __launch_bounds__(256) zero_occupied_kernel(const BcgBatch b, co
   BcgMapDesc* m = const_cast<BcgMapDesc*>(b.maps) + first + k;
   m->occupied = 0;
   m->flags &= ~BCG_MAP_CELL_INDEX;                      // set again by cell_index_kernel once the index matches the plane
-  if (b.occ_tile_arena && b.occ_sum_arena) {            // tiles_kernel only sets summary bits
-    uint32_t* sum = const_cast<uint32_t*>(b.occ_sum_arena) + m->sum_off;
-    const int words = m->tiles_y * ((m->tiles_x + 31) >> 5);
-    for (int i = 0; i < words; ++i) sum[i] = 0u;
-  }
+  uint32_t* sum = const_cast<uint32_t*>(b.occ_sum_arena) + m->sum_off;     // tiles_kernel only sets summary bits
+  const int words = m->tiles_y * ((m->tiles_x + 31) >> 5);
+  for (int i = 0; i < words; ++i) sum[i] = 0u;
 }
 
 // Cell index of one map per CTA (BCG_BATCH_CELL_INDEX trailer, after tiles_kernel): per 32 x 16 tile of the occupancy
@@ -1364,8 +1345,8 @@ __global__ void __launch_bounds__(256) cell_tiles_kernel(const BcgBatch b, const
   }
 }
 
-// pose_collides of the poses whose work records are in b.work; one warp per env.  MODE 0: lethal tile plane,
-// 1: tile plane + in-map pixel count, 2: raw uint8 rows.
+// pose_collides of the poses whose work records are in b.work; one warp per env.  MODE 1: lethal tile plane + in-map
+// pixel count, 2: raw uint8 rows.
 template <int MODE>
 __global__ void __launch_bounds__(256, 6) collision_kernel(const BcgBatch b, uint8_t* __restrict__ flags,
                                                         int32_t* __restrict__ pixels) {
@@ -1376,16 +1357,15 @@ __global__ void __launch_bounds__(256, 6) collision_kernel(const BcgBatch b, uin
   bool hit;
   int cnt = 0;
   if (MODE == 2) hit = collide_u8(b, f, lane);
-  else if (MODE == 1) hit = collide_tiles<true>(b, f, lane, &cnt);
-  else hit = collide_tiles<false>(b, f, lane, nullptr);
+  else hit = collide_tiles<true>(b, f, lane, &cnt);
   if (lane == 0) {
     flags[e] = hit ? 1 : 0;
     if (MODE == 1) pixels[e] = cnt;
   }
 }
 
-// pose_collides of the poses whose work records are in b.work, one THREAD per env (collide_thread): the form the state
-// kernel uses, and the one the collision roofline is measured on.  Per env it reads the 48-byte record, one or two tile
+// pose_collides of the poses whose work records are in b.work, one THREAD per env (collide_warp_balanced): the form the
+// state kernel uses, and the one the collision roofline is measured on.  Per env it reads the 48-byte record, one or two tile
 // summary words per 16-row band and 16-byte quarters of the non-empty tiles under the footprint only.
 __global__ void __launch_bounds__(64) collision_thread_kernel(const BcgBatch b, uint8_t* __restrict__ flags) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1401,13 +1381,8 @@ __global__ void __launch_bounds__(64) collision_thread_kernel(const BcgBatch b, 
   fb.nrows = f.nrows;
   fb.fwidth = f.fwidth;
   fb.bin = f.bin;
-  const uint32_t* sum = b.occ_sum_arena ? b.occ_sum_arena + f.sum_off : nullptr;
-#if BCG_COLLIDE_BALANCED
-  flags[e] = collide_warp_balanced(b.lut, b.tile_arena, f.tile_off, sum, f.tiles_x, f.map_w, f.map_h, fb,
-                                   warp_item_mask(e - (int)(threadIdx.x & 31), b.n_envs), threadIdx.x & 31) ? 1 : 0;
-#else
-  flags[e] = collide_thread(b.lut, b.tile_arena + f.tile_off, sum, f.tiles_x, f.map_w, f.map_h, fb) ? 1 : 0;
-#endif
+  flags[e] = collide_warp_balanced(b.lut, b.tile_arena, f.tile_off, b.occ_sum_arena + f.sum_off, f.tiles_x, f.map_w, f.map_h,
+                                   fb, warp_item_mask(e - (int)(threadIdx.x & 31), b.n_envs), threadIdx.x & 31) ? 1 : 0;
 }
 
 // ---- shared-memory and cp.async primitives ----------------------------------------------------------
@@ -1651,18 +1626,12 @@ __global__ void __launch_bounds__(BCG_EGT_THREADS, BCG_EGT_CTAS) ego_tiles_kerne
 #define BCG_EGS_ZERO_BYTES 2048      // shared page of zeros the bulk stores read
 #endif
 #ifndef BCG_EGS_SUM_ROUNDS
-#define BCG_EGS_SUM_ROUNDS 3         // with the tile summary: rounds of 16 non-empty tiles loaded per pass (2: 0.2454 ms, 3: 0.2457, 4: 0.2488)
-#endif
-#ifndef BCG_EGS_DYNAMIC
-#define BCG_EGS_DYNAMIC 1            // 1: envs beyond a CTA's first four are drawn from a global counter
+#define BCG_EGS_SUM_ROUNDS 3         // rounds of 16 non-empty tiles loaded per pass (2: 0.2454 ms, 3: 0.2457, 4: 0.2488)
 #endif
 #define BCG_EGS_QCAP 64              // ring slots per warp: a push adds <= 32 to <= 31 left over
 #ifndef BCG_EGS_CELL_ROUNDS
 #define BCG_EGS_CELL_ROUNDS 8        // with a cell index: cells loaded per thread before the first is resolved (65 536
                                      // envs: 2: 0.2884 ms per step, 4: 0.2792, 8: 0.2773; profiles/r3b_notes.md)
-#endif
-#ifndef BCG_EGS_SPANS
-#define BCG_EGS_SPANS 1              // clip the listed cells to the tile spans of the rotated crop (0: to its bounding box)
 #endif
 // The fixed-point tables of the crop live in dynamic shared memory, sized by the crop: adxy[ego_w] = (rint(a11 u 2^10),
 // rint(a21 u 2^10)), then bxy[ego_h] = rint((a12 v + b1) 2^10) + 512 - (X0 << 10), same for y (2 KB for a 117 x 133 crop)
@@ -1709,7 +1678,7 @@ __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.a
 // ENDS: items n_envs .. n_envs + min(count[0], capacity) - 1 are the final crops of the step's episode ends
 // (BcgEpisodeEnds): item n_envs + s renders the record final_ego_work[s] into final_ego_image[s], hands slot s over to the
 // dense kernel through final_list, and records no compact hit list
-template <bool SUM, bool HITS, bool ENDS>
+template <bool HITS, bool ENDS>
 __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kernel(const BcgParams p, const BcgBatch b,
                                                                                    uint8_t* __restrict__ image,
                                                                                    uint32_t* __restrict__ hit_list,
@@ -1728,7 +1697,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     alignas(16) EgoSparseTab T;
     alignas(16) uint4 qword[NT / 32][BCG_EGS_QCAP];
     uint32_t qtag[NT / 32][BCG_EGS_QCAP];
-    uint16_t tlist[SUM ? BCG_EGS_MAX_TILES : 2];                // non-empty tiles of the window (every warp writes the same values)
+    uint16_t tlist[BCG_EGS_MAX_TILES];                          // non-empty tiles of the window (every warp writes the same values)
     uint16_t span[2][BCG_EGT_MAX_TILE_ROWS];                    // tile spans of the window rows, double buffered
     int ids[8];                                                 // envs this CTA renders next
   };
@@ -1764,7 +1733,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
       cp_async_16(rec_u32 + slot * BCG_EGO_WORK_BYTES + tid * 16, src + tid * 16, 16u);
     }
   };
-  const bool cix_batch = SUM && (b.flags & BCG_BATCH_CELL_INDEX) != 0;
+  const bool cix_batch = (b.flags & BCG_BATCH_CELL_INDEX) != 0;
   // Tile-summary words of the window of record `q`, lane <-> band of 16 rows (zero where the band or the word lies
   // outside the map, or the env will not take the sparse path).  With a cell index (BCG_BATCH_CELL_INDEX) they are the
   // band's prefix counts at the window's first tile column and one past its last instead: the band's cells are
@@ -1794,24 +1763,21 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
   for (int i = tid * 16; i < BCG_EGS_ZERO_BYTES; i += NT * 16) *reinterpret_cast<uint4*>(zero_s + i) = make_uint4(0u, 0u, 0u, 0u);
   if (tid < 2) T.count[tid] = T.hits[tid] = 0;
   pdl_wait();                                 // the records (and, on a reset, the state) are reward_kernel's
-  pdl_launch_next();
   if (ENDS) n_items = n + min(ends.count[0], ends.capacity);
 #pragma unroll
   for (int k = 0; k < RD; ++k) fetch_record(e0 + k * G, k);
   cp_async_commit();
-#if BCG_EGS_DYNAMIC
   // Which envs a CTA renders: its first RD + 1 are blockIdx.x + k G; the later ones come from a global counter
   // (ego_list[n + 1], zeroed with the hand-over count), drawn RD + 1 iterations ahead so that the record can be
   // prefetched -- CTAs whose windows are light take more envs, and the 24-or-25 envs per CTA quantisation goes away.
   if (tid <= RD) ids_s[tid] = e0 + tid * G;
-#endif
   fence_async_smem();                         // the zeros are visible to the bulk-copy engine
   cp_async_wait_all();
   __syncthreads();
 
   // tile spans of the window rows (ego_band_span), lane <-> tile row, computed by the last warp one env ahead of their use
   auto make_spans = [&](int slot, int buf) {
-    if (!BCG_EGS_SPANS || warp != NT / 32 - 1) return;
+    if (warp != NT / 32 - 1) return;
     const EgoTileWork* q = reinterpret_cast<const EgoTileWork*>(rec_s + slot * BCG_EGO_WORK_BYTES);
     if (q->mode != BCG_EGO_MODE_TILES || (q->dense_map & 1)) return;
     for (int t = lane; t < q->nty; t += 32)
@@ -1820,8 +1786,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
   make_spans(0, 0);
   __syncthreads();
   uint32_t pf_lo = 0u, pf_hi = 0u;              // summary words of the env about to be rendered
-  if (SUM) summary_words(reinterpret_cast<const EgoTileWork*>(rec_s), pf_lo, pf_hi, true);
-#if BCG_EGS_DYNAMIC
+  summary_words(reinterpret_cast<const EgoTileWork*>(rec_s), pf_lo, pf_hi, true);
   for (int it = 0;; ++it) {
     const int e = ids_s[it & 7];
     if (e >= n_items) break;
@@ -1831,17 +1796,9 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     fetch_record(ids_s[(it + RD) & 7], (it + RD) & (BCG_EGS_REC_SLOTS - 1));
     cp_async_commit();
     const int e_next = ids_s[(it + 1) & 7];
-#else
-  int e = e0;
-  for (int it = 0; e < n_items; e += G, ++it) {
-    const int slot = it & (BCG_EGS_REC_SLOTS - 1), par = it & 1;
-    fetch_record(e + RD * G, (it + RD) & (BCG_EGS_REC_SLOTS - 1));
-    cp_async_commit();
-    const int e_next = e + G;
-#endif
     // record it + 1 has landed (only the newest fetch may still be in flight): start its summary loads now
     const uint32_t cur_lo = pf_lo, cur_hi = pf_hi;
-    if (SUM && e_next < n_items)
+    if (e_next < n_items)
       summary_words(reinterpret_cast<const EgoTileWork*>(rec_s + ((it + 1) & (BCG_EGS_REC_SLOTS - 1)) * BCG_EGO_WORK_BYTES), pf_lo, pf_hi, true);
     if (e_next < n_items) make_spans((it + 1) & (BCG_EGS_REC_SLOTS - 1), (it + 1) & 1);
     const EgoTileWork* r = reinterpret_cast<const EgoTileWork*>(rec_s + slot * BCG_EGO_WORK_BYTES);
@@ -1854,7 +1811,8 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     // maps with more than one cell in 20 occupied (filled regions, inflation gradients) overflow the cell list in
     // almost every window: they go straight to the dense kernel instead of paying for a scan that is thrown away
     const bool dense_map = (r->dense_map & 1) != 0;     // decided by the record writer, which holds the map descriptor
-    const bool try_sparse = mode == BCG_EGO_MODE_TILES && ntile <= BCG_EGS_MAX_TILES && !dense_map && (!SUM || (nby <= 32 && nwx <= 32));
+    // (<= 32 bands and <= 32 word columns: a band's summary bits are one lane's, a band's tile mask one word)
+    const bool try_sparse = mode == BCG_EGO_MODE_TILES && ntile <= BCG_EGS_MAX_TILES && !dense_map && (nby <= 32 && nwx <= 32);
     // With a cell index (BCG_BATCH_CELL_INDEX, map bit in the record) band b's cells are cells[lo_b .. hi_b) (the words
     // `summary_words` loaded, lane <-> band).  An inclusive warp scan of the band counts numbers the window's cells
     // 0 .. total - 1, and cell j of band b is cells[j + lo_b - start_b]: the scatter reads them straight from there.
@@ -1862,7 +1820,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     // any other.  A window with more than BCG_EGS_LIST cells in its bands (whose cells inside the crop's tile spans may
     // or may not overflow the list) is listed from the occupancy plane instead, so that the overflow rule -- and with it
     // which envs report a compact hit list -- stays exactly that of the listing.
-    const bool has_index = SUM && cix_batch && try_sparse && (r->dense_map & 4);
+    const bool has_index = cix_batch && try_sparse && (r->dense_map & 4);
     int bincl = 0, boff = 0, total = 0;
     const uint32_t* cells = nullptr;
     if (has_index) {
@@ -1886,11 +1844,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
         const int body = (npx - head) & ~15, tail = npx - head - body;
         // one bulk store of the zero page per lane of warp 0 (a loop in one thread was 16 instructions per store; a
         // bulk group belongs to the thread that committed it, so the same lanes wait for theirs below)
-#ifdef BCG_EGS_EXP_NO_ZERO                  // experiment: no bulk zero stores
-        if (warp == 0 && ego_w < 0) {
-#else
         if (warp == 0) {
-#endif
           for (int o = lane * BCG_EGS_ZERO_BYTES; o < body; o += 32 * BCG_EGS_ZERO_BYTES) {
             if (e >= evict_from) bulk_store_evict_first(dst + head + o, zero_u32, (uint32_t)min(body - o, BCG_EGS_ZERO_BYTES));
             else bulk_store(dst + head + o, zero_u32, (uint32_t)min(body - o, BCG_EGS_ZERO_BYTES));
@@ -1927,7 +1881,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
       // Walls are thin: only a few of a warp's 32 pieces hold a cell, so expanding them where they were loaded would
       // keep most lanes idle.  Each warp queues its non-empty pieces (16 bytes + band / column / row-group tag) in a
       // shared ring and expands them 32 at a time, one piece per lane. ------------------------------------------------
-      const int tiles_x = (int)(r->tiles_xy & 0xffffu), tiles_y = (int)(r->tiles_xy >> 16);
+      const int tiles_x = (int)(r->tiles_xy & 0xffffu);
       const uint4* occ = reinterpret_cast<const uint4*>(b.occ_tile_arena + ((int64_t)r->tile_off16 << 4));
       const int g = lane & 3;                                                     // rows 4 g .. 4 g + 3 of the tile
       constexpr int TPR = NT / 4;                                                // tiles per round
@@ -1947,11 +1901,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
         uint32_t bits[4] = {wd.x, wd.y, wd.z, wd.w};
         uint32_t keep = 0u;
         if (yr0 >= 0 && yr0 < 8 * nty) {                                          // clip to the tile span of these rows
-#if BCG_EGS_SPANS
           const uint32_t sp = lds_u16(span_u32 + 2 * (yr0 >> 3));
-#else
-          const uint32_t sp = (uint32_t)(ntx - 1) << 8;                          // experiment: the window's bounding box only
-#endif
           const int lo = max(X0 + 16 * (int)(sp & 0xff) - (tx << 5), 0);
           const int hi = min(X0 + 16 * (int)(sp >> 8) + 15 - (tx << 5), 31);
           if (lo <= hi) keep = (0xffffffffu >> (31 - hi)) & (0xffffffffu << lo);
@@ -2000,7 +1950,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
       };
       if (cix) {
         // cell index: nothing to list, the scatter below reads the window's cells from the index
-      } else if constexpr (SUM) {
+      } else {
         uint32_t slo = cur_lo, shi = cur_hi;
         if (has_index) summary_words(r, slo, shi, false);                       // the prefetched words were prefix counts
         // (a) which tiles of the window hold a cell at all: lane <-> band of 16 rows, one or two words of the map's tile
@@ -2045,23 +1995,6 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
 #pragma unroll
           for (int rd = 0; rd < RS; ++rd) push(word[rd], tag[rd]);
         }
-      } else {
-        const uint32_t inv = (65536u + (uint32_t)nwx - 1u) / (uint32_t)nwx;       // t / nwx == (t * inv) >> 16 for t < 4096
-        constexpr int RMAX = (BCG_EGS_MAX_TILES + TPR - 1) / TPR;
-        uint4 word[RMAX];
-        uint32_t tag[RMAX];
-#pragma unroll
-        for (int rd = 0; rd < RMAX; ++rd) {
-          const int t = (tid >> 2) + rd * TPR;
-          const int band = (int)(((uint32_t)t * inv) >> 16), jw = t - band * nwx;
-          const int ty = by0 + band, tx = wx0 + jw;
-          word[rd] = make_uint4(0u, 0u, 0u, 0u);
-          tag[rd] = (uint32_t)((band << 8) | (jw << 2) | g);
-          if (t < ntile && (unsigned)ty < (unsigned)tiles_y && (unsigned)tx < (unsigned)tiles_x)
-            word[rd] = __ldg(occ + (((ty * tiles_x + tx) << 2) + g));
-        }
-#pragma unroll
-        for (int rd = 0; rd < RMAX; ++rd) push(word[rd], tag[rd]);
       }
       if (qtail != qhead) {
         __syncwarp();
@@ -2113,16 +2046,10 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
         const bool h11 = (ax1 + b1.x) < 1024u && (ay1 + b1.y) < 1024u;
         const int o00 = fv * ego_w + fu;                                      // may lie outside the crop; only hits are stored
         uint8_t* const p0 = dst + o00, * const p1 = p0 + ego_w;
-#ifdef BCG_EGS_EXP_NO_HITS                  // experiment: everything but the hit stores (the compiler cannot drop the tests)
-        if (ego_w < 0) {
-#endif
         if (h00) p0[0] = (uint8_t)val;
         if (h10) p0[1] = (uint8_t)val;
         if (h01) p1[0] = (uint8_t)val;
         if (h11) p1[1] = (uint8_t)val;
-#ifdef BCG_EGS_EXP_NO_HITS
-        }
-#endif
         if (HITS && !final_crop) {
           // compact observation (BcgStepOut.ego_hits): pixel offset | value << 16 of every non-zero crop pixel.  A crop
           // pixel samples exactly one cell and the four candidates of a cell are distinct pixels: no duplicates.
@@ -2207,9 +2134,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
       if (sparse && tid == 0 && !final_crop) hit_count[e] = (int32_t)T.hits[par];      // > hit_cap: the list overflowed, read the image
       if (tid == 0) T.hits[par ^ 1] = 0;
     }
-#if BCG_EGS_DYNAMIC
     if (tid == 0) ids_s[(it + RD + 1) & 7] = drawn;
-#endif
     __syncthreads();                            // list, tables and record `it` are free
   }
 }
@@ -2419,6 +2344,8 @@ int bcg_state_layout(const BcgParams* p, BcgStateLayout* out) {
 
 int bcg_build_lethal_tiles(const BcgBatch* b, int32_t first, int32_t count, void* stream) {
   BCG_REQUIRE(b && b->maps && b->map_arena && b->tile_arena, "null map arena");
+  BCG_REQUIRE(b->occ_tile_arena, "null occupancy plane (BcgBatch.occ_tile_arena)");
+  BCG_REQUIRE(b->occ_sum_arena, "null tile summary (BcgBatch.occ_sum_arena)");
   BCG_REQUIRE(first >= 0 && count >= 0 && first + count <= b->n_maps, "map range out of bounds");
   cudaStream_t s = (cudaStream_t)stream;
   if (count > 0) zero_occupied_kernel<<<blocks_for(count, 256), 256, 0, s>>>(*b, first, count);
@@ -2427,7 +2354,7 @@ int bcg_build_lethal_tiles(const BcgBatch* b, int32_t first, int32_t count, void
     tiles_kernel<<<dim3(8, chunk), 256, 0, s>>>(*b, first + done);
     BCG_CHECK_CUDA(cudaGetLastError());
   }
-  if ((b->flags & BCG_BATCH_CELL_INDEX) && b->occ_tile_arena && b->occ_sum_arena && count > 0) {
+  if ((b->flags & BCG_BATCH_CELL_INDEX) && count > 0) {
     cell_index_kernel<<<count, BCG_CIX_THREADS, 0, s>>>(*b, first);
     BCG_CHECK_CUDA(cudaGetLastError());
   }
@@ -2656,25 +2583,22 @@ static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego
   // (the hand-over count and the env counter in ego_list[n_envs ..] were zeroed by the state / prep kernel)
   // persistent CTAs, as many per SM as fit with this crop's tables (18 for the 117 x 133 crop)
   const int tab_bytes = (p->ego_w + p->ego_h + 4) * (int)sizeof(int2);     // + a sentinel before and after each table
-  const bool sum = b->occ_sum_arena != nullptr;
-  using SparseKernel = decltype(&ego_sparse_kernel<false, false, false>);
-  static const SparseKernel kernels[2][2][2] = {      // [SUM][HITS][ENDS]
-      {{ego_sparse_kernel<false, false, false>, ego_sparse_kernel<false, false, true>},
-       {ego_sparse_kernel<false, true, false>, ego_sparse_kernel<false, true, true>}},
-      {{ego_sparse_kernel<true, false, false>, ego_sparse_kernel<true, false, true>},
-       {ego_sparse_kernel<true, true, false>, ego_sparse_kernel<true, true, true>}}};
-  static int per_sm_cache[2][64] = {{0}}, tab_cache[2][64] = {{0}};
+  using SparseKernel = decltype(&ego_sparse_kernel<false, false>);
+  static const SparseKernel kernels[2][2] = {         // [HITS][ENDS]
+      {ego_sparse_kernel<false, false>, ego_sparse_kernel<false, true>},
+      {ego_sparse_kernel<true, false>, ego_sparse_kernel<true, true>}};
+  static int per_sm_cache[64] = {0}, tab_cache[64] = {0};
   int dev = 0;
   BCG_CHECK_CUDA(cudaGetDevice(&dev));
   int per_sm = 0;
-  if (dev >= 0 && dev < 64 && per_sm_cache[sum][dev] > 0 && tab_cache[sum][dev] == tab_bytes) {
-    per_sm = per_sm_cache[sum][dev];
+  if (dev >= 0 && dev < 64 && per_sm_cache[dev] > 0 && tab_cache[dev] == tab_bytes) {
+    per_sm = per_sm_cache[dev];
   } else {
-    BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernels[sum][0][0], BCG_EGS_THREADS, tab_bytes));
+    BCG_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernels[0][0], BCG_EGS_THREADS, tab_bytes));
     BCG_REQUIRE(per_sm > 0, "the sparse egocentric kernel does not fit an SM with this crop size");
     if (dev >= 0 && dev < 64) {
-      per_sm_cache[sum][dev] = per_sm;
-      tab_cache[sum][dev] = tab_bytes;
+      per_sm_cache[dev] = per_sm;
+      tab_cache[dev] = tab_bytes;
     }
   }
   const int grid = b->n_envs < per_sm * sms ? b->n_envs : per_sm * sms;
@@ -2692,7 +2616,7 @@ static int launch_ego_sparse(const BcgParams* p, const BcgBatch* b, uint8_t* ego
   const bool with_hits = hits.list != nullptr;
   // (the final crops of episode ends, when asked for, are the items behind the envs)
   const BcgEpisodeEnds en = ends ? *ends : BcgEpisodeEnds{};
-  BCG_CHECK_CUDA(launch_step_kernel(kernels[sum][with_hits][ends != nullptr], grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b,
+  BCG_CHECK_CUDA(launch_step_kernel(kernels[with_hits][ends != nullptr], grid, BCG_EGS_THREADS, tab_bytes, s, hits.pdl, *p, *b,
                                     ego_image, hits.list, with_hits ? hits.count : nullptr, with_hits ? hits.cap : 0, evict, en));
   BCG_CHECK_CUDA(cudaGetLastError());
   if (b->flags & BCG_BATCH_SPARSE_EGO_ONLY) return BCG_OK;     // the sparse kernel rendered every env itself
@@ -2712,7 +2636,7 @@ static bool ego_dense_kernel_requested() {
 // may be NULL, in ends->final_ego_work)
 static int launch_ego_image(const BcgParams* p, const BcgBatch* b, uint8_t* ego_image, const EgoHits& hits, const BcgEpisodeEnds* ends,
                             cudaStream_t s) {
-  if (b->occ_tile_arena && b->ego_list && !ego_dense_kernel_requested()) return launch_ego_sparse(p, b, ego_image, hits, ends, s);
+  if (b->ego_list && !ego_dense_kernel_requested()) return launch_ego_sparse(p, b, ego_image, hits, ends, s);
   BCG_REQUIRE(!hits.list, "the compact egocentric output (BcgStepOut.ego_hits) comes from the sparse kernel: ego_list is needed");
   return launch_ego_dense(p, b, ego_image, nullptr, ends, s);
 }

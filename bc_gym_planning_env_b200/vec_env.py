@@ -465,13 +465,9 @@ class VecPlanEnv(object):
         b.lut.n_bins, b.lut.n_verts, b.lut.max_rows, b.lut.wpr = self.lut.n_bins, self.lut.n_verts, self.lut.max_rows, self.lut.wpr
         b.status, b.stats = self._status.data_ptr(), self._stats.data_ptr()
         b.cell_tile_arena = self.cell_tile_arena.data_ptr()
-        b.occ_tile_arena = self.occ_tile_arena.data_ptr()
-        # BCG_EGO_SUMMARY=0: A/B switch, the sparse kernel then scans every tile of a window (and the collision check
-        # loads every tile under the footprint)
-        if os.environ.get("BCG_EGO_SUMMARY", "1") != "0":
-            b.occ_sum_arena = self.occ_sum_arena.data_ptr()
-            if getattr(self, '_cell_index_trailers', False):
-                b.flags |= nat.BATCH_CELL_INDEX
+        b.occ_tile_arena, b.occ_sum_arena = self.occ_tile_arena.data_ptr(), self.occ_sum_arena.data_ptr()
+        if getattr(self, '_cell_index_trailers', False):
+            b.flags |= nat.BATCH_CELL_INDEX
         self._ego_list = None
         if getattr(self, '_ego_sparse', True):
             self._ego_list = torch.zeros(self.n_envs + 4, dtype=torch.int32, device=self.device)

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define BCG_ABI_VERSION 13
+#define BCG_ABI_VERSION 14
 
 /* error codes */
 #define BCG_OK 0
@@ -213,17 +213,19 @@ typedef struct BcgBatch {
                             (and by the world generators): the egocentric kernels stage only the 128-byte tiles
                             the rotated source window touches (zero fill outside the map); may be NULL when no
                             egocentric image is ever requested                                                */
-  const uint32_t* occ_tile_arena; /* optional: the occupancy plane (1 bit per cell, value != 0), laid out exactly
-                            like the lethal tile plane (same tile_off); filled by bcg_build_lethal_tiles.
-                            With it, cell_tile_arena and ego_list the egocentric observation takes the sparse
-                            path: zero the crop, then scatter only the occupied source cells of its window   */
+  const uint32_t* occ_tile_arena; /* required: the occupancy plane (1 bit per cell, value != 0), laid out exactly
+                            like the lethal tile plane (same tile_off); filled by bcg_build_lethal_tiles and kept
+                            by the generators.  With cell_tile_arena and ego_list the egocentric observation takes
+                            the sparse path: zero the crop, then scatter only the occupied source cells of its
+                            window                                                                          */
   int32_t* ego_list;      /* optional scratch [n_envs + 4]: envs whose window holds too many occupied cells
                             for the sparse path, handed to the dense cell-tile kernel (count at [n_envs]; [n_envs + 1] is
                             the sparse kernel's env counter)                                                 */
-  const uint32_t* occ_sum_arena; /* optional: one bit per tile of the occupancy plane (BcgMapDesc.sum_off), filled by
+  const uint32_t* occ_sum_arena; /* required: one bit per tile of the occupancy plane (BcgMapDesc.sum_off), filled by
                             bcg_build_lethal_tiles and kept by the generators; must start out zero (but for the capacity
-                            words of BCG_BATCH_CELL_INDEX trailers).  With it the sparse egocentric kernel loads only
-                            the non-empty tiles of a window, or with a cell index only the window's cells              */
+                            words of BCG_BATCH_CELL_INDEX trailers).  The collision check loads only the non-empty tiles
+                            under a footprint, and the sparse egocentric kernel only those of a window, or with a cell
+                            index only the window's cells                                                           */
   uint32_t* status; /* [BCG_STATUS_WORDS] */
   double* stats;    /* [BCG_STATS_WORDS]  */
   uint64_t* step_counter; /* optional device [2], zero at start: when set, bcg_step ignores its step_index argument,
@@ -372,7 +374,8 @@ int bcg_device_count(void);
 int bcg_state_layout(const BcgParams* p, BcgStateLayout* out);
 
 /* -- setup (at reset time, not per step) ------------------------------------------------------------ */
-/* derive the lethal bit-plane (cell == 254, costmap_2d.py:21) of maps [first, first+count) */
+/* derive the lethal bit-plane (cell == 254, costmap_2d.py:21), the occupancy plane and its tile summary (both required:
+ * BcgBatch.occ_tile_arena, occ_sum_arena) of maps [first, first+count) */
 int bcg_build_lethal_tiles(const BcgBatch* b, int32_t first, int32_t count, void* stream);
 /* derive the cell tiles (see BcgMapDesc) of maps [first, first+count) from the uint8 rows (CostMap2D.get_data,
  * costmap_2d.py:91-96: the bytes extract_egocentric_costmap samples, costmap_utils.py:25-75) */

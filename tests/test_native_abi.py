@@ -9,6 +9,7 @@ import pytest
 from bc_gym_planning_env_b200 import _native as nat
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+BCG_ERR_INVALID = -1                                   # include/bcg_b200.h
 
 
 def _declared_symbols():
@@ -17,14 +18,14 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(bcg_[a-z0-9_]+)\s*\(", text)))
 
 
-def test_library_exports_the_declared_abi():
+def test_library_exports_the_declared_abi_version_14():
     lib = nat.lib()
     declared = _declared_symbols()
     assert len(declared) >= 18
     for name in declared:
         assert hasattr(lib, name), "libbcg_b200.so does not export %s" % name
     assert sorted(nat.SYMBOLS) == declared, "ctypes binding and header disagree"
-    assert lib.bcg_abi_version() == 13
+    assert lib.bcg_abi_version() == 14
 
 
 def test_one_entry_point_per_operation():
@@ -63,6 +64,38 @@ def test_bad_arguments_return_error_codes():
     p, b = nat.BcgParams(), nat.BcgBatch()
     assert lib.bcg_step(C.byref(p), C.byref(b), None, None, 0, 0, None, None, None, None) < 0
     assert "n_envs" in nat.last_error()
+
+
+def _batch_with_dummy_pointers():
+    # every field check_batch requires, as non-null pointers that no kernel ever reads (the calls below launch nothing)
+    p, b = nat.BcgParams(), nat.BcgBatch()
+    L = nat.state_layout(p)
+    b.n_envs, b.n_frows, b.n_irows = 1, L.n_frows, L.n_irows
+    dummy = 0x1000
+    for name in ("state_f", "state_i", "init_f", "init_i", "cand", "cand_i", "work", "map_id", "path_id", "maps", "paths",
+                 "map_arena", "tile_arena", "path_arena", "occ_tile_arena", "occ_sum_arena", "status", "stats"):
+        setattr(b, name, dummy)
+    for name in ("edges", "verts", "header", "rows", "fp_pix", "bucket_first"):
+        setattr(b.lut, name, dummy)
+    b.lut.n_buckets, b.lut.bucket_scale, b.lut.n_verts = 1, 1.0, 4
+    b.lut.n_bins, b.lut.wpr, b.lut.max_rows = 1, 1, 1
+    return p, b
+
+
+@pytest.mark.parametrize("field", ["occ_tile_arena", "occ_sum_arena"])
+def test_batch_without_occupancy_plane_or_summary_is_refused(field):
+    # the collision check, the egocentric kernels and the world generators read the occupancy plane and its tile
+    # summary unconditionally: a batch without either is refused before anything is launched
+    lib = nat.lib()
+    p, b = _batch_with_dummy_pointers()
+    plan = C.c_void_p(0x1000)
+    assert lib.bcg_rollout(C.byref(p), C.byref(b), None, plan, 0, 0, None, None, None) == 0
+    assert lib.bcg_build_lethal_tiles(C.byref(b), 0, 0, None) == 0
+    setattr(b, field, None)
+    assert lib.bcg_rollout(C.byref(p), C.byref(b), None, plan, 0, 0, None, None, None) == BCG_ERR_INVALID
+    assert field in nat.last_error()
+    assert lib.bcg_build_lethal_tiles(C.byref(b), 0, 0, None) == BCG_ERR_INVALID
+    assert field in nat.last_error()
 
 
 def test_no_cpu_fallback_without_a_device():
