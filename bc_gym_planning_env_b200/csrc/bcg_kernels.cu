@@ -204,6 +204,14 @@ __device__ __forceinline__ EgoAffine ego_affine(const BcgParams& p, const BcgMap
   return a;
 }
 
+// The path point goal_n_state points at.  envs/egocentric.py:141-160 takes the first point of Observation.path: path[target:]
+// with the continuous reward, so the next way point; path[:target + 1] with pure pursuit (reward.py:120-124), so the first
+// point of the path.  The colored variant (synth_turn_env.py:412-418) points at the last path point.
+__device__ __forceinline__ int goal_point_index(const BcgParams& p, int n, int target) {
+  if (p.ego_variant == 1) return n - 1;
+  return p.reward_kind == BCG_REWARD_PURE_PURSUIT ? 0 : target;
+}
+
 // goal_n_state (envs/egocentric.py:141-160) by one thread
 // `target` and `drobot` (the delayed robot state x, y, th, v, w, steer, wheel) are those of the state being observed
 __device__ __forceinline__ void write_goal_n_state(const BcgParams& p, const BcgBatch& b, int e, const BcgPathDesc& pd,
@@ -217,7 +225,7 @@ __device__ __forceinline__ void write_goal_n_state(const BcgParams& p, const Bcg
   }
   // from_global_to_egocentric (coordinate_transformations.py:341-362 -> :57-84 -> :310-328)
   const double* P = b.path_arena + pd.off;
-  const int gi = p.ego_variant == 1 ? pd.n - 1 : target;      // last path point vs next way point
+  const int gi = goal_point_index(p, pd.n, target);
   const double gx = P[gi], gy = P[pd.pitch + gi], gt = P[2 * pd.pitch + gi];
   double sn, cs;
   sincos(pth, &sn, &cs);
@@ -499,7 +507,7 @@ __device__ __forceinline__ void write_goal_from_transform(const BcgParams& p, co
     for (int k = 0; k < 9; ++k) g[k] = 0.f;
     return;
   }
-  const int gi = p.ego_variant == 1 ? n - 1 : target;      // last path point vs next way point
+  const int gi = goal_point_index(p, n, target);
   const double gx = P[gi], gy = P[pitch + gi], gt = P[2 * pitch + gi];
   const double ex = ct * gx - st * gy + tx;
   const double ey = st * gx + ct * gy + ty;

@@ -200,14 +200,20 @@ def test_live_reference_beside_the_cuda_batch():
 
 
 def test_move_kernel_register_tiers_give_the_same_bits():
-    """move_kernel is built three times (230 / 168 / 128 registers) and the launch picks one by batch size.  The same
-    envs stepped as the head of a 4 096-, a 30 000- and a 60 000-env batch (one tier each on a 148-SM B200) agree bit
-    for bit: state, rewards, done flags, compact observation, with noise, delays and auto-reset on."""
+    """move_kernel is built three times (230 / 168 / 128 registers) and bcg_step picks one by its block count (64 threads
+    per block) on S SMs: tier 0 up to 4 S blocks, tier 1 up to 6 S, tier 2 above.  The same envs stepped as the head of
+    a 4 096-env batch (tier 0), of a 320 S + 13 one (the middle of tier 1: 47 373 envs on a 148-SM B200) and of a
+    448 S + 29 one (tier 2: 66 333) agree bit for bit: state, rewards, done flags, compact observation, egocentric crops
+    and goal vectors, with noise, delays and auto-reset on."""
+    from tests.test_gpu_step_matrix import move_tier
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
     params = EnvParams(control_delay=2, pose_delay=1, state_delay=1)
     costmaps, paths = random_aisle_pool(16, 31, params)
     head = 4096
-    envs = [VecPlanEnv(costmaps, paths, params, n_envs=n, seed=9, auto_reset=True, with_ego=False, noise_parameters=DEFAULT_NOISE)
-            for n in (head, 30000, 60000)]
+    sizes = (head, 320 * sms + 13, 448 * sms + 29)
+    assert [move_tier(n, sms) for n in sizes] == [0, 1, 2], (sms, sizes)
+    envs = [VecPlanEnv(costmaps, paths, params, n_envs=n, seed=9, auto_reset=True, with_ego=True, noise_parameters=DEFAULT_NOISE)
+            for n in sizes]
     acts = _actions(envs[0], 120, 11)
     for t, act in enumerate(acts):
         for env in envs:
@@ -219,6 +225,8 @@ def test_move_kernel_register_tiers_give_the_same_bits():
                 assert torch.equal(ref.state_f, env.state_f[:, :head]) and torch.equal(ref.state_i, env.state_i[:, :head]), (t, env.n_envs)
                 assert torch.equal(ref.reward, env.reward[:head]) and torch.equal(ref.done, env.done[:head]), (t, env.n_envs)
                 assert torch.equal(ref.obs_vec, env.obs_vec[:head]), (t, env.n_envs)
+                assert torch.equal(ref.ego_image, env.ego_image[:head]), (t, env.n_envs)
+                assert torch.equal(ref.goal_n_state, env.goal_n_state[:head]), (t, env.n_envs)
     assert float(envs[0].episode_stats()[0]) > 0
     for env in envs:
         env.check_status()
