@@ -66,6 +66,7 @@ class BcgBatch(C.Structure):
         ("lut", BcgFootprintLut),
         ("cell_tile_arena", C.c_void_p), ("occ_tile_arena", C.c_void_p), ("ego_list", C.c_void_p),
         ("occ_sum_arena", C.c_void_p), ("status", C.c_void_p), ("stats", C.c_void_p), ("step_counter", C.c_void_p),
+        ("world_gen", C.c_void_p),
     ]
 
 
@@ -94,6 +95,13 @@ class BcgMiniGenParams(C.Structure):
 class BcgMiniParams(C.Structure):
     _fields_ = [("h", C.c_double), ("w", C.c_double), ("start", C.c_double * 3), ("end", C.c_double * 3),
                 ("a", C.c_double * 2), ("o", C.c_double * 2), ("b", C.c_double * 2)]
+
+
+class BcgWorldGen(C.Structure):
+    _fields_ = [
+        ("kind", C.c_int32), ("reserved", C.c_int32), ("slots", BcgAisleSlots), ("mini", BcgMiniGenParams),
+        ("path_delta", C.c_double), ("list", C.c_void_p), ("count", C.c_void_p),
+    ]
 
 
 class BcgStateLayout(C.Structure):
@@ -125,7 +133,7 @@ class BcgEpisodeEnds(C.Structure):
 
 
 _STRUCTS = [BcgParams, BcgMapDesc, BcgPathDesc, BcgFootprintLut, BcgBatch, BcgStateLayout, BcgStepOut, BcgTurnParams,
-            BcgAisleSlots, BcgMiniGenParams, BcgMiniParams, BcgEnvRows, BcgEpisodeEnds]
+            BcgAisleSlots, BcgMiniGenParams, BcgMiniParams, BcgEnvRows, BcgEpisodeEnds, BcgWorldGen]
 
 # fixed rows / words of include/bcg_b200.h
 F_ROBOT, F_DROBOT, F_DPOSE, F_TIME, F_MIN_DIST, F_EP_RETURN, F_FIXED = 0, 7, 14, 17, 18, 19, 20
@@ -140,6 +148,10 @@ REWARD_CONTINUOUS, REWARD_PURE_PURSUIT = 0, 1
 # per-env parameter rows (BcgEnvRows)
 EP_F_SP, EP_F_AP, EP_F_PM, EP_F_ALPHA, EP_F_ROWS = 0, 1, 2, 3, 9
 EP_I_DELAY_CONTROL, EP_I_DELAY_POSE, EP_I_DELAY_STATE, EP_I_TIMEOUT, EP_I_NOISE_ON, EP_I_ROWS = 0, 1, 2, 3, 4, 5
+# BcgParams.auto_reset, BcgWorldGen.kind, the draw-index domain of the worlds a step draws
+AUTO_RESET_NEW_WORLD = 2
+WORLD_AISLE, WORLD_MINI = 0, 1
+NEW_WORLD_DRAW = 1 << 63
 # episode-end reason bits (BcgEpisodeEnds.reason)
 END_GOAL, END_COLLIDED, END_TIMEOUT, END_NOW = 1, 2, 4, 8
 

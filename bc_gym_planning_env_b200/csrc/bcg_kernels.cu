@@ -11,6 +11,8 @@
 //                                               scatter of the occupied cells of the source window
 //   (ego_tiles_kernel      persistent, 256-thread CTAs -- the dense per-pixel gather: pools of dense maps, and the envs
 //                                               the sparse kernel hands over when a batch mixes sparse and dense maps)
+//   (regenerate_kernel     fixed grid, between reward_kernel and the egocentric kernels when the batch auto-resets into new
+//                                               worlds: the done envs' final crops, new worlds and initial observations)
 // plus the set-up kernels (tile planes and summary, cell tiles, initial state), the device-side world generators and
 // the stand-alone entry points of the hook seam.
 // No tensor cores: nothing here is a dense contraction.
@@ -133,6 +135,12 @@ int check_batch(const BcgParams* p, const BcgBatch* b) {
   BCG_REQUIRE(b->lut.n_verts > 0 && b->lut.n_verts <= 32, "footprint must have 1..32 vertices");
   BCG_REQUIRE(b->lut.n_bins > 0 && b->lut.wpr > 0 && b->lut.max_rows > 0, "empty footprint table");
   BCG_REQUIRE(b->status && b->stats, "null status/stats");
+  if (p->auto_reset == BCG_AUTO_RESET_NEW_WORLD) {
+    BCG_REQUIRE(b->world_gen, "auto_reset BCG_AUTO_RESET_NEW_WORLD needs the world generator (BcgBatch.world_gen)");
+    BCG_REQUIRE(b->n_maps == b->n_envs && b->n_paths == b->n_envs && b->cell_tile_arena,
+                "auto_reset BCG_AUTO_RESET_NEW_WORLD (BcgBatch.world_gen) needs a batch of per-env world slots: n_maps == n_paths == "
+                "n_envs and the cell-tile arena");
+  }
   return BCG_OK;
 }
 
@@ -696,13 +704,10 @@ move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, c
 
 // auto-reset of env e (env.py:293-303) by its lane group: the rows, the observation and the egocentric record of the
 // initial state
-template <int G>
-__device__ __forceinline__ void reset_env_rows(const BcgParams& p, const BcgBatch& b, const BcgStepOut& out, int e, int ego_cap,
-                                               unsigned gl) {
+// the observation of env e's initial state (init_f / init_i) by one thread: obs_vec, goal_n_state and the egocentric record
+__device__ __forceinline__ void write_initial_observation(const BcgParams& p, const BcgBatch& b, const BcgStepOut& out, int e,
+                                                          int ego_cap) {
   const int64_t N = b.n_envs;
-  for (int r = gl; r < b.n_frows; r += G) b.state_f[(int64_t)r * N + e] = b.init_f[(int64_t)r * N + e];
-  for (int r = gl; r < b.n_irows; r += G) b.state_i[(int64_t)r * N + e] = b.init_i[(int64_t)r * N + e];
-  if (gl != 0) return;
   double dpose[3], dstate[7], c[3];
 #pragma unroll
   for (int r = 0; r < 3; ++r) dpose[r] = b.init_f[(int64_t)(BCG_F_DPOSE + r) * N + e];
@@ -728,6 +733,16 @@ __device__ __forceinline__ void reset_env_rows(const BcgParams& p, const BcgBatc
   }
 }
 
+template <int G>
+__device__ __forceinline__ void reset_env_rows(const BcgParams& p, const BcgBatch& b, const BcgStepOut& out, int e, int ego_cap,
+                                               unsigned gl) {
+  const int64_t N = b.n_envs;
+  for (int r = gl; r < b.n_frows; r += G) b.state_f[(int64_t)r * N + e] = b.init_f[(int64_t)r * N + e];
+  for (int r = gl; r < b.n_irows; r += G) b.state_i[(int64_t)r * N + e] = b.init_i[(int64_t)r * N + e];
+  if (gl != 0) return;
+  write_initial_observation(p, b, out, e, ego_cap);
+}
+
 // G lanes per env (power of two, 1 < G <= 32): 32 / G envs per warp.  Measured (profiles/r2_notes.md): 65 536 envs G = 8
 // 0.045 ms, 16: 0.050, 32: 0.065; 8 192 envs 0.022 / 0.018 / 0.019; 256 envs 0.0147 / 0.0121 / 0.0108 -- a large batch
 // wants few warps (the straight-line code is paid per warp), a small one a short chain (a chunk in one round).
@@ -735,6 +750,8 @@ __device__ __forceinline__ void reset_env_rows(const BcgParams& p, const BcgBatc
 // move_kernel left them (in the kernel body for the reason given at move_kernel)
 // ENDS: the step reports episode ends (BcgEpisodeEnds): the reason byte of every env and the final record of every env
 // whose episode ends now, taken before the auto-reset overwrites its rows and its egocentric record
+// With auto_reset == BCG_AUTO_RESET_NEW_WORLD a done env is not reset here: it is appended to BcgWorldGen.list, and
+// regenerate_kernel gives it a new world, its initial state and its initial observation.
 template <int G, bool ROWS, bool ENDS>
 __global__ void __launch_bounds__(BCG_REWARD_THREADS, BCG_REWARD_RESIDENT / BCG_REWARD_THREADS)
 reward_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStepOut out, const int ego_cap, const BcgEpisodeEnds ends) {
@@ -855,7 +872,14 @@ reward_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStepOut out, c
       }
     }
     if (active && done && p.auto_reset) {
-      reset_env_rows<G>(p, b, out, e, ego_cap, gl);
+      if (p.auto_reset != BCG_AUTO_RESET_NEW_WORLD) {
+        reset_env_rows<G>(p, b, out, e, ego_cap, gl);
+      } else if (gl == 0) {
+        // a new world: regenerate_kernel, launched behind this kernel, rewrites the rows and the observation (the final
+        // record above still read the old episode)
+        const BcgWorldGen* const wg = b.world_gen;
+        wg->list[atomicAdd(wg->count, 1)] = e;
+      }
     } else if (active && gl == 0) {
       b.state_f[BCG_F_MIN_DIST * N + e] = min_dist;
       b.state_f[BCG_F_EP_RETURN * N + e] = ep_return;
@@ -929,17 +953,13 @@ __global__ void __launch_bounds__(256) init_kernel(const BcgParams p, const BcgB
     init_env_state(p, b, L, e, path_ref(b, b.paths[b.path_id[e]]), lane);
 }
 
-// bcg_generate_aisles: one CTA per env (see bcg_generate.cuh); ROWS: the initial state uses the env's own goal tolerances
+// env e of bcg_generate_aisles by the whole CTA (see bcg_generate.cuh): the world of turn `tp` in the env's slots, its path,
+// chunk bounds and initial state.  Returns false (CTA-uniform) when the world does not fit the slots: the env is left
+// exactly as it was.  ROWS: the initial state uses the env's own goal tolerances
 template <bool ROWS>
-__global__ void __launch_bounds__(256) generate_aisles_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L,
-                                                              const BcgAisleSlots slots, const uint8_t* __restrict__ mask,
-                                                              const BcgTurnParams* __restrict__ turn_params,
-                                                              const uint64_t draw_index, const double path_delta,
-                                                              const BcgEnvRows rows) {
-  const int e = blockIdx.x;
-  if (mask && !mask[e]) return;
+__device__ __forceinline__ bool aisle_world(const BcgParams& p, const BcgBatch& b, const BcgStateLayout& L, const BcgAisleSlots& slots,
+                                            const BcgEnvRows& rows, const int e, const BcgTurnParams& tp, const double path_delta) {
   const int tid = threadIdx.x, nthr = blockDim.x;
-  const BcgTurnParams tp = turn_params ? turn_params[e] : draw_turn_params(p.seed, p.env_id_base + (uint64_t)e, draw_index);
   // every thread works the geometry out for itself (a few hundred flops; no broadcast, no barrier)
   const AisleGeometry g = aisle_geometry(tp, p.inv_resolution);
   const RefinedShape shape = refined_shape(g.way, path_delta);
@@ -954,7 +974,7 @@ __global__ void __launch_bounds__(256) generate_aisles_kernel(const BcgParams p,
                     (shape.n + 31) / 32 <= slots.chunk_pitch;
   if (!fits) {                                  // leave the env exactly as it was
     if (tid == 0) atomicAdd(b.status + BCG_STATUS_SLOT_OVERFLOW, 1u);
-    return;
+    return false;
   }
   AisleGenState* gs = reinterpret_cast<AisleGenState*>(slots.gen_state) + e;
   MapLayout m;
@@ -1041,17 +1061,30 @@ __global__ void __launch_bounds__(256) generate_aisles_kernel(const BcgParams p,
     else
       init_env_state(p, b, L, e, pr, lane);
   }
+  return true;
 }
 
-// bcg_generate_minis: one CTA per env.  Thread 0 samples (the draw count depends on the data), the CTA rasterises the
-// two walls, warp 0 checks the two end poses against them; accepted parameters get their path and initial state.
-__global__ void __launch_bounds__(128) generate_minis_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L,
-                                                             const BcgAisleSlots slots, const uint8_t* __restrict__ mask,
-                                                             const BcgMiniGenParams g, const BcgMiniParams* __restrict__ explicit_params,
-                                                             BcgMiniParams* __restrict__ params_out, const uint64_t draw_index,
-                                                             const double path_delta) {
+// bcg_generate_aisles: one CTA per env
+template <bool ROWS>
+__global__ void __launch_bounds__(256) generate_aisles_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L,
+                                                              const BcgAisleSlots slots, const uint8_t* __restrict__ mask,
+                                                              const BcgTurnParams* __restrict__ turn_params,
+                                                              const uint64_t draw_index, const double path_delta,
+                                                              const BcgEnvRows rows) {
   const int e = blockIdx.x;
   if (mask && !mask[e]) return;
+  const BcgTurnParams tp = turn_params ? turn_params[e] : draw_turn_params(p.seed, p.env_id_base + (uint64_t)e, draw_index);
+  aisle_world<ROWS>(p, b, L, slots, rows, e, tp, path_delta);
+}
+
+// env e of bcg_generate_minis by the whole CTA.  Thread 0 samples (the draw count depends on the data), the CTA rasterises
+// the two walls, warp 0 checks the two end poses against them; accepted parameters get their path and initial state.
+// Returns (CTA-uniform) 1 when a world was accepted, 0 when a world did not fit the slots, -1 when the sampler ran out of
+// tries; the status word of either failure is counted.
+__device__ __forceinline__ int mini_world(const BcgParams& p, const BcgBatch& b, const BcgStateLayout& L, const BcgAisleSlots& slots,
+                                          const BcgMiniGenParams& g, const BcgMiniParams* __restrict__ explicit_params,
+                                          BcgMiniParams* __restrict__ params_out, const int e, const uint64_t draw_index,
+                                          const double path_delta) {
   const int tid = threadIdx.x, nthr = blockDim.x, warp = tid >> 5, lane = tid & 31;
   __shared__ BcgMiniParams mp_s;
   __shared__ int verdict_s;          // 1 drawn / accepted, 0 draw again, -1 give up
@@ -1092,7 +1125,7 @@ __global__ void __launch_bounds__(128) generate_minis_kernel(const BcgParams p, 
                       (n_path + 31) / 32 <= slots.chunk_pitch;
     if (!fits) {
       if (tid == 0) atomicAdd(b.status + BCG_STATUS_SLOT_OVERFLOW, 1u);
-      return;                                     // (before anything of the slot was touched in this attempt)
+      return 0;                                   // (before anything of the slot was touched in this attempt)
     }
     if (gs->valid) {                              // erase what the slot holds, with the layout it was drawn in
       MapLayout old = m;
@@ -1203,6 +1236,18 @@ __global__ void __launch_bounds__(128) generate_minis_kernel(const BcgParams p, 
     }
   }
   if (!accepted && tid == 0) atomicAdd(b.status + BCG_STATUS_SAMPLER_EMPTY, 1u);
+  return accepted ? 1 : -1;
+}
+
+// bcg_generate_minis: one CTA per env
+__global__ void __launch_bounds__(128) generate_minis_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L,
+                                                             const BcgAisleSlots slots, const uint8_t* __restrict__ mask,
+                                                             const BcgMiniGenParams g, const BcgMiniParams* __restrict__ explicit_params,
+                                                             BcgMiniParams* __restrict__ params_out, const uint64_t draw_index,
+                                                             const double path_delta) {
+  const int e = blockIdx.x;
+  if (mask && !mask[e]) return;
+  mini_world(p, b, L, slots, g, explicit_params, params_out, e, draw_index, path_delta);
 }
 
 __global__ void __launch_bounds__(256) reset_kernel(const BcgBatch b, const uint8_t* __restrict__ mask) {
@@ -1683,6 +1728,34 @@ __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.comm
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
+// cv2.warpAffine(INTER_NEAREST) of one crop (record affine map A, map `map_id`) as a bounds-checked per-pixel gather from
+// the map's uint8 rows by the CTA's `nthr` threads: fixed-point tables in `tab` (ego_w + ego_h entries of shared memory),
+// then every crop pixel samples its cell, 0 outside the map.  Exact for any window; it holds a barrier, so every thread of
+// the CTA calls it.
+__device__ __forceinline__ void ego_gather_crop(const BcgBatch& b, const EgoAffine& A, const int map_id, const int ego_w, const int ego_h,
+                                                uint8_t* __restrict__ dst, int2* tab, const int tid, const int nthr) {
+  for (int i = tid; i < ego_w + ego_h; i += nthr) {
+    if (i < ego_w) {
+      tab[i] = make_int2(__double2int_rn(A.a11 * i * 1024), __double2int_rn(A.a21 * i * 1024));
+    } else {
+      const int t = i - ego_w;
+      tab[i] = make_int2(__double2int_rn((A.a12 * t + A.b1) * 1024) + 512, __double2int_rn((A.a22 * t + A.b2) * 1024) + 512);
+    }
+  }
+  __syncthreads();
+  const BcgMapDesc* md = b.maps + map_id;
+  const uint8_t* src = b.map_arena + md->data_off;
+  const int mw = md->width, mh = md->height, mpitch = md->pitch, npx = ego_w * ego_h;
+  for (int i = tid; i < npx; i += nthr) {
+    const int vv = i / ego_w, uu = i - vv * ego_w;
+    const int2 aa = tab[uu], bb = tab[ego_w + vv];
+    const long long X = ((long long)aa.x + bb.x) >> 10, Y = ((long long)aa.y + bb.y) >> 10;
+    uint8_t val = 0;
+    if (X >= 0 && X < mw && Y >= 0 && Y < mh) val = __ldg(src + Y * mpitch + X);
+    dst[i] = val;
+  }
+}
+
 // ENDS: items n_envs .. n_envs + min(count[0], capacity) - 1 are the final crops of the step's episode ends
 // (BcgEpisodeEnds): item n_envs + s renders the record final_ego_work[s] into final_ego_image[s], hands slot s over to the
 // dense kernel through final_list, and records no compact hit list
@@ -2108,27 +2181,7 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     } else if (b.flags & BCG_BATCH_SPARSE_EGO_ONLY) {
       // No dense pass follows this kernel (the host knows that no map of the batch is dense): the rare window that
       // overflows the cell list, or lies outside any sane range, is rendered here by the bounds-checked per-pixel gather.
-      const EgoAffine A = r->aff;
-      for (int i = tid; i < ego_w + ego_h; i += NT) {
-        if (i < ego_w) {
-          egs_tab[i] = make_int2(__double2int_rn(A.a11 * i * 1024), __double2int_rn(A.a21 * i * 1024));
-        } else {
-          const int t = i - ego_w;
-          egs_tab[i] = make_int2(__double2int_rn((A.a12 * t + A.b1) * 1024) + 512, __double2int_rn((A.a22 * t + A.b2) * 1024) + 512);
-        }
-      }
-      __syncthreads();
-      const BcgMapDesc* md = b.maps + r->map_id;
-      const uint8_t* src = b.map_arena + md->data_off;
-      const int mw = md->width, mh = md->height, mpitch = md->pitch;
-      for (int i = tid; i < npx; i += NT) {
-        const int vv = i / ego_w, uu = i - vv * ego_w;
-        const int2 aa = egs_tab[uu], bb = egs_tab[ego_w + vv];
-        const long long X = ((long long)aa.x + bb.x) >> 10, Y = ((long long)aa.y + bb.y) >> 10;
-        uint8_t val = 0;
-        if (X >= 0 && X < mw && Y >= 0 && Y < mh) val = __ldg(src + Y * mpitch + X);
-        dst[i] = val;
-      }
+      ego_gather_crop(b, r->aff, r->map_id, ego_w, ego_h, dst, egs_tab, tid, NT);
     } else if (final_crop) {
       if (tid == 0) ends.final_list[atomicAdd(ends.count + 1, 1)] = e - n;
     } else if (tid == 0) {
@@ -2144,6 +2197,70 @@ __global__ void __launch_bounds__(BCG_EGS_THREADS, BCG_EGS_CTAS) ego_sparse_kern
     }
     if (tid == 0) ids_s[(it + RD + 1) & 7] = drawn;
     __syncthreads();                            // list, tables and record `it` are free
+  }
+}
+
+// Auto-reset into a new world (BcgParams.auto_reset == BCG_AUTO_RESET_NEW_WORLD), launched behind reward_kernel: a fixed
+// grid (a captured graph replays it unchanged) whose CTAs take the envs reward_kernel listed in BcgWorldGen.list through the
+// item counter.  For each listed env:
+//   1. with episode ends, the egocentric image and a final slot: the final crop, gathered from the OLD world before its
+//      walls are erased (the egocentric kernels behind this one render the step's crops only);
+//   2. the new world, built by the body bcg_generate_aisles / bcg_generate_minis run for a masked env, drawn with
+//      (seed; env id, BCG_NEW_WORLD_DRAW | the step's index);
+//   3. the initial observation, written like the in-kernel reset writes it.  When the world failed (slot overflow, sampler
+//      out of tries; counted in the status words) the env restarts its current world, as auto_reset 1 does.
+// The last CTA to finish zeroes the list counters, so that every step's reward_kernel finds them zero.
+// ROWS: the aisle initial states use each env's own goal tolerances (as bcg_generate_aisles with rows).
+#define BCG_REGEN_THREADS 128
+#define BCG_REGEN_CTAS 4          // CTAs per SM of the fixed grid
+template <bool ROWS>
+__global__ void __launch_bounds__(BCG_REGEN_THREADS) regenerate_kernel(const BcgParams p, const BcgBatch b, const BcgStateLayout L,
+                                                                       const BcgEnvRows rows, const BcgStepOut out, const int ego_cap,
+                                                                       const BcgEpisodeEnds ends, const uint64_t step_index_arg) {
+  __shared__ int item_s;
+  __shared__ int2 tab_s[2 * BCG_EGO_MAX];
+  pdl_wait();                                            // reward_kernel's list, final records and step counter
+  const BcgWorldGen* const wg = b.world_gen;
+  const int tid = threadIdx.x, nthr = blockDim.x;
+  const int64_t N = b.n_envs;
+  // (reward_kernel has advanced the device-side step counter already: this step's index is one less)
+  const uint64_t step_index = b.step_counter ? *reinterpret_cast<const volatile uint64_t*>(b.step_counter) - 1ull : step_index_arg;
+  const uint64_t draw = BCG_NEW_WORLD_DRAW | step_index;
+  const int listed = *reinterpret_cast<const volatile int32_t*>(wg->count);
+  const int kind = wg->kind;
+  const BcgAisleSlots slots = wg->slots;
+  const bool finals = out.ego_image && ends.final_ego_image;
+  for (;;) {
+    if (tid == 0) item_s = atomicAdd(wg->count + 1, 1);
+    __syncthreads();
+    const int item = item_s;
+    __syncthreads();                                     // item_s is written again at the next item
+    if (item >= listed) break;
+    const int e = wg->list[item];
+    const int slot = finals ? ends.final_slot[e] : -1;
+    if (slot >= 0) {
+      const EgoTileWork* const rec =
+          reinterpret_cast<const EgoTileWork*>(reinterpret_cast<const uint8_t*>(ends.final_ego_work) + (int64_t)slot * BCG_EGO_WORK_BYTES);
+      ego_gather_crop(b, rec->aff, rec->map_id, p.ego_w, p.ego_h, ends.final_ego_image + (int64_t)slot * p.ego_w * p.ego_h, tab_s,
+                      tid, nthr);
+      __syncthreads();                                   // the old walls are read before they are erased
+    }
+    bool made;
+    if (kind == BCG_WORLD_MINI)
+      made = mini_world(p, b, L, slots, wg->mini, nullptr, reinterpret_cast<BcgMiniParams*>(slots.params_out), e, draw,
+                        wg->path_delta) == 1;
+    else
+      made = aisle_world<ROWS>(p, b, L, slots, rows, e, draw_turn_params(p.seed, p.env_id_base + (uint64_t)e, draw), wg->path_delta);
+    if (!made) {                                         // the current world's initial state
+      for (int r = tid; r < b.n_frows; r += nthr) b.state_f[(int64_t)r * N + e] = b.init_f[(int64_t)r * N + e];
+      for (int r = tid; r < b.n_irows; r += nthr) b.state_i[(int64_t)r * N + e] = b.init_i[(int64_t)r * N + e];
+    }
+    __syncthreads();                                     // the initial rows, path and map descriptor are complete
+    if (tid == 0) write_initial_observation(p, b, out, e, ego_cap);
+  }
+  if (tid == 0) {
+    __threadfence();
+    if (atomicAdd(wg->count + 2, 1) == (int)gridDim.x - 1) wg->count[0] = wg->count[1] = wg->count[2] = 0;
   }
 }
 
@@ -2329,6 +2446,7 @@ int64_t bcg_sizeof(int32_t which) {
     case 10: return sizeof(BcgMiniParams);
     case 11: return sizeof(BcgEnvRows);
     case 12: return sizeof(BcgEpisodeEnds);
+    case 13: return sizeof(BcgWorldGen);
     default: return -1;
   }
 }
@@ -2691,6 +2809,7 @@ int bcg_step(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, cons
   }
   cudaStream_t s = (cudaStream_t)stream;
   const BcgStateLayout L = make_layout(*p);
+  const bool new_world = p->auto_reset == BCG_AUTO_RESET_NEW_WORLD;
   if (events && events[0]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[0], s));
   {
     if (events && events[1]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[1], s));
@@ -2727,13 +2846,19 @@ int bcg_step(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, cons
     BCG_CHECK_CUDA(launch_step_kernel(rewards[group][rows != nullptr][ends != nullptr], blocks_for(ns * (8 << group), BCG_REWARD_THREADS),
                                       BCG_REWARD_THREADS, 0, s, pdl_reward, *p, *b, *out, cap, en));
     BCG_CHECK_CUDA(cudaGetLastError());
+    if (new_world) {
+      const int grid = b->n_envs < BCG_REGEN_CTAS * sms ? b->n_envs : BCG_REGEN_CTAS * sms;
+      BCG_CHECK_CUDA(launch_step_kernel(rows ? regenerate_kernel<true> : regenerate_kernel<false>, grid, BCG_REGEN_THREADS, 0, s, true,
+                                        *p, *b, L, r, *out, cap, en, step_index));
+    }
   }
   if (events && events[3]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[3], s));
   if (out->ego_image) {
     BCG_REQUIRE((out->ego_hits != nullptr) == (out->ego_hit_count != nullptr) && (!out->ego_hits || out->ego_hit_cap > 0),
                 "ego_hits, ego_hit_count and ego_hit_cap go together");
+    // (a new-world batch's final crops were rendered by regenerate_kernel)
     if (int rc = launch_ego_image(p, b, out->ego_image, EgoHits{out->ego_hits, out->ego_hit_count, out->ego_hit_cap, !(events && events[3])},
-                                  ends, s))
+                                  new_world ? nullptr : ends, s))
       return rc;
   }
   if (events && events[4]) BCG_CHECK_CUDA(cudaEventRecord((cudaEvent_t)events[4], s));

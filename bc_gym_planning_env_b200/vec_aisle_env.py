@@ -64,8 +64,10 @@ class _VecSlotEnv(VecPlanEnv):
     cell-tile, tile-plane and path arenas, and host accessors that read a world back."""
 
     def _setup_slots(self, params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
-                     footprint_scale, footprint, map_cells, path_points, record_bytes, params_ids=None, episode_ends=False,
-                     episode_end_capacity=None):
+                     footprint_scale, footprint, map_cells, path_points, record_bytes, world_kind, params_ids=None,
+                     episode_ends=False, episode_end_capacity=None):
+        if auto_reset == 'new_world' and not self._draw_new_turn_on_reset:
+            raise ValueError("auto_reset='new_world' draws a new world at every episode end: it needs draw_new_turn_on_reset=True")
         self._configure(params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego, 'tiles',
                         params_ids, episode_ends, episode_end_capacity)
         if not self.params.refine_path:
@@ -83,6 +85,24 @@ class _VecSlotEnv(VecPlanEnv):
         self._make_batch()
         # generated worlds are thin walls (BcgMapDesc.occupied stays 0): no env ever needs the dense egocentric kernel
         self._batch.flags |= nat.BATCH_SPARSE_EGO_ONLY
+        if self.new_world_reset:
+            self._setup_world_gen(world_kind)
+
+    def _setup_world_gen(self, kind):
+        """auto_reset='new_world': the BcgWorldGen the step's regeneration kernel reads (in device memory), its list of the
+        envs to regenerate and its counters"""
+        self._regen_list = torch.zeros(self.n_envs, dtype=torch.int32, device=self.device)
+        self._regen_count = torch.zeros(4, dtype=torch.int32, device=self.device)
+        wg = nat.BcgWorldGen()
+        wg.kind = kind
+        C.memmove(C.addressof(wg.slots), C.addressof(self._slots), C.sizeof(nat.BcgAisleSlots))
+        wg.slots.params_out = self._records.data_ptr()
+        if kind == nat.WORLD_MINI:
+            wg.mini = self._gen
+        wg.path_delta = float(self.params.path_delta)
+        wg.list, wg.count = self._regen_list.data_ptr(), self._regen_count.data_ptr()
+        self._world_gen = self._to_device(np.frombuffer(bytes(wg), dtype=np.uint8).copy())
+        self._batch.world_gen = self._world_gen.data_ptr()
 
     def _alloc_slots(self, record_bytes):
         n, dev = self.n_envs, self.device
@@ -153,31 +173,38 @@ class VecRandomAisleTurnEnv(_VecSlotEnv):
     def __init__(self, n_envs, params=None, draw_new_turn_on_reset=True, seed=0, turn_params=None,
                  noise_parameters=DEFAULT_NOISE, auto_reset=False, device=None, env_id_base=0, with_ego=False,
                  footprint_scale=1.0, footprint=None, resolution=0.03, max_map_cells=None, max_path_points=None,
-                 params_ids=None, episode_ends=False, episode_end_capacity=None):
+                 params_ids=None, episode_ends=False, episode_end_capacity=None, compact_ego=False):
         """
         :param n_envs: batch size; env e draws from the Philox stream (seed; env_id_base + e, draw index)
         :param params, noise_parameters, params_ids: one EnvParams and noise setting for the batch, or a pool of them
             and the set of every env (see VecPlanEnv); `reset(mask, params_ids=...)` moves envs to other sets
         :param draw_new_turn_on_reset: `reset` draws a new turn for the envs it resets (reference default)
-        :param auto_reset: the step's own in-kernel reset.  It restores the initial state of the env's CURRENT world
-            (no launch, no host round trip) and does NOT draw a new turn, whatever draw_new_turn_on_reset says: an
-            episode that ends is replayed on the same aisle.  For the reference's behaviour -- a new turn for every
-            episode (synth_turn_env.py:278-291) -- keep auto_reset=False and call `env.reset(done)` after the step:
-            one generation launch for the envs that finished.
+        :param auto_reset: the step's own reset of the envs whose episodes end (no host round trip).
+            'new_world': the reference's behaviour -- a new turn for every episode (synth_turn_env.py:278-291) -- inside
+            the step: its regeneration kernel draws the finished envs' new turns (Philox (seed; env id, 2^63 | step
+            index)), builds them and writes their initial observations; works with step_graph, rollout(_graph) and
+            step_host.  Needs draw_new_turn_on_reset.  A turn that overflows its slot restarts the env's current
+            world and `check_status()` raises.
+            True: restores the initial state of the env's CURRENT world and does NOT draw a new turn, whatever
+            draw_new_turn_on_reset says: an episode that ends is replayed on the same aisle.
+            False: no reset; `env.reset(done)` after the step gives the finished envs new turns (one generation launch
+            plus a full egocentric pass).
         :param turn_params: optional list of n_envs TurnParams for the first worlds (default: drawn on device)
         :param max_map_cells, max_path_points: slot capacities per env (default: worst case of the distribution)
-        :param episode_ends, episode_end_capacity: see VecPlanEnv.  With auto_reset, `reset(done)` after a step gives the
-            envs that finished a new turn; their final observations (`final_observation()`) are those of the old one
+        :param episode_ends, episode_end_capacity: see VecPlanEnv.  The final observations (`final_observation()`) of
+            envs that got a new turn, in the step ('new_world') or by `reset(done)` after it, are those of the old one
+        :param compact_ego: see VecPlanEnv (`step_host(images='compact')`)
         """
         from bc_gym_planning_env_b200.envs.base.params import EnvParams
         first = params[0] if envp.is_pool(params) and len(params) else params
         pd = (first if first is not None else EnvParams()).path_delta
         cells, points = worst_case_world(float(resolution), pd)
         self._draw_new_turn_on_reset = bool(draw_new_turn_on_reset)
+        self._compact_ego = bool(compact_ego)
         self._setup_slots(params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
                           footprint_scale, footprint, max_map_cells if max_map_cells is not None else cells,
-                          max_path_points if max_path_points is not None else points, TURN_DTYPE.itemsize, params_ids,
-                          episode_ends, episode_end_capacity)
+                          max_path_points if max_path_points is not None else points, TURN_DTYPE.itemsize, nat.WORLD_AISLE,
+                          params_ids, episode_ends, episode_end_capacity)
         self._turns = self._records
         self._slots.params_out = self._turns.data_ptr()
         self.generate(turn_params=turn_params)
@@ -281,9 +308,10 @@ class VecRandomMiniEnv(_VecSlotEnv):
             goal tolerances 0.2 m / pi/8)
         :param mini_params: optional list of n_envs MiniEnvParams for the first worlds (built as they are, like
             MiniEnv(config)); default: sampled on the device
-        :param auto_reset: in-kernel reset to the initial state of the env's CURRENT world; it never samples a new
-            world (see VecRandomAisleTurnEnv).  The reference builds a new env per episode (mini_env.py:447-470):
-            auto_reset=False + `env.reset(done)` does that here.
+        :param auto_reset: 'new_world': the reference's new env per episode (mini_env.py:447-470) inside the step,
+            sampled with (seed; env id, 2^63 | step index); a sampler that runs out of tries restarts the env's current
+            world and `check_status()` raises.  True: in-kernel reset to the initial state of the env's CURRENT world,
+            never a new one (see VecRandomAisleTurnEnv).  False: no reset; `env.reset(done)` samples new worlds.
         :param episode_ends, episode_end_capacity: see VecPlanEnv
         """
         from bc_gym_planning_env_b200.envs.base.params import EnvParams
@@ -308,7 +336,7 @@ class VecRandomMiniEnv(_VecSlotEnv):
         diag = np.hypot(params.inner_w + 2 * params.mid_margin, params.inner_h + 2 * params.mid_margin)
         self._setup_slots(ep, n_envs, ep.resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
                           footprint_scale, footprint, side_x * side_y, int(np.ceil(diag / ep.path_delta)) + 8, MINI_DTYPE.itemsize,
-                          episode_ends=episode_ends, episode_end_capacity=episode_end_capacity)
+                          nat.WORLD_MINI, episode_ends=episode_ends, episode_end_capacity=episode_end_capacity)
         self.generate(mini_params=mini_params)
         self.check_status()
 

@@ -174,6 +174,13 @@ class VecPlanEnv(object):
     def _configure(self, params, n_envs, resolution, noise_parameters, seed, auto_reset, device, env_id_base, with_ego,
                    ego_staging, params_ids=None, episode_ends=False, episode_end_capacity=None):
         """Everything that does not depend on where the maps and paths come from."""
+        if isinstance(auto_reset, str):
+            if auto_reset != 'new_world':
+                raise ValueError("auto_reset must be True, False or 'new_world', got %r" % (auto_reset,))
+            if not isinstance(self, _device_world_types()):
+                raise ValueError("auto_reset='new_world' needs worlds drawn on the device (VecRandomAisleTurnEnv, "
+                                 "VecRandomMiniEnv): the maps of this batch were uploaded by the host and have no slots")
+        self.new_world_reset = auto_reset == 'new_world'      # (the batch of device-drawn worlds sets it up)
         self.episode_ends = bool(episode_ends)
         self.episode_end_capacity = None
         if self.episode_ends:
@@ -251,7 +258,7 @@ class VecPlanEnv(object):
         if p.reward_provider_name not in kinds:          # reward_provider_examples_factory.py:44-47
             raise AssertionError("Unknown reward provider: {}. Should be one of {}".format(p.reward_provider_name, list(kinds)))
         cp.reward_kind = kinds[p.reward_provider_name]
-        cp.auto_reset = 1 if self.auto_reset else 0
+        cp.auto_reset = nat.AUTO_RESET_NEW_WORLD if self.new_world_reset else 1 if self.auto_reset else 0
         return cp
 
     def _to_device(self, arr):
@@ -645,8 +652,9 @@ class VecPlanEnv(object):
         self._step_index += horizon
 
     def launches_per_step(self):
-        """Kernels one `step` launches: move_kernel + reward_kernel, then the egocentric kernel(s)."""
-        n = 2
+        """Kernels one `step` launches: move_kernel + reward_kernel (+ regenerate_kernel with auto_reset='new_world'), then
+        the egocentric kernel(s)."""
+        n = 3 if self.new_world_reset else 2
         if not self.with_ego:
             return n
         if self._ego_list is None or os.environ.get("BCG_EGO_KERNEL") == "dense":

@@ -106,7 +106,9 @@ typedef struct BcgParams {
   int32_t reward_kind;        /* 0 ContinuousRewardProvider (reward.py:173-288), 1 ContinuousRewardPurePursuitProvider
                                  (reward.py:291-371) */
   int32_t reserved;
-  int32_t auto_reset;         /* restore the initial state of envs that report done */
+  int32_t auto_reset;         /* envs that report done start their next episode inside the step: 0 no, 1 in the same world
+                                 (the initial state the env has), BCG_AUTO_RESET_NEW_WORLD in a newly drawn world
+                                 (needs BcgBatch.world_gen) */
   int32_t ego_variant;        /* 0: EgocentricCostmap wrapper (egocentric.py:125-160): crop about the delayed pose,
                                  9-vector goal_n_state.  1: ColoredEgoCostmapRandomAisleTurnEnv
                                  (synth_turn_env.py:396-420): crop about the TRUE robot pose, goal = unit vector
@@ -232,6 +234,8 @@ typedef struct BcgBatch {
                             takes the step index from word 0 and increments it on the device when the step is done
                             (word 1 is its scratch) -- so that a captured CUDA graph of a step can be replayed
                             without changing a kernel argument                                                    */
+  const struct BcgWorldGen* world_gen; /* device pointer, needed when BcgParams.auto_reset == BCG_AUTO_RESET_NEW_WORLD
+                            (NULL otherwise): how the step draws a new world for an env whose episode ends */
 } BcgBatch;
 
 /* TurnParams (envs/synth_turn_env.py:18-31): geometry of one aisle turn */
@@ -271,6 +275,35 @@ typedef struct BcgMiniParams {
   double start[3], end[3];
   double a[2], o[2], b[2];
 } BcgMiniParams;
+
+/* BcgParams.auto_reset */
+#define BCG_AUTO_RESET_NEW_WORLD 2
+/* BcgWorldGen.kind */
+#define BCG_WORLD_AISLE 0 /* bcg_generate_aisles' worlds */
+#define BCG_WORLD_MINI 1  /* bcg_generate_minis' worlds   */
+
+/* Auto-reset into a newly drawn world (BcgParams.auto_reset == BCG_AUTO_RESET_NEW_WORLD), in device memory, reached through
+ * BcgBatch.world_gen.  The batch must be made of the generators' per-env slots (n_maps == n_paths == n_envs, cell tiles).
+ * At a step, reward_kernel appends every env that is done to `list` (count[0] of them) instead of restoring its initial
+ * state; a regeneration kernel behind it then gives each listed env what bcg_generate_aisles / bcg_generate_minis give a
+ * masked env -- a drawn world in its slot, its path and initial state -- and writes its initial observation (obs_vec,
+ * goal_n_state, egocentric record), so that the step's egocentric kernels render the new world.  With BcgEpisodeEnds and the
+ * egocentric image, the final crop of an env with a slot is rendered from the old world before it is erased.  Draws are
+ * keyed (p->seed; p->env_id_base + e, BCG_NEW_WORLD_DRAW | step index), a domain the host's draw indices never reach (see
+ * bcg_generate_aisles).  A world that does not fit its slot (BCG_STATUS_SLOT_OVERFLOW) or a sampler that runs out of tries
+ * (BCG_STATUS_SAMPLER_EMPTY) restarts the env in its current world, as auto_reset 1 does; the status word counts it. */
+#define BCG_NEW_WORLD_DRAW 0x8000000000000000ull
+typedef struct BcgWorldGen {
+  int32_t kind;              /* BCG_WORLD_AISLE or BCG_WORLD_MINI                                                     */
+  int32_t reserved;
+  BcgAisleSlots slots;       /* the slots, as passed to the generator; params_out (optional) points at BcgTurnParams [n]
+                                for aisles, BcgMiniParams [n] for minis                                              */
+  BcgMiniGenParams mini;     /* the sampling space (BCG_WORLD_MINI)                                                   */
+  double path_delta;
+  int32_t* list;             /* device [n_envs] scratch: the envs to regenerate at this step                          */
+  int32_t* count;            /* device [4], zero before the first step: [0] listed envs, [1] item counter, [2] finished
+                                CTAs of the regeneration kernel (whose last CTA zeroes the words for the next step)    */
+} BcgWorldGen;
 
 typedef struct BcgStateLayout {
   int32_t n_frows, n_irows;
@@ -365,7 +398,7 @@ int bcg_abi_version(void);
 size_t bcg_last_error(char* buf, size_t cap);
 /* sizeof() of the ABI structs, in declaration order: 0 BcgParams, 1 BcgMapDesc, 2 BcgPathDesc,
  * 3 BcgFootprintLut, 4 BcgBatch, 5 BcgStateLayout, 6 BcgStepOut, 7 BcgTurnParams, 8 BcgAisleSlots, 9 BcgMiniGenParams,
- * 10 BcgMiniParams, 11 BcgEnvRows, 12 BcgEpisodeEnds; -1 for anything else.  Lets a
+ * 10 BcgMiniParams, 11 BcgEnvRows, 12 BcgEpisodeEnds, 13 BcgWorldGen; -1 for anything else.  Lets a
  * binding (ctypes, cffi, ...) verify its struct mirrors before the first call. */
 int64_t bcg_sizeof(int32_t which);
 /* number of CUDA devices visible, <0 on error; makes a missing GPU a loud failure for callers */
@@ -394,7 +427,12 @@ int bcg_reset_where(const BcgBatch* b, const uint8_t* mask, void* stream);
  * `path_delta`), derive both tile planes, and make the initial state (env.py:179-214, reward.py:261-288).
  * The previous walls of the slot are erased pixel by pixel, so a reset costs O(wall pixels), not O(map).
  * With `rows` the initial states use each env's own goal tolerances (NULL: those of p); rows changed before the call (a
- * new parameter set at a reset) are what the new worlds' initial states see.  Needs BcgBatch.cell_tile_arena. */
+ * new parameter set at a reset) are what the new worlds' initial states see.  Needs BcgBatch.cell_tile_arena.
+ * Draw keys: the host's calls use draw indices below BCG_NEW_WORLD_DRAW (2^63).  A step with auto_reset ==
+ * BCG_AUTO_RESET_NEW_WORLD draws the new world of env e with (p->seed; p->env_id_base + e, BCG_NEW_WORLD_DRAW | s), s the
+ * step index its odometry noise uses (bcg_step's step_index, or word 0 of BcgBatch.step_counter); an env ends at most
+ * once per step, so every key is drawn once, a batch split over shards (env_id_base) draws the worlds one batch draws,
+ * and a replay from the same step index draws the same worlds.  bcg_generate_minis keys its draws the same way. */
 int bcg_generate_aisles(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const BcgAisleSlots* slots,
                         const uint8_t* mask, const BcgTurnParams* turn_params, uint64_t draw_index, double path_delta,
                         void* stream);
@@ -434,10 +472,14 @@ int bcg_generate_minis(const BcgParams* p, const BcgBatch* b, const BcgAisleSlot
  * ended envs before it resets them, and the egocentric kernels render the final crops after the step's own.  Final
  * crops need the cell-tile planes (BcgBatch.cell_tile_arena).
  *
+ * p->auto_reset == BCG_AUTO_RESET_NEW_WORLD (see BcgWorldGen): reward_kernel lists the done envs instead of resetting them
+ * and regenerate_kernel, launched between reward_kernel and the egocentric kernels, gives them new worlds, initial states
+ * and initial observations (and renders their final crops from the old worlds).
+ *
  * events (NULL: none are recorded): per-kernel hooks, events[0..4] are caller-created cudaEvent_t handles recorded on
- * `stream`: [0], [1] before move_kernel, [2] between move_kernel and reward_kernel, [3] after reward_kernel (reward /
- * done / compact observation are final: a host consumer's copies can start here while the egocentric kernel runs), [4]
- * after the egocentric kernels.  Any entry may be NULL (not recorded).  A kernel with an event recorded right before it
+ * `stream`: [0], [1] before move_kernel, [2] between move_kernel and reward_kernel, [3] after reward_kernel, or after
+ * regenerate_kernel when it runs (reward / done / compact observation are final: a host consumer's copies can start here
+ * while the egocentric kernel runs), [4] after the egocentric kernels.  Any entry may be NULL (not recorded).  A kernel with an event recorded right before it
  * is not launched as a programmatic dependent of its predecessor. */
 int bcg_step(const BcgParams* p, const BcgBatch* b, const BcgEnvRows* rows, const void* actions, int32_t action_is_f64,
              uint64_t step_index, const BcgStepOut* out, const BcgEpisodeEnds* ends, void* const* events, void* stream);
