@@ -412,16 +412,35 @@ __device__ __forceinline__ int find_foot_bin_header(const BcgFootprintLut& lut, 
   return bin;
 }
 
+// The footprint mask of pose (x, y, th) placed on a map: its angle bin and its box in map pixels.
+struct FootBox {
+  int X0, Y0;          // map pixel of the mask's top-left corner
+  int nrows, fwidth;   // mask bounding box
+  int bin;
+};
+
+__device__ __forceinline__ FootBox foot_box(const BcgFootprintLut& lut, double origin_x, double origin_y, double inv_res,
+                                            double x, double y, double th, uint32_t* status) {
+  FootBox f;
+  short4 h;                                              // xmin, ymin, nrows, width
+  f.bin = find_foot_bin_header(lut, th, status, h);
+  f.X0 = world_to_pixel_1d(x, origin_x, inv_res) + h.x;
+  f.Y0 = world_to_pixel_1d(y, origin_y, inv_res) + h.y;
+  f.nrows = h.z;
+  f.fwidth = h.w;
+  return f;
+}
+
 __device__ __forceinline__ WorkCollide make_work_collide(const BcgParams& p, const BcgBatch& b, int map_id, double x, double y,
                                                          double th) {
   const BcgMapDesc m = b.maps[map_id];
+  const FootBox f = foot_box(b.lut, m.origin_x, m.origin_y, p.inv_resolution, x, y, th, b.status);
   WorkCollide w;
-  short4 h;                                                                          // xmin, ymin, nrows, width
-  w.bin = find_foot_bin_header(b.lut, th, b.status, h);
-  w.X0 = world_to_pixel_1d(x, m.origin_x, p.inv_resolution) + h.x;
-  w.Y0 = world_to_pixel_1d(y, m.origin_y, p.inv_resolution) + h.y;
-  w.nrows = h.z;
-  w.fwidth = h.w;
+  w.bin = f.bin;
+  w.X0 = f.X0;
+  w.Y0 = f.Y0;
+  w.nrows = (int16_t)f.nrows;
+  w.fwidth = (int16_t)f.fwidth;
   w.tile_off = m.tile_off;
   w.data_off = m.data_off;
   w.tiles_x = m.tiles_x;
@@ -492,19 +511,75 @@ __device__ __forceinline__ bool collide_tiles(const BcgBatch& b, const WorkColli
   return __any_sync(BCG_FULL, hit != 0u);
 }
 
-// pose_collides (envs/base/env.py:464-489) by ONE thread, for the thread-per-env kinematics + collision kernel.  The
-// footprint box spans a few bands of 16 rows x <= 3 tiles of 32 columns.  A thread-serial gather pays a full memory
-// round trip per dependent load, so the loads are batched: (1) the tile-summary words of ALL bands (`sum`: 1 bit per
-// tile of the occupancy plane, a superset of the lethal plane), one round trip; (2) per non-empty tile under the
+// pose_collides (envs/base/env.py:464-489) by ONE thread per env (collide_warp_balanced, collide_thread_listed,
+// collide_thread), for the thread-per-env kinematics + collision kernels.  The footprint box spans a few bands of 16 rows x
+// a few tiles of 32 columns.  A thread-serial gather pays a full memory round trip per dependent load, so the loads are
+// batched: (1) the tile-summary words of up to BCG_BANDS bands (`sum`:
+// 1 bit per tile of the occupancy plane, a superset of the lethal plane), one round trip; (2) per non-empty tile under the
 // footprint -- a corridor is mostly free space: typically 0..3 of the 15 -- its four 16-byte quarters and the 16
-// footprint-mask rows of its band, 20 independent loads, one round trip; early exit on the first hit.
-// Same verdict as collide_tiles.
-struct FootBox {
-  int X0, Y0;          // map pixel of the mask's top-left corner
-  int nrows, fwidth;   // mask bounding box
-  int bin;
-};
+// footprint-mask rows of its band, one round trip; early exit on the first hit.  Same verdict as collide_tiles.
+constexpr int BCG_BANDS = 6;                             // bands per batch of summary words (a 64-row mask spans <= 5)
 
+// tm[k] = the non-empty-tile bits of band tyb + k over the tile columns tx0 .. tx1 (bit j <-> column tx0 + j), from one or
+// two summary words; 0 for the bands past ty1
+__device__ __forceinline__ void summary_bands(const uint32_t* __restrict__ sum, int tiles_x, int tyb, int ty1, int tx0, int tx1,
+                                              uint32_t (&tm)[BCG_BANDS]) {
+  const int sw = (tiles_x + 31) >> 5;
+  const uint32_t colmask = (2u << (tx1 - tx0)) - 1u;
+#pragma unroll
+  for (int k = 0; k < BCG_BANDS; ++k) {
+    tm[k] = 0u;
+    if (tyb + k <= ty1) {
+      const uint32_t* srow = sum + (tyb + k) * sw;
+      const int w0 = tx0 >> 5;
+      uint64_t two = __ldg(srow + w0);
+      if ((tx1 >> 5) != w0) two |= (uint64_t)__ldg(srow + w0 + 1) << 32;
+      tm[k] = (uint32_t)(two >> (tx0 & 31)) & colmask;
+    }
+  }
+}
+
+// The 16 mask rows of the band whose first tile row is mask row dy0, for one-word rows whose bins start 16-byte aligned:
+// nine aligned 16-byte pairs from the even row at or below dy0 (rows beyond the mask are zero in the table; pairs outside
+// the bin's max_rows rows are not loaded).
+__device__ __forceinline__ void load_band_rows(const uint64_t* __restrict__ rows, int max_rows, int dy0, uint64_t (&v)[18]) {
+  const int base = dy0 & ~1;
+#pragma unroll
+  for (int jj = 0; jj < 9; ++jj) {
+    const int r0 = base + 2 * jj;
+    ulonglong2 q = make_ulonglong2(0ull, 0ull);
+    if ((unsigned)r0 < (unsigned)max_rows) q = __ldg(reinterpret_cast<const ulonglong2*>(rows + r0));
+    v[2 * jj] = q.x;
+    v[2 * jj + 1] = q.y;
+  }
+}
+
+// the 16 rows of the tile at `tile` (bit j of a row <-> its column j), as four 16-byte loads
+__device__ __forceinline__ void load_tile(const uint32_t* __restrict__ tile, uint32_t (&ws)[16]) {
+  const uint4* tq = reinterpret_cast<const uint4*>(tile);
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const uint4 w = __ldg(tq + q);
+    ws[4 * q] = w.x;
+    ws[4 * q + 1] = w.y;
+    ws[4 * q + 2] = w.z;
+    ws[4 * q + 3] = w.w;
+  }
+}
+
+// whether a tile's 16 rows ws meet the band's mask rows v (load_band_rows with the same dy0); rel = the tile's first
+// column - X0.  (The callers load the tile before the rows: both are then in flight together.)
+__device__ __forceinline__ bool tile_meets_rows(const uint32_t (&ws)[16], const uint64_t (&v)[18], int dy0, int rel) {
+  const int odd = dy0 & 1;
+  uint32_t hit = 0u;
+#pragma unroll
+  for (int r = 0; r < 16; ++r) hit |= ws[r] & mask_window32(odd ? v[r + 1] : v[r], rel);
+  return hit != 0u;
+}
+
+// The boxes collide_warp_balanced does not take (multi-word mask rows, > 4 tile columns, > 6 bands, rows not in aligned
+// pairs): per batch of BCG_BANDS bands the summary words, then the non-empty tiles band by band, each row's 32 mask bits
+// by mask_bits32, which is exact for any number of words per row.
 __device__ __forceinline__ bool collide_thread(const BcgFootprintLut& lut, const uint32_t* __restrict__ tiles,
                                                const uint32_t* __restrict__ sum, int tiles_x, int map_w, int map_h,
                                                const FootBox& f) {
@@ -515,96 +590,45 @@ __device__ __forceinline__ bool collide_thread(const BcgFootprintLut& lut, const
   const int ty0 = max(Y0, 0) >> 4, ty1 = min(Y1, map_h - 1) >> 4;
   const int wpr = lut.wpr;
   const uint64_t* __restrict__ rows = lut.rows + (int64_t)f.bin * lut.max_rows * wpr;
-  const int sw = (tiles_x + 31) >> 5;
-  const uint32_t colmask = (2u << (tx1 - tx0)) - 1u;     // bit j <-> tile column tx0 + j
-  const bool pair_rows = (lut.max_rows & 1) == 0 && (reinterpret_cast<uintptr_t>(lut.rows) & 15) == 0;   // rows of a bin start 16-byte aligned
-  constexpr int MAXB = 6;                                // bands per batch (a 64-row mask spans <= 5)
-  for (int tyb = ty0; tyb <= ty1; tyb += MAXB) {
-    uint32_t tm[MAXB];
+  for (int tyb = ty0; tyb <= ty1; tyb += BCG_BANDS) {
+    uint32_t tm[BCG_BANDS];
+    summary_bands(sum, tiles_x, tyb, ty1, tx0, tx1, tm);
+    // the non-empty tiles of each band's first four columns (all of them under a mask <= 97 px wide) are asked into L2
+    // right away (no register, no wait): the walk below then pays one DRAM round trip in all instead of one per tile
+    uint32_t ahead = 0u;
 #pragma unroll
-    for (int k = 0; k < MAXB; ++k) {
-      tm[k] = 0u;
-      if (tyb + k <= ty1) {
-        const uint32_t* srow = sum + (tyb + k) * sw;
-        const int w0 = tx0 >> 5;
-        uint64_t two = __ldg(srow + w0);
-        if ((tx1 >> 5) != w0) two |= (uint64_t)__ldg(srow + w0 + 1) << 32;
-        tm[k] = (uint32_t)(two >> (tx0 & 31)) & colmask;
-      }
-    }
-    // Non-empty tiles of all bands as ONE per-thread list (4 bits per band: a 64-column mask spans <= 3 tiles), so that
-    // a warp iterates max-over-lanes(tiles of a lane) times, not sum-over-bands(max-over-lanes(tiles of the band)).
-    uint32_t todo = 0u;
-    const bool flat = (tx1 - tx0) < 4;
-#pragma unroll
-    for (int k = 0; k < MAXB; ++k) todo |= flat ? (tm[k] << (4 * k)) : 0u;
-    // every listed tile is asked into L2 right away (no register, no wait): the loop below then pays one DRAM round trip
-    // in all instead of one per tile
-    for (uint32_t ahead = todo; ahead != 0u; ahead &= ahead - 1u) {
+    for (int k = 0; k < BCG_BANDS; ++k) ahead |= (tm[k] & 15u) << (4 * k);
+    for (; ahead != 0u; ahead &= ahead - 1u) {
       const int bit = __ffs((int)ahead) - 1;
       const uint32_t* tp = tiles + ((((int64_t)(tyb + (bit >> 2)) * tiles_x) + tx0 + (bit & 3)) << 4);
       asm volatile("prefetch.global.L2 [%0];" ::"l"(tp));
     }
-    int kb = 0;                                            // wide footprints: band by band
-    int vband = -1;                                        // band whose mask rows v[] holds
-    uint64_t v[18];
-    while (flat ? (todo != 0u) : (kb < MAXB)) {
-      int k, j;
-      if (flat) {
-        const int bit = __ffs((int)todo) - 1;
-        todo &= todo - 1u;
-        k = bit >> 2;
-        j = bit & 3;
-      } else {
-        uint32_t mk = 0u;
+    int k = 0;
+    while (k < BCG_BANDS) {                                // band by band
+      uint32_t mk = 0u;                                    // tm[k] by selects: a runtime index would put tm[] in local memory
 #pragma unroll
-        for (int q = 0; q < MAXB; ++q) mk = (q == kb) ? tm[q] : mk;
-        if (mk == 0u) { ++kb; continue; }
-        k = kb;
-        j = __ffs((int)mk) - 1;
+      for (int q = 0; q < BCG_BANDS; ++q) mk = (q == k) ? tm[q] : mk;
+      if (mk == 0u) { ++k; continue; }
 #pragma unroll
-        for (int q = 0; q < MAXB; ++q) if (q == kb) tm[q] &= tm[q] - 1u;
-      }
-      const int ty = tyb + k, tx = tx0 + j;
+      for (int q = 0; q < BCG_BANDS; ++q) if (q == k) tm[q] &= tm[q] - 1u;
+      const int ty = tyb + k, tx = tx0 + __ffs((int)mk) - 1;
       const int dy0 = (ty << 4) - Y0;                      // mask row of the band's first tile row
-      const uint4* tq = reinterpret_cast<const uint4*>(tiles + ((((int64_t)ty * tiles_x) + tx) << 4));
-      const uint4 w0 = __ldg(tq), w1 = __ldg(tq + 1), w2 = __ldg(tq + 2), w3 = __ldg(tq + 3);
+      uint32_t ws[16];
+      load_tile(tiles + ((((int64_t)ty * tiles_x) + tx) << 4), ws);
       const int rel = (tx << 5) - X0;
       uint32_t hit = 0u;
-      if (wpr == 1 && pair_rows) {
-        // the band's 16 mask rows as nine aligned 16-byte pairs starting at the even row at or below dy0 (rows beyond
-        // the mask are zero in the table; pairs outside the bin's max_rows rows are not loaded).  The tiles of a thread's
-        // list come band by band, so the rows are kept for the next tile of the same band
-        const int base = dy0 & ~1, odd = dy0 & 1;
-        if (k != vband) {
-          vband = k;
 #pragma unroll
-          for (int jj = 0; jj < 9; ++jj) {
-            const int r0 = base + 2 * jj;
-            ulonglong2 q = make_ulonglong2(0ull, 0ull);
-            if ((unsigned)r0 < (unsigned)lut.max_rows) q = __ldg(reinterpret_cast<const ulonglong2*>(rows + r0));
-            v[2 * jj] = q.x;
-            v[2 * jj + 1] = q.y;
-          }
-        }
-        const uint32_t ws[16] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w, w2.x, w2.y, w2.z, w2.w, w3.x, w3.y, w3.z, w3.w};
-#pragma unroll
-        for (int r = 0; r < 16; ++r) hit |= ws[r] & mask_window32(odd ? v[r + 1] : v[r], rel);
-      } else {
-        const uint32_t ws[16] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w, w2.x, w2.y, w2.z, w2.w, w3.x, w3.y, w3.z, w3.w};
-#pragma unroll
-        for (int r = 0; r < 16; ++r)                       // (unrolled: a dynamic index would put the tile words in local memory)
-          if (ws[r] != 0u && (unsigned)(dy0 + r) < (unsigned)f.nrows) hit |= ws[r] & mask_bits32(rows + (int64_t)(dy0 + r) * wpr, wpr, rel);
-      }
+      for (int r = 0; r < 16; ++r)                         // (unrolled: a dynamic index would put the tile words in local memory)
+        if (ws[r] != 0u && (unsigned)(dy0 + r) < (unsigned)f.nrows) hit |= ws[r] & mask_bits32(rows + (int64_t)(dy0 + r) * wpr, wpr, rel);
       if (hit) return true;
     }
   }
   return false;
 }
 
-// The tile loop of collide_thread for a box in the fast shape (one-word mask rows in aligned pairs, <= 4 tile columns,
-// <= 6 bands) whose non-empty tiles are already listed in `todo` (4 bits per band from band ty0, bit j <-> column tx0 + j):
-// per tile its four 16-byte quarters + the band's mask rows, which are kept for the next tile of the same band.
+// The tile loop for a box in the fast shape (one-word mask rows in aligned pairs, <= 4 tile columns, <= 6 bands) whose
+// non-empty tiles are already listed in `todo` (4 bits per band from band ty0, bit j <-> column tx0 + j).  The list comes
+// band by band, so a band's mask rows are kept for its next tile.
 __device__ __forceinline__ bool collide_thread_listed(const BcgFootprintLut& lut, const uint32_t* __restrict__ tiles,
                                                       int tiles_x, const FootBox& f, int ty0, int tx0, uint32_t todo) {
   const uint64_t* __restrict__ rows = lut.rows + (int64_t)f.bin * lut.max_rows;
@@ -615,32 +639,19 @@ __device__ __forceinline__ bool collide_thread_listed(const BcgFootprintLut& lut
     todo &= todo - 1u;
     const int k = bit >> 2, ty = ty0 + k, tx = tx0 + (bit & 3);
     const int dy0 = (ty << 4) - f.Y0;
-    const uint4* tq = reinterpret_cast<const uint4*>(tiles + ((((int64_t)ty * tiles_x) + tx) << 4));
-    const uint4 w0 = __ldg(tq), w1 = __ldg(tq + 1), w2 = __ldg(tq + 2), w3 = __ldg(tq + 3);
-    const int rel = (tx << 5) - f.X0;
-    const int base = dy0 & ~1, odd = dy0 & 1;
+    uint32_t ws[16];
+    load_tile(tiles + ((((int64_t)ty * tiles_x) + tx) << 4), ws);
     if (k != vband) {
       vband = k;
-#pragma unroll
-      for (int jj = 0; jj < 9; ++jj) {
-        const int r0 = base + 2 * jj;
-        ulonglong2 q = make_ulonglong2(0ull, 0ull);
-        if ((unsigned)r0 < (unsigned)lut.max_rows) q = __ldg(reinterpret_cast<const ulonglong2*>(rows + r0));
-        v[2 * jj] = q.x;
-        v[2 * jj + 1] = q.y;
-      }
+      load_band_rows(rows, lut.max_rows, dy0, v);
     }
-    const uint32_t ws[16] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w, w2.x, w2.y, w2.z, w2.w, w3.x, w3.y, w3.z, w3.w};
-    uint32_t hit = 0u;
-#pragma unroll
-    for (int r = 0; r < 16; ++r) hit |= ws[r] & mask_window32(odd ? v[r + 1] : v[r], rel);
-    if (hit) return true;
+    if (tile_meets_rows(ws, v, dy0, (tx << 5) - f.X0)) return true;
   }
   return false;
 }
 
-// collide_thread with the tiles of a WARP's 32 envs dealt out evenly.  In collide_thread a warp walks its tile loop as often
-// as its busiest lane has non-empty tiles under the footprint (~9 times for ~3 tiles per lane on the aisle workload), and
+// collide_thread with the tiles of a WARP's 32 envs dealt out evenly.  In collide_thread_listed a warp walks its tile loop as
+// often as its busiest lane has non-empty tiles under the footprint (~9 times for ~3 tiles per lane on the aisle workload), and
 // that loop was three quarters of move_kernel's instructions.  Here every lane still reads its own env's summary words and
 // lists its tiles (4 bits per band), then the warp's (env, tile) pairs are numbered by a prefix sum and lane l takes pair
 // (lanes present) r + l of round r: it finds the owner by binary search over the inclusive counts, gets the owner's box by shuffles,
@@ -656,28 +667,15 @@ __device__ __forceinline__ bool collide_warp_balanced(const BcgFootprintLut& lut
   const bool inside = !(X1 < 0 || X0 >= map_w || Y1 < 0 || Y0 >= map_h);
   const int tx0 = max(X0, 0) >> 5, tx1 = min(X1, map_w - 1) >> 5;
   const int ty0 = max(Y0, 0) >> 4, ty1 = min(Y1, map_h - 1) >> 4;
-  constexpr int MAXB = 6;
   const bool pair_rows = lut.wpr == 1 && (lut.max_rows & 1) == 0 && (reinterpret_cast<uintptr_t>(lut.rows) & 15) == 0;
-  const bool fast = inside && pair_rows && (tx1 - tx0) < 4 && (ty1 - ty0) < MAXB && tiles_x < 2048 && ty0 < 2048 && tx0 < 1024 &&
-                    X0 > -32768 && Y0 > -32768;
+  const bool fast = inside && pair_rows && (tx1 - tx0) < 4 && (ty1 - ty0) < BCG_BANDS && tiles_x < 2048 && ty0 < 2048 &&
+                    tx0 < 1024 && X0 > -32768 && Y0 > -32768;
   uint32_t todo = 0u;
   if (fast) {
-    const int sw = (tiles_x + 31) >> 5;
-    const uint32_t colmask = (2u << (tx1 - tx0)) - 1u;
-    uint32_t tm[MAXB];
+    uint32_t tm[BCG_BANDS];
+    summary_bands(sum, tiles_x, ty0, ty1, tx0, tx1, tm);
 #pragma unroll
-    for (int k = 0; k < MAXB; ++k) {
-      tm[k] = 0u;
-      if (ty0 + k <= ty1) {
-        const uint32_t* srow = sum + (ty0 + k) * sw;
-        const int w0 = tx0 >> 5;
-        uint64_t two = __ldg(srow + w0);
-        if ((tx1 >> 5) != w0) two |= (uint64_t)__ldg(srow + w0 + 1) << 32;
-        tm[k] = (uint32_t)(two >> (tx0 & 31)) & colmask;
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < MAXB; ++k) todo |= tm[k] << (4 * k);
+    for (int k = 0; k < BCG_BANDS; ++k) todo |= tm[k] << (4 * k);
   }
   const int cnt = __popc(todo);
   int incl = cnt;
@@ -693,64 +691,52 @@ __device__ __forceinline__ bool collide_warp_balanced(const BcgFootprintLut& lut
   // tiles: a dealt round costs about 1.5 of its iterations.
   const int longest = (int)__reduce_max_sync(act, (unsigned)cnt);
   const int rounds = (total + last) / (last + 1);
-  if (3 * rounds >= 2 * longest) {
-    bool h = false;
-    if (fast) h = collide_thread_listed(lut, tile_arena + tile_off, tiles_x, f, ty0, tx0, todo);
-    else if (inside) h = collide_thread(lut, tile_arena + tile_off, sum, tiles_x, map_w, map_h, f);
-    return h;
-  }
-  // what a lane needs of a pair's owner, packed for the shuffles
-  const uint32_t pk_xy = ((uint32_t)X0 & 0xffffu) | ((uint32_t)Y0 << 16);
-  const uint32_t pk_t = (uint32_t)ty0 | ((uint32_t)tx0 << 11) | ((uint32_t)tiles_x << 21);
-  const int excl = incl - cnt;
   bool myhit = false;
-  for (int base = 0; base < total; base += last + 1) {     // a round deals one pair to each lane that is there
-    const int i = base + (int)lane;
-    const bool has = i < total;
-    int o = 0;                                             // owner = the first lane whose inclusive count exceeds i
+  if (3 * rounds >= 2 * longest) {
+    if (fast) myhit = collide_thread_listed(lut, tile_arena + tile_off, tiles_x, f, ty0, tx0, todo);
+  } else {
+    // what a lane needs of a pair's owner, packed for the shuffles
+    const uint32_t pk_xy = ((uint32_t)X0 & 0xffffu) | ((uint32_t)Y0 << 16);
+    const uint32_t pk_t = (uint32_t)ty0 | ((uint32_t)tx0 << 11) | ((uint32_t)tiles_x << 21);
+    const int excl = incl - cnt;
+    for (int base = 0; base < total; base += last + 1) {   // a round deals one pair to each lane that is there
+      const int i = base + (int)lane;
+      const bool has = i < total;
+      int o = 0;                                           // owner = the first lane whose inclusive count exceeds i
 #pragma unroll
-    for (int st = 16; st >= 1; st >>= 1) {
-      const int probe = o + st - 1;
-      const int t = __shfl_sync(act, incl, min(probe, last));
-      if (probe <= last && t <= i) o += st;
-    }
-    o = min(o, last);
-    const uint32_t otodo = __shfl_sync(act, todo, o);
-    const int r = i - __shfl_sync(act, excl, o);
-    const uint32_t oxy = __shfl_sync(act, pk_xy, o), ot = __shfl_sync(act, pk_t, o);
-    const int obin = __shfl_sync(act, f.bin, o);
-    const unsigned long long ooff = __shfl_sync(act, (unsigned long long)tile_off, o);
-    uint32_t hit = 0u;
-    if (has) {
-      uint32_t m = otodo;                                  // the pair's tile: set bit number r of the owner's list
-      for (int q = 0; q < r; ++q) m &= m - 1u;
-      const int bit = __ffs((int)m) - 1;
-      const int ty = (int)(ot & 2047u) + (bit >> 2), tx = (int)((ot >> 11) & 1023u) + (bit & 3);
-      const int oX0 = (int)(short)(oxy & 0xffffu), oY0 = (int)(short)(oxy >> 16);
-      const uint4* tq = reinterpret_cast<const uint4*>(tile_arena + (int64_t)ooff + ((((int64_t)ty * (int)(ot >> 21)) + tx) << 4));
-      const uint4 w0 = __ldg(tq), w1 = __ldg(tq + 1), w2 = __ldg(tq + 2), w3 = __ldg(tq + 3);
-      const int dy0 = (ty << 4) - oY0, rel = (tx << 5) - oX0;
-      const uint64_t* __restrict__ rows = lut.rows + (int64_t)obin * lut.max_rows;
-      const int rbase = dy0 & ~1, odd = dy0 & 1;
-      uint64_t v[18];
-#pragma unroll
-      for (int jj = 0; jj < 9; ++jj) {
-        const int r0 = rbase + 2 * jj;
-        ulonglong2 q = make_ulonglong2(0ull, 0ull);
-        if ((unsigned)r0 < (unsigned)lut.max_rows) q = __ldg(reinterpret_cast<const ulonglong2*>(rows + r0));
-        v[2 * jj] = q.x;
-        v[2 * jj + 1] = q.y;
+      for (int st = 16; st >= 1; st >>= 1) {
+        const int probe = o + st - 1;
+        const int t = __shfl_sync(act, incl, min(probe, last));
+        if (probe <= last && t <= i) o += st;
       }
-      const uint32_t ws[16] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w, w2.x, w2.y, w2.z, w2.w, w3.x, w3.y, w3.z, w3.w};
-#pragma unroll
-      for (int rr = 0; rr < 16; ++rr) hit |= ws[rr] & mask_window32(odd ? v[rr + 1] : v[rr], rel);
-    }
-    const uint32_t hb = __ballot_sync(act, hit != 0u);
-    for (uint32_t h2 = hb; h2 != 0u; h2 &= h2 - 1u) {      // rare: a collision ends the episode
-      const int l = __ffs((int)h2) - 1;
-      if (__shfl_sync(act, o, l) == (int)lane) myhit = true;
+      o = min(o, last);
+      const uint32_t otodo = __shfl_sync(act, todo, o);
+      const int r = i - __shfl_sync(act, excl, o);
+      const uint32_t oxy = __shfl_sync(act, pk_xy, o), ot = __shfl_sync(act, pk_t, o);
+      const int obin = __shfl_sync(act, f.bin, o);
+      const unsigned long long ooff = __shfl_sync(act, (unsigned long long)tile_off, o);
+      bool hit = false;
+      if (has) {
+        uint32_t m = otodo;                                // the pair's tile: set bit number r of the owner's list
+        for (int q = 0; q < r; ++q) m &= m - 1u;
+        const int bit = __ffs((int)m) - 1;
+        const int ty = (int)(ot & 2047u) + (bit >> 2), tx = (int)((ot >> 11) & 1023u) + (bit & 3);
+        const int oX0 = (int)(short)(oxy & 0xffffu), oY0 = (int)(short)(oxy >> 16);
+        const int dy0 = (ty << 4) - oY0;
+        uint32_t ws[16];
+        load_tile(tile_arena + (int64_t)ooff + ((((int64_t)ty * (int)(ot >> 21)) + tx) << 4), ws);
+        uint64_t v[18];
+        load_band_rows(lut.rows + (int64_t)obin * lut.max_rows, lut.max_rows, dy0, v);
+        hit = tile_meets_rows(ws, v, dy0, (tx << 5) - oX0);
+      }
+      const uint32_t hb = __ballot_sync(act, hit);
+      for (uint32_t h2 = hb; h2 != 0u; h2 &= h2 - 1u) {    // rare: a collision ends the episode
+        const int l = __ffs((int)h2) - 1;
+        if (__shfl_sync(act, o, l) == (int)lane) myhit = true;
+      }
     }
   }
+  // boxes outside the fast shape, after either branch: one call site, so one inlined copy of collide_thread
   if (inside && !fast) myhit = collide_thread(lut, tile_arena + tile_off, sum, tiles_x, map_w, map_h, f);
   return myhit;
 }

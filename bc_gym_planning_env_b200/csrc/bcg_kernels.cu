@@ -428,7 +428,7 @@ __device__ __forceinline__ uint32_t ego_band_span(const EgoAffine& A, int ego_w,
 //
 //   move_kernel    one THREAD per env.  Everything that is scalar per env and one long dependent chain: control delay
 //                  (:371-373), robot model (tricycle_model.py:478-538 / differential_drive.py:236-265) with Philox
-//                  noise, footprint lookup, pose_collides (env.py:464-489; collide_thread: batched loads of the
+//                  noise, footprint lookup, pose_collides (env.py:464-489; collide_warp_balanced: batched loads of the
 //                  non-empty lethal tiles under the footprint only), rollback (:458-459), pose / robot-state delay lines
 //                  (:377-389), time / iter / sticky collision (:383-393), the compact observation and the 128-byte
 //                  record of the egocentric kernel.  Every state access is a coalesced SoA row.  It leaves a 144-byte
@@ -612,15 +612,7 @@ move_kernel(const BcgParams p_batch, const BcgBatch b, const BcgStateLayout L, c
     for (int r = 0; r < 3; ++r) b.cand[r * N + e] = s[r];
   }
   // ---- env.py:455 pose_collides of the proposed pose --------------------------------------------------------------------------
-  FootBox fb;
-  {
-    short4 h;                                            // xmin, ymin, nrows, width
-    fb.bin = find_foot_bin_header(b.lut, s[2], b.status, h);
-    fb.X0 = world_to_pixel_1d(s[0], m.origin_x, p.inv_resolution) + h.x;
-    fb.Y0 = world_to_pixel_1d(s[1], m.origin_y, p.inv_resolution) + h.y;
-    fb.nrows = h.z;
-    fb.fwidth = h.w;
-  }
+  const FootBox fb = foot_box(b.lut, m.origin_x, m.origin_y, p.inv_resolution, s[0], s[1], s[2], b.status);
   const bool hit = collide_warp_balanced(b.lut, b.tile_arena, m.tile_off, b.occ_sum_arena + m.sum_off, m.tiles_x, m.width,
                                          m.height, fb, warp_item_mask(e - (int)(threadIdx.x & 31), b.n_envs), threadIdx.x & 31);
   if (hit) {  // env.py:458-459 + tricycle_model.py:471-476: pose restored, v = w = 0, wheel / steer command kept
@@ -1428,12 +1420,7 @@ __global__ void __launch_bounds__(64) collision_thread_kernel(const BcgBatch b, 
   uint4* fw = reinterpret_cast<uint4*>(&f);
 #pragma unroll
   for (int k = 0; k < 3; ++k) fw[k] = __ldg(rec + k);
-  FootBox fb;
-  fb.X0 = f.X0;
-  fb.Y0 = f.Y0;
-  fb.nrows = f.nrows;
-  fb.fwidth = f.fwidth;
-  fb.bin = f.bin;
+  const FootBox fb = {f.X0, f.Y0, f.nrows, f.fwidth, f.bin};
   flags[e] = collide_warp_balanced(b.lut, b.tile_arena, f.tile_off, b.occ_sum_arena + f.sum_off, f.tiles_x, f.map_w, f.map_h,
                                    fb, warp_item_mask(e - (int)(threadIdx.x & 31), b.n_envs), threadIdx.x & 31) ? 1 : 0;
 }
